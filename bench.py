@@ -3,11 +3,23 @@
 
     python bench.py [--gpus N] [--steps K] [--warmup W]          # this repo, on GPUs
     python bench.py --impl reference [--steps K] [--warmup W]    # reference CPU algorithm
+    python bench.py --steps K --dump-outputs DIR                 # also write the results (one GPU)
 
 Workload (N=1): config C4 -- the 30-qubit complex128 random circuit, depth 200
 (200 x (30 single-qubit gates from {H,T,RZ,X,P} + 15 CZ on a random perfect
 matching) = 9000 gates, ``workloads.sv_random_circuit(30, 200, seed=30)``).
-One *step* = the whole circuit applied to |0...0>.
+One *step* = the whole circuit applied to |0...0>.  Every timed loop (kernel-only,
+HBM-roof operating point, end to end) runs exactly --steps steps.
+
+--dump-outputs DIR writes, after the timed steps, what the last step computed, as
+float64 .npy files (48 MiB at n = 30), so that two builds can be compared output for
+output; the circuit and the sample are seeded, so the same arguments give the same inputs:
+  state_sample_index  2^20 basis-state indices drawn without replacement (seed DUMP_SEED)
+  state_sample        the final amplitudes of the kernel-only path at those indices, (k, 2) = (re, im)
+  state_marginal      probabilities of the 2^20 basis states of qubits 0..19 (summed over the
+                      other qubits): every amplitude of the state contributes
+  e2e_sample          the array Simulator.run returned in the last end-to-end step, at the same
+                      indices (unless the end-to-end run is skipped)
 
 Reported on one JSON line:
   value      gates/s with the state resident in HBM and the fused plan compiled
@@ -82,7 +94,14 @@ def parse_args():
     ap.add_argument("--cpu-seconds", type=float, default=20.0)
     ap.add_argument("--traffic-bytes", type=float, default=None,
                     help="dram bytes per k_tile_pass launch from an ncu --set full capture")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last step computed as DIR/<name>.npy")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "b200" or int(os.environ.get("WORLD_SIZE", "1")) > 1):
+        ap.error("--dump-outputs is implemented for the single-GPU run")
+    return args
 
 
 # ---- helpers ---------------------------------------------------------------------------------
@@ -394,6 +413,36 @@ def time_plan(backend, plan, state, reset, steps: int):
     return total
 
 
+DUMP_SEED = 20251020
+DUMP_SAMPLE_LOG2 = 20
+DUMP_MARGINAL_QUBITS = 20
+
+
+def dump_sample_index(n: int) -> np.ndarray:
+    """The sorted basis-state indices whose amplitudes --dump-outputs writes (every index up to n = 20)."""
+    size = 1 << min(n, DUMP_SAMPLE_LOG2)
+    return np.sort(np.random.default_rng(DUMP_SEED).choice(1 << n, size=size, replace=False))
+
+
+def as_re_im(amps: np.ndarray) -> np.ndarray:
+    return np.ascontiguousarray(amps, dtype=np.complex128).view(np.float64).reshape(-1, 2)
+
+
+def dump_device_state(out_dir: str, buf, n: int) -> None:
+    """Sample and qubit-0..19 marginal of the 2^n device state ``buf`` (torch complex128)."""
+    import torch
+    idx = dump_sample_index(n)
+    np.save(os.path.join(out_dir, "state_sample_index.npy"), idx.astype(np.float64))
+    np.save(os.path.join(out_dir, "state_sample.npy"),
+            as_re_im(buf[torch.from_numpy(idx).to(buf.device)].cpu().numpy()))
+    m = min(n, DUMP_MARGINAL_QUBITS)
+    rows = buf.reshape(1 << m, -1)                    # row r: the basis states whose qubits 0..m-1 read r
+    chunk = max(1, (1 << 26) // rows.shape[1])        # bounds the temporary to 1 GiB
+    marginal = torch.cat([torch.view_as_real(rows[r:r + chunk]).square().sum(dim=(1, 2))
+                          for r in range(0, rows.shape[0], chunk)])
+    np.save(os.path.join(out_dir, "state_marginal.npy"), marginal.cpu().numpy())
+
+
 def run_b200(args):
     import torch
     from quantum_computations_b200 import _capi, engine, workloads
@@ -441,6 +490,9 @@ def run_b200(args):
         kernel_ms = time_plan(backend, plan, state, reset, args.steps)
     launches = engine.launch_count(backend) - launches0 - args.steps      # minus the reset kernels
     norm = state.norm()
+    if args.dump_outputs:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        dump_device_state(args.dump_outputs, state.buf, n)
     value = args.steps * ngates / (kernel_ms * 1e-3)
     ms_per_step = kernel_ms / args.steps
 
@@ -464,8 +516,8 @@ def run_b200(args):
         alt = engine.Plan(backend, n, ops, alt_opts)
         reset()
         alt.execute(state.buf)
-        alt_ms = time_plan(backend, alt, state, reset, max(1, min(2, args.steps)))
-        alt_steps = max(1, min(2, args.steps))
+        alt_steps = args.steps
+        alt_ms = time_plan(backend, alt, state, reset, alt_steps)
         alt_launch = alt_ms / (alt_steps * alt.stats["n_passes"])
         alt_ach = bytes_per_launch / (alt_launch * 1e-3) / 1e9
         roofline_hbm_point = {"bound": "hbm", "kernel": "k_tile_pass", "achieved": alt_ach, "peak": peak,
@@ -491,7 +543,7 @@ def run_b200(args):
             sim = Simulator(circuit, plan_options=opts)
             sim.run(init, out=outs[0])                          # warm-up
             # one call after the other, each blocking until its result is in host memory
-            e2e_steps = max(1, min(args.steps, 2))
+            e2e_steps = args.steps
             t0 = time.perf_counter()
             for _ in range(e2e_steps):
                 sim.run(init, out=outs[0])
@@ -503,7 +555,7 @@ def run_b200(args):
             dt = dt_serial
             piped_steps = 0
             if len(outs) == 2:
-                piped_steps = max(6, args.steps)        # the last copy has nothing to hide behind: amortise the drain
+                piped_steps = args.steps
                 t0 = time.perf_counter()
                 pending = None
                 for k in range(piped_steps):
@@ -514,8 +566,10 @@ def run_b200(args):
                 pending.result()
                 torch.cuda.synchronize()
                 dt = (time.perf_counter() - t0) / piped_steps
-            out = outs[0]
+            out = outs[(piped_steps - 1) % 2] if piped_steps else outs[0]     # the result of the last step
             assert abs(np.vdot(out[:1 << 20], out[:1 << 20]).real) >= 0.0
+            if args.dump_outputs:
+                np.save(os.path.join(args.dump_outputs, "e2e_sample.npy"), as_re_im(out[dump_sample_index(n)]))
             h2d = passes * PASS_PARAM_BYTES + 64 * n            # kernel-parameter blocks + product-state amplitudes
             e2e = {"value": ngates / dt, "unit": "gates/s", "h2d_bytes_per_step": h2d, "d2h_bytes_per_step": need,
                    "seconds_per_step": dt, "steps": piped_steps or e2e_steps,

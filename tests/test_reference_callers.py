@@ -1,73 +1,57 @@
-"""Unmodified REFERENCE callers on top of this package (drop-in claim, SURVEY.md section 8b).
+"""REFERENCE callers on top of this package (drop-in claim, SURVEY.md section 8b).
 
-``compat.install()`` registers this package as ``simulators.dv_simulator``; the reference's own
-scripts -- ``randomised_benchmarking.random_circ``, ``gkp_simulator.transpiler.MBGKPCircuit`` and
-``dv_circuits.grover`` -- are then imported from /root/reference as they are and must build,
-type-dispatch and simulate with this package's classes.  Runs in a subprocess (it rewires
-``sys.modules``); skipped where the reference checkout does not exist (the GPU box)."""
-import os
-import subprocess
-import sys
-import textwrap
+``compat.install()`` registers this package as ``simulators.dv_simulator``, the import path the
+reference's scripts use.  The scripts themselves are not part of this repository, so what they
+built and computed is replayed from the vectors recorded from them by tests/golden/make_golden.py:
+the circuits of ``randomised_benchmarking.random_circ`` with the depth its ``MBGKPCircuit``
+reported (rb.npz), and the circuits of ``dv_circuits.grover`` with their output kets
+(grover.npz).  Rebuilt from the classes found under the reference's import path, they must be
+this package's classes, draw the same gates as ``workloads.rb_random_circuit`` and reproduce the
+recorded results."""
+import pickle
 
-import pytest
+import numpy as np
 
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = "/root/reference"
-PAPER = os.path.join(REF, "impact_of_finite_squeezing_on_near-term_quantum_computations_using_gkp_qubits")
+import parity_cases as pc
+from golden.specs import as_oracle_ops, from_spec
+from oracle import strided
+from quantum_computations_b200 import compat, gates, layering, simulator, workloads
 
-SCRIPT = textwrap.dedent(r'''
-    import pickle, sys
-    import numpy as np
-    sys.path.insert(0, {root!r}); sys.path.insert(0, {root!r} + "/tests")
-    sys.path.insert(0, {ref!r}); sys.path.insert(0, {paper!r})
-    import quantum_computations_b200.compat as compat
+
+def test_recorded_reference_callers_run_on_this_package(emu_backend):
     compat.install()
-    from quantum_computations_b200 import gates, simulator, workloads
-    from quantum_computations_b200.states import State
-    from emu_backend import emu
-    from golden.specs import as_oracle_ops
-    from oracle import strided
+    from simulators.dv_simulator import gates as dv_gates
+    from simulators.dv_simulator import simulator as dv_simulator
+    from simulators.dv_simulator import states as dv_states
+    assert dv_gates is gates and dv_simulator.Simulator is simulator.Simulator
 
-    # 1. the reference's RB generator builds OUR gate objects, the same ones workloads.rb_random_circuit draws
-    import randomised_benchmarking as rb                      # unmodified reference script
-    assert rb.dv_gates is gates and rb.DVSimulator is simulator.Simulator
-    for seed, depth in ((1, 8), (2, 15), (3, 20)):
-        dv_circ, gkp_circ = rb.random_circ(2, depth, seed)
+    # 1. the reference's RB generator: the same draws as workloads.rb_random_circuit, and the
+    #    measurement-based depth its MBGKPCircuit reported is the layer depth of this package
+    meta, z = pc.load("rb.npz")
+    rng = np.random.default_rng(meta["seed"])
+    for i, rec in enumerate(meta["samples"]):
+        dv_circ = [from_spec(s, dv_gates, dv_simulator, z, states=dv_states) for s in rec["circuit"]]
         assert all(type(g).__module__ == gates.__name__ for g in dv_circ)
-        mine = workloads.rb_random_circuit(2, depth, np.random.default_rng(seed))
+        mine = workloads.rb_random_circuit(2, rec["depth"], rng)
         assert [(type(g).__name__, list(g.indices)) for g in dv_circ] == \
-               [(type(g).__name__, list(g.indices)) for g in mine]
-        assert gkp_circ.depth() == depth
+               [(type(g).__name__, list(g.indices)) for g in mine], i
+        assert layering.MBLayering.of(dv_circ, 2).depth() == rec["mb_depth"] == rec["depth"], i
 
-    # 2. the measurement-based transpiler dispatches on our classes (GKP/transpiler.py:41-63)
-    from simulators.gkp_simulator.transpiler import MBGKPCircuit
-    circ = MBGKPCircuit(3)
-    for g in (gates.H(0), gates.CZ(0, 1), gates.P(2), gates.SWAP(1, 2), gates.Pdg(0), gates.I(1)):
-        circ.add_gate(g)
-    circ.fill()
-    assert circ.depth() >= 3
-
-    # 3. the reference's Grover circuit, simulated by this package (host emulator backend) == CPU oracle
-    import dv_circuits as ccs
-    for tagged in ([3, 6], [0, 4]):
-        gcirc = ccs.grover(ccs.oracle(tagged))
+    # 2. the reference's Grover circuit, simulated by this package (host emulator backend) ==
+    #    the reference's own output == CPU oracle
+    meta, z = pc.load("grover.npz")
+    full = [rec for rec in meta if rec["kind"] == "full"]
+    assert len(full) >= 2
+    for rec in full:
+        gcirc = [from_spec(s, dv_gates, dv_simulator, z, states=dv_states) for s in rec["circuit"]]
         assert all(type(g).__module__ in (gates.__name__, simulator.__name__) for g in gcirc)
-        out = simulator.Simulator(gcirc, backend=emu()).run(None)
+        out = dv_simulator.Simulator(gcirc, backend=emu_backend).run(None)
+        assert pc.rel_err(out, z[rec["out"]]) < pc.RTOL
         ref, _ = strided.run(as_oracle_ops(gcirc), np.ones(1, dtype=np.complex128))
         assert np.abs(out - ref).max() < 1e-12
         probs = np.abs(out) ** 2
-        assert all(abs(probs[t] - 0.5) < 1e-12 for t in tagged)
+        assert all(abs(probs[t] - 0.5) < 1e-12 for t in rec["tagged"])
 
-    # 4. gate objects survive pickling (the reference farms samples out with multiprocessing)
+    # 3. gate objects survive pickling (the reference farms samples out with multiprocessing)
     g2 = pickle.loads(pickle.dumps([gates.H(0), gates.RZ(1, 0.3), gates.CZ(0, 1)]))
     assert [type(g).__name__ for g in g2] == ["H", "RZ", "CZ"] and np.allclose(g2[1].matrix, gates.RZ(1, 0.3).matrix)
-    print("REFERENCE-CALLERS-OK")
-''')
-
-
-@pytest.mark.skipif(not os.path.isdir(PAPER), reason="the reference checkout is not present on this machine")
-def test_unmodified_reference_callers_run_on_this_package():
-    out = subprocess.run([sys.executable, "-c", SCRIPT.format(root=ROOT, ref=REF, paper=PAPER)],
-                         capture_output=True, text=True, timeout=600, cwd=ROOT)
-    assert out.returncode == 0 and "REFERENCE-CALLERS-OK" in out.stdout, out.stdout[-2000:] + out.stderr[-4000:]

@@ -139,6 +139,23 @@ int qsim_reduce_expect(const void* ket, const void* rho, int n_qubits, double* o
 int qsim_reduce_purity(const void* rho, int n_qubits, double* out_re_im, void* stream);
 int qsim_reduce_trace(const void* rho, int n_qubits, double* out_re_im, void* stream);
 
+/* ---- Pauli-sum expectation values (npq.expect / expecth on Pauli strings) -------------
+ * A Pauli string on n qubits is a pair of masks (x, z); bit q of each stands for reference
+ * qubit q (as in qsim_plan_options_t::apply_tail_mask).  I = (0,0), X = (1,0), Z = (0,1),
+ * Y = (1,1); the operator is P = i^popc(x & z) X^x Z^z (Z applied first), so every string is
+ * Hermitian.  Masks with bits at or above n_qubits, and n_qubits outside [1, 63], are
+ * QSIM_ERR_ARG; n_terms == 0 does nothing.  Results come back in the caller's term order; a
+ * fixed grid and a fixed summation tree make repeated calls bit-identical. */
+/* <psi|P_t|psi> for n_terms Pauli strings on a ket (real; P_t Hermitian, see convention above).
+ * x_masks/z_masks/out are HOST arrays of n_terms; synchronises the stream.  Terms are grouped
+ * by X mask; one read of the state serves up to 32 terms whose X masks span at most 4 dimensions. */
+int qsim_expect_pauli(const void* state, int n_qubits, int64_t n_terms, const uint64_t* x_masks,
+                      const uint64_t* z_masks, double* out, void* stream);
+/* tr(rho P_t) on the row-major vec of an N-qubit density matrix (N <= 31); out = n_terms x (re, im).
+ * Reads the 2^N entries rho[c, c^x] per term; no Hermiticity assumed. */
+int qsim_expect_pauli_dm(const void* vec_rho, int n_qubits, int64_t n_terms, const uint64_t* x_masks,
+                         const uint64_t* z_masks, double* out_re_im, void* stream);
+
 /* ---- batched tiny-circuit executor (replaces the sample loop of
  *      PAPER/randomised_benchmarking.py:65-75) --------------------------------------
  * B independent registers of nq <= 2 qubits kept as density matrices (dim = 2^nq).

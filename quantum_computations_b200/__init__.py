@@ -14,6 +14,7 @@ plus what the hot path needs on a GPU:
     channels        ``Channel`` (Kraus) and the GKP finite-squeezing noise model
     batched         ``BatchedSimulator`` for many small independent circuits
     sharded         state sharded over ranks with global-qubit swaps
+    observables     Pauli-sum expectation values (``PauliSum``, ``expect``) on the GPU
     trajectories    Pauli-trajectory sampling of noisy circuits on kets
     layering        measurement-based layer scheduling           (GKP/circuit.py)
     cliffords       two-qubit Clifford table and Clifford RB    (PAPER/average_clifford_fidelity.py)

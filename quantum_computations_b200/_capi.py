@@ -75,6 +75,9 @@ SIGNATURES = {
     "qsim_reduce_expect": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, c_double_p, C.c_void_p]),
     "qsim_reduce_purity": (C.c_int, [C.c_void_p, C.c_int, c_double_p, C.c_void_p]),
     "qsim_reduce_trace": (C.c_int, [C.c_void_p, C.c_int, c_double_p, C.c_void_p]),
+    "qsim_expect_pauli": (C.c_int, [C.c_void_p, C.c_int, C.c_int64, C.c_void_p, C.c_void_p, c_double_p, C.c_void_p]),
+    "qsim_expect_pauli_dm": (C.c_int, [C.c_void_p, C.c_int, C.c_int64, C.c_void_p, C.c_void_p, c_double_p,
+                                       C.c_void_p]),
     "qsim_rb_batch": (C.c_int, [C.c_int, C.c_int64, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p,
                                 C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "qsim_traj_batch": (C.c_int, [C.c_int, C.c_int64, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64,

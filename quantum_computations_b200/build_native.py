@@ -21,7 +21,7 @@ EMU_DIR = os.path.join(ROOT, "tests", "_build")
 EMU_LIB = os.path.join(EMU_DIR, "libqsim_emu.so")
 
 _HEADERS = ["plan.h", "planner.h", "tile_exec.h", "elem_ops.h"]
-_HOST_SRCS = ["planner.cpp", "capi_host.cpp"]
+_HOST_SRCS = ["planner.cpp", "capi_host.cpp", "pauli.cpp"]
 
 
 def _newer_than(target: str, sources) -> bool:

@@ -13,7 +13,7 @@ extern "C" {
 
 const char* qsim_last_error(void) { return qs::last_error(); }
 
-int qsim_version(void) { return 100; }
+int qsim_version(void) { return 101; }
 
 int qsim_circuit_create(int n_qubits, qsim_circuit_t** out) {
   if (!out) return qs::fail(QSIM_ERR_ARG, "qsim_circuit_create: out is null");

@@ -200,3 +200,94 @@ QS_HD void qs_traj_apply(qs_c128* state, int n, const QsTrajOp& op, const qs_c12
     }
   }
 }
+
+// ---- Pauli-sum expectation values (qsim_expect_pauli, qsim_expect_pauli_dm; plan.h) --------
+QS_HD uint32_t qs_par64(uint64_t v) {
+#if defined(__CUDA_ARCH__)
+  return (uint32_t)__popcll(v) & 1u;
+#else
+  return (uint32_t)__builtin_popcountll(v) & 1u;
+#endif
+}
+
+// In-place Walsh-Hadamard transform: v[s] <- sum_m (-1)^popc(m & s) v[m].
+template <int D>
+QS_HD void qs_walsh(double* v) {
+#pragma unroll
+  for (int h = 0; h < D; ++h)
+#pragma unroll
+    for (int m = 0; m < (1 << D); ++m)
+      if (!((m >> h) & 1)) {
+        const double x = v[m], y = v[m | (1 << h)];
+        v[m] = x + y;
+        v[m | (1 << h)] = x - y;
+      }
+}
+
+// One work item (outer index o) of a Pauli pass: acc[t * stride] += this item's share of term t;
+// wal[k * stride], k < 2^(D+1), is the thread's spectrum scratch (Re, then Im).
+// For a group, b[m] = a[m ^ xl] comes from a conditional swap per generator bit (uniform
+// branches, so a[] and b[] stay in registers for any xl), and w[m] = conj(b[m]) a[m].  Summing
+// over all m visits each pair (u, u ^ xl) from both ends: w[u ^ xl] = conj(w[u]) and the signs
+// differ by (-1)^popc(x & z), so the real parts add up for an even popc(x & z) and the
+// imaginary parts for an odd one -- the part the term takes -- while the other part cancels
+// exactly by never being accumulated.
+template <int D>
+QS_HD void qs_pauli_item(const QsPauliPass& P, const qs_c128* __restrict__ state, uint64_t o, double* acc,
+                         double* wal, uint32_t stride) {
+  uint64_t base = o;
+#pragma unroll
+  for (int i = 0; i < D; ++i) base = qs_insert_bit(base, P.pivot[i], 0);
+  qs_c128 a[1 << D];
+#pragma unroll
+  for (int m = 0; m < (1 << D); ++m) a[m] = state[base ^ P.off[m]];
+  for (uint32_t g = 0; g < P.ngroups; ++g) {
+    const QsPauliGroup G = P.groups[g];
+    const uint32_t t1 = (uint32_t)G.first + G.count;
+    qs_c128 b[1 << D];
+#pragma unroll
+    for (int m = 0; m < (1 << D); ++m) b[m] = a[m];
+#pragma unroll
+    for (int k = 0; k < D; ++k) {
+      if ((G.xl >> k) & 1) {
+#pragma unroll
+        for (int m = 0; m < (1 << D); ++m)
+          if (!((m >> k) & 1)) {
+            const qs_c128 tmp = b[m];
+            b[m] = b[m | (1 << k)];
+            b[m | (1 << k)] = tmp;
+          }
+      }
+    }
+    if (G.parts & 1u) {
+      double w[1 << D];
+#pragma unroll
+      for (int m = 0; m < (1 << D); ++m) w[m] = b[m].x * a[m].x + b[m].y * a[m].y;
+      qs_walsh<D>(w);
+#pragma unroll
+      for (int m = 0; m < (1 << D); ++m) wal[m * stride] = w[m];
+    }
+    if (G.parts & 2u) {
+      double w[1 << D];
+#pragma unroll
+      for (int m = 0; m < (1 << D); ++m) w[m] = b[m].x * a[m].y - b[m].y * a[m].x;
+      qs_walsh<D>(w);
+#pragma unroll
+      for (int m = 0; m < (1 << D); ++m) wal[((1 << D) + m) * stride] = w[m];
+    }
+    for (uint32_t t = G.first; t < t1; ++t) {
+      const uint32_t cls = P.cls[t];
+      const double v = wal[((cls & 1u) << D | P.spec[t]) * stride];
+      const uint32_t neg = qs_par64(base & P.z[t]) ^ (cls >> 1);
+      acc[t * stride] += neg ? -v : v;
+    }
+  }
+}
+
+// Density matrix: entry c of tr(rho X^x Z^z) = sum_c (-1)^popc(c & z) rho[c, c ^ x] (the phase
+// i^popc(x & z) is applied by the host).  rho is the row-major vec of an N-qubit matrix.
+QS_HD qs_c128 qs_pauli_dm_elem(const qs_c128* __restrict__ rho, int N, uint64_t x, uint64_t z, uint64_t c) {
+  qs_c128 v = rho[(c << N) | (c ^ x)];
+  if (qs_par64(c & z)) { v.x = -v.x; v.y = -v.y; }
+  return v;
+}

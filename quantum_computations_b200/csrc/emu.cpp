@@ -338,6 +338,59 @@ int qsim_reduce_trace(const void* rho, int n_qubits, double* out_re_im, void*) {
   return QSIM_OK;
 }
 
+// Pauli expectation values: the same grouping (pauli.cpp) and the same per-thread bodies
+// (elem_ops.h) as the CUDA library; one launch per pass plus the final sum, as there.
+int qsim_expect_pauli(const void* state, int n_qubits, int64_t n_terms, const uint64_t* x_masks,
+                      const uint64_t* z_masks, double* out, void*) {
+  int rc = qs::check_pauli_args("qsim_expect_pauli", n_qubits, n_terms, x_masks, z_masks, out);
+  if (rc != QSIM_OK || n_terms == 0) return rc;
+  if (!state) return qs::fail(QSIM_ERR_ARG, "qsim_expect_pauli: null state");
+  qs::PauliPlan plan;
+  rc = qs::plan_pauli(n_qubits, n_terms, x_masks, z_masks, &plan);
+  if (rc != QSIM_OK) return rc;
+  std::vector<double> sums(2 * (size_t)n_terms, 0.0);
+  const uint64_t count = 1ull << (n_qubits - plan.d);
+  const qs_c128* s = (const qs_c128*)state;
+  for (const QsPauliPass& P : plan.passes) {
+    double acc[QS_PAULI_MAX_TERMS] = {0.0}, wal[2 << QS_PAULI_MAX_D];
+    for (uint64_t o = 0; o < count; ++o) {
+      switch (plan.d) {
+        case 1: qs_pauli_item<1>(P, s, o, acc, wal, 1); break;
+        case 2: qs_pauli_item<2>(P, s, o, acc, wal, 1); break;
+        case 3: qs_pauli_item<3>(P, s, o, acc, wal, 1); break;
+        default: qs_pauli_item<4>(P, s, o, acc, wal, 1); break;
+      }
+    }
+    for (uint32_t t = 0; t < P.nterms; ++t) sums[2 * ((size_t)P.term0 + t)] = acc[t];
+    ++g_launches;
+  }
+  ++g_launches;                              // the final sum
+  qs::pauli_finish(plan, sums.data(), out);
+  return QSIM_OK;
+}
+
+int qsim_expect_pauli_dm(const void* vec_rho, int n_qubits, int64_t n_terms, const uint64_t* x_masks,
+                         const uint64_t* z_masks, double* out_re_im, void*) {
+  int rc = qs::check_pauli_args("qsim_expect_pauli_dm", n_qubits, n_terms, x_masks, z_masks, out_re_im);
+  if (rc != QSIM_OK || n_terms == 0) return rc;
+  if (!vec_rho) return qs::fail(QSIM_ERR_ARG, "qsim_expect_pauli_dm: null state");
+  if (n_qubits > 31) return qs::fail(QSIM_ERR_ARG, "qsim_expect_pauli_dm: n_qubits must be in [1, 31]");
+  std::vector<uint64_t> xi, zi;
+  std::vector<uint8_t> phase;
+  qs::pauli_index_masks(n_qubits, n_terms, x_masks, z_masks, &xi, &zi, &phase);
+  std::vector<double> sums(2 * (size_t)n_terms, 0.0);
+  const qs_c128* rho = (const qs_c128*)vec_rho;
+  for (int64_t t = 0; t < n_terms; ++t)
+    for (uint64_t c = 0; c < (1ull << n_qubits); ++c) {
+      const qs_c128 v = qs_pauli_dm_elem(rho, n_qubits, xi[t], zi[t], c);
+      sums[2 * t] += v.x;
+      sums[2 * t + 1] += v.y;
+    }
+  g_launches += 2;
+  qs::pauli_finish_dm(n_terms, phase, sums.data(), out_re_im);
+  return QSIM_OK;
+}
+
 int qsim_rb_batch(int nq, int64_t n_seq, const uint16_t* opcodes, const int64_t* offsets, int n_opcodes,
                   const double* superops, const double* unitaries, const double* rho0, const double* psi0,
                   double* out_fidelity, double* out_purity, double* out_rho, void*) {

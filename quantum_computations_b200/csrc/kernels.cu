@@ -39,6 +39,13 @@ struct DevCtx {
   double* d_partials = nullptr;   // [kReduceBlocks][2]
   double* d_out = nullptr;        // [2]
   double* h_out = nullptr;        // pinned [2]
+  // scratch of the Pauli expectation values (qsim_expect_pauli / _dm), also under reduce_lock;
+  // allocated at the first such call and grown when a call has more terms than any before
+  double* d_pauli_partials = nullptr;   // [terms][blocks][2]
+  double* d_pauli_sums = nullptr;       // [terms][2]
+  double* h_pauli_sums = nullptr;       // pinned [terms][2]
+  uint64_t* d_pauli_masks = nullptr;    // [terms][2] (density matrices: x, z)
+  size_t pauli_partials_cap = 0, pauli_terms_cap = 0;
   std::mutex occ_lock;
   int occ[12] = {0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0};   // resident CTAs/SM of the k_tile_pass variants at the last smem size
   int occ_smem = -1;
@@ -635,6 +642,130 @@ int reduce_to_host(DevCtx* ctx, F f, uint64_t count, double* out2, cudaStream_t 
 }
 
 // =====================================================================================
+// Pauli-sum expectation values (plan.h, elem_ops.h, pauli.cpp)
+// =====================================================================================
+constexpr int kPauliThreads = 64;         // 32 KiB of accumulators and spectra per CTA (static shared memory)
+constexpr int kPauliBlocksPerSM = 5;       // 195 registers: 5 x 64 threads x 16 loads of 16 B in flight per SM
+constexpr int kPauliDmBlocks = 64;         // per term
+
+// Sum of col[0 .. kPauliThreads-1] in a fixed order (lane 0 of the calling warp holds it).
+__device__ __forceinline__ double pauli_warp_sum(const double* col) {
+  const int lane = threadIdx.x & 31;
+  double s = col[lane];
+#pragma unroll
+  for (int k = 1; k < kPauliThreads / 32; ++k) s += col[lane + 32 * k];
+#pragma unroll
+  for (int off = 16; off > 0; off >>= 1) s += __shfl_down_sync(0xffffffffu, s, off);
+  return s;
+}
+
+// One Pauli pass over a ket: every thread keeps one accumulator per term and its group spectra in
+// shared memory ([entry][thread]: conflict-free), the block writes one partial per term.
+template <int D>
+__global__ void __launch_bounds__(kPauliThreads)
+k_pauli_expect(const qs_c128* __restrict__ state, const __grid_constant__ QsPauliPass P, uint64_t count,
+               double* __restrict__ partials) {
+  __shared__ double acc[QS_PAULI_MAX_TERMS * kPauliThreads];
+  __shared__ double wal[(2 << D) * kPauliThreads];
+  for (uint32_t t = 0; t < P.nterms; ++t) acc[t * kPauliThreads + threadIdx.x] = 0.0;
+  for (uint64_t o = blockIdx.x * (uint64_t)kPauliThreads + threadIdx.x; o < count;
+       o += (uint64_t)gridDim.x * kPauliThreads)
+    qs_pauli_item<D>(P, state, o, acc + threadIdx.x, wal + threadIdx.x, kPauliThreads);
+  __syncthreads();
+  const int warp = threadIdx.x >> 5;
+  for (uint32_t t = warp; t < P.nterms; t += kPauliThreads / 32) {
+    const double s = pauli_warp_sum(acc + t * kPauliThreads);
+    if ((threadIdx.x & 31) == 0) {
+      double* dst = partials + 2 * ((uint64_t)(P.term0 + t) * gridDim.x + blockIdx.x);
+      dst[0] = s;
+      dst[1] = 0.0;
+    }
+  }
+}
+
+// Density matrix: all terms in one launch, blockIdx.y strides over the terms, one thread per
+// (term, c); masks = [term][x, z] in index bits.
+__global__ void __launch_bounds__(kReduceThreads)
+k_pauli_expect_dm(const qs_c128* __restrict__ rho, int N, const uint64_t* __restrict__ masks, int64_t n_terms,
+                  double* __restrict__ partials) {
+  const uint64_t dim = 1ull << N;
+  for (int64_t t = blockIdx.y; t < n_terms; t += gridDim.y) {
+    const uint64_t x = masks[2 * t], z = masks[2 * t + 1];
+    double s0 = 0.0, s1 = 0.0;
+    for (uint64_t c = blockIdx.x * (uint64_t)kReduceThreads + threadIdx.x; c < dim;
+         c += (uint64_t)gridDim.x * kReduceThreads) {
+      const qs_c128 v = qs_pauli_dm_elem(rho, N, x, z, c);
+      s0 += v.x;
+      s1 += v.y;
+    }
+    block_reduce2(s0, s1);
+    if (threadIdx.x == 0) {
+      double* dst = partials + 2 * ((uint64_t)t * gridDim.x + blockIdx.x);
+      dst[0] = s0;
+      dst[1] = s1;
+    }
+    __syncthreads();                       // block_reduce2's shared words are reused next term
+  }
+}
+
+// sums[t] = partials[t][0] + ... + partials[t][nblocks - 1], fixed tree: bit-reproducible.
+__global__ void __launch_bounds__(kReduceThreads)
+k_pauli_final(const double* __restrict__ partials, int nblocks, int64_t n_terms, double* __restrict__ sums) {
+  for (int64_t t = blockIdx.x; t < n_terms; t += gridDim.x) {
+    const double* row = partials + 2 * (uint64_t)t * nblocks;
+    double s0 = 0.0, s1 = 0.0;
+    for (int i = threadIdx.x; i < nblocks; i += blockDim.x) { s0 += row[2 * i]; s1 += row[2 * i + 1]; }
+    block_reduce2(s0, s1);
+    if (threadIdx.x == 0) { sums[2 * t] = s0; sums[2 * t + 1] = s1; }
+    __syncthreads();
+  }
+}
+
+// Grows the per-device Pauli scratch (caller holds reduce_lock).  Growing frees the old
+// buffers, which waits for the device: it happens only when a call has more terms than any before.
+int pauli_scratch(DevCtx* ctx, size_t terms, size_t blocks) {
+  const size_t partials = terms * blocks * 2;
+  if (partials > ctx->pauli_partials_cap) {
+    if (ctx->d_pauli_partials) QS_CUDA(cudaFree(ctx->d_pauli_partials));
+    ctx->d_pauli_partials = nullptr;
+    ctx->pauli_partials_cap = 0;
+    QS_CUDA(cudaMalloc(&ctx->d_pauli_partials, sizeof(double) * partials));
+    ctx->pauli_partials_cap = partials;
+  }
+  if (terms > ctx->pauli_terms_cap) {
+    if (ctx->d_pauli_sums) QS_CUDA(cudaFree(ctx->d_pauli_sums));
+    if (ctx->h_pauli_sums) QS_CUDA(cudaFreeHost(ctx->h_pauli_sums));
+    if (ctx->d_pauli_masks) QS_CUDA(cudaFree(ctx->d_pauli_masks));
+    ctx->d_pauli_sums = ctx->h_pauli_sums = nullptr;
+    ctx->d_pauli_masks = nullptr;
+    ctx->pauli_terms_cap = 0;
+    QS_CUDA(cudaMalloc(&ctx->d_pauli_sums, sizeof(double) * 2 * terms));
+    QS_CUDA(cudaMallocHost(&ctx->h_pauli_sums, sizeof(double) * 2 * terms));
+    QS_CUDA(cudaMalloc(&ctx->d_pauli_masks, sizeof(uint64_t) * 2 * terms));
+    ctx->pauli_terms_cap = terms;
+  }
+  return QSIM_OK;
+}
+
+// Final sum of a call's partials and the one download; synchronises the stream.
+int pauli_sums_to_host(DevCtx* ctx, int64_t n_terms, int nblocks, cudaStream_t stream) {
+  const unsigned grid = (unsigned)std::min<int64_t>(n_terms, 65535);
+  k_pauli_final<<<grid, kReduceThreads, 0, stream>>>(ctx->d_pauli_partials, nblocks, n_terms, ctx->d_pauli_sums);
+  g_launches.fetch_add(1, std::memory_order_relaxed);
+  QS_CUDA(cudaGetLastError());
+  QS_CUDA(cudaMemcpyAsync(ctx->h_pauli_sums, ctx->d_pauli_sums, sizeof(double) * 2 * n_terms, cudaMemcpyDeviceToHost,
+                          stream));
+  QS_CUDA(cudaStreamSynchronize(stream));
+  return QSIM_OK;
+}
+
+template <int D>
+void launch_pauli_pass(const QsPauliPass& P, const qs_c128* state, uint64_t count, unsigned blocks, double* partials,
+                       cudaStream_t stream) {
+  k_pauli_expect<D><<<blocks, kPauliThreads, 0, stream>>>(state, P, count, partials);
+}
+
+// =====================================================================================
 // Batched tiny-circuit executor
 // =====================================================================================
 template <int DIM>
@@ -1169,6 +1300,79 @@ int qsim_reduce_trace(const void* rho, int n_qubits, double* out_re_im, void* st
   if (rc != QSIM_OK) return rc;
   FnTrace f{(const qs_c128*)rho, n_qubits};
   return reduce_to_host(ctx, f, 1ull << n_qubits, out_re_im, (cudaStream_t)stream);
+}
+
+int qsim_expect_pauli(const void* state, int n_qubits, int64_t n_terms, const uint64_t* x_masks,
+                      const uint64_t* z_masks, double* out, void* stream) {
+  int rc = qs::check_pauli_args("qsim_expect_pauli", n_qubits, n_terms, x_masks, z_masks, out);
+  if (rc != QSIM_OK || n_terms == 0) return rc;
+  if (!state) return qs::fail(QSIM_ERR_ARG, "qsim_expect_pauli: null state");
+  qs::PauliPlan plan;
+  try {
+    rc = qs::plan_pauli(n_qubits, n_terms, x_masks, z_masks, &plan);
+  } catch (const std::bad_alloc&) {
+    rc = qs::fail(QSIM_ERR_NOMEM, "out of host memory while grouping the Pauli terms");
+  }
+  if (rc != QSIM_OK) return rc;
+  Bound bound;
+  rc = bind_device(state, &bound);
+  DevCtx* ctx = bound.ctx;
+  if (rc != QSIM_OK) return rc;
+  const uint64_t count = 1ull << (n_qubits - plan.d);
+  uint64_t blocks = (count + kPauliThreads - 1) / kPauliThreads;
+  blocks = std::min<uint64_t>(blocks, (uint64_t)ctx->sms * kPauliBlocksPerSM);
+  const cudaStream_t st = (cudaStream_t)stream;
+  std::lock_guard<std::mutex> guard(ctx->reduce_lock);
+  rc = pauli_scratch(ctx, (size_t)n_terms, (size_t)blocks);
+  if (rc != QSIM_OK) return rc;
+  const qs_c128* s = (const qs_c128*)state;
+  for (const QsPauliPass& P : plan.passes) {
+    switch (plan.d) {
+      case 1: launch_pauli_pass<1>(P, s, count, (unsigned)blocks, ctx->d_pauli_partials, st); break;
+      case 2: launch_pauli_pass<2>(P, s, count, (unsigned)blocks, ctx->d_pauli_partials, st); break;
+      case 3: launch_pauli_pass<3>(P, s, count, (unsigned)blocks, ctx->d_pauli_partials, st); break;
+      default: launch_pauli_pass<4>(P, s, count, (unsigned)blocks, ctx->d_pauli_partials, st); break;
+    }
+    g_launches.fetch_add(1, std::memory_order_relaxed);
+    QS_CUDA(cudaGetLastError());
+  }
+  rc = pauli_sums_to_host(ctx, n_terms, (int)blocks, st);
+  if (rc != QSIM_OK) return rc;
+  qs::pauli_finish(plan, ctx->h_pauli_sums, out);
+  return QSIM_OK;
+}
+
+int qsim_expect_pauli_dm(const void* vec_rho, int n_qubits, int64_t n_terms, const uint64_t* x_masks,
+                         const uint64_t* z_masks, double* out_re_im, void* stream) {
+  int rc = qs::check_pauli_args("qsim_expect_pauli_dm", n_qubits, n_terms, x_masks, z_masks, out_re_im);
+  if (rc != QSIM_OK || n_terms == 0) return rc;
+  if (!vec_rho) return qs::fail(QSIM_ERR_ARG, "qsim_expect_pauli_dm: null state");
+  if (n_qubits > 31) return qs::fail(QSIM_ERR_ARG, "qsim_expect_pauli_dm: n_qubits must be in [1, 31]");
+  std::vector<uint64_t> xi, zi;
+  std::vector<uint8_t> phase;
+  qs::pauli_index_masks(n_qubits, n_terms, x_masks, z_masks, &xi, &zi, &phase);
+  std::vector<uint64_t> masks(2 * (size_t)n_terms);
+  for (int64_t t = 0; t < n_terms; ++t) { masks[2 * t] = xi[t]; masks[2 * t + 1] = zi[t]; }
+  Bound bound;
+  rc = bind_device(vec_rho, &bound);
+  DevCtx* ctx = bound.ctx;
+  if (rc != QSIM_OK) return rc;
+  const uint64_t dim = 1ull << n_qubits;
+  const unsigned bx = (unsigned)std::min<uint64_t>((dim + kReduceThreads - 1) / kReduceThreads, kPauliDmBlocks);
+  const unsigned by = (unsigned)std::min<int64_t>(n_terms, 65535);
+  const cudaStream_t st = (cudaStream_t)stream;
+  std::lock_guard<std::mutex> guard(ctx->reduce_lock);
+  rc = pauli_scratch(ctx, (size_t)n_terms, (size_t)bx);
+  if (rc != QSIM_OK) return rc;
+  QS_CUDA(cudaMemcpyAsync(ctx->d_pauli_masks, masks.data(), sizeof(uint64_t) * masks.size(), cudaMemcpyHostToDevice, st));
+  k_pauli_expect_dm<<<dim3(bx, by), kReduceThreads, 0, st>>>((const qs_c128*)vec_rho, n_qubits, ctx->d_pauli_masks,
+                                                            n_terms, ctx->d_pauli_partials);
+  g_launches.fetch_add(1, std::memory_order_relaxed);
+  QS_CUDA(cudaGetLastError());
+  rc = pauli_sums_to_host(ctx, n_terms, (int)bx, st);
+  if (rc != QSIM_OK) return rc;
+  qs::pauli_finish_dm(n_terms, phase, ctx->h_pauli_sums, out_re_im);
+  return QSIM_OK;
 }
 
 int qsim_rb_batch(int nq, int64_t n_seq, const uint16_t* opcodes, const int64_t* offsets, int n_opcodes,

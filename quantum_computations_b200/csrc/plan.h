@@ -184,3 +184,37 @@ struct QsTmaGeom {
   int32_t shift[5];
   uint32_t mask[5];
 };
+
+// ---- Pauli-sum expectation values on a ket (qsim_expect_pauli) ---------------------------
+// A Pauli string is a pair of index-bit masks (x, z): P = i^popc(x & z) X^x Z^z, Z first.
+// One *Pauli pass* streams the state once, read only.  Every thread owns the 2^d amplitudes
+// base ^ off[m], m < 2^d, where off[m] is the XOR of the pass's generators v_i selected by the
+// bits of m; base runs over the indices whose pivot bits (one per generator, chosen so that
+// the generators restricted to them are invertible) are zero.  Every term whose x lies in the
+// span of the generators -- x = off[xl] -- pairs amplitude m with m ^ xl inside the thread's
+// registers.  Terms are grouped by xl; a group forms w[m] = conj(a[m ^ xl]) a[m] once.  A term
+// takes the real part of w (even popc(x & z)) or the imaginary part (odd) with the sign
+// (-1)^popc((base ^ off[m]) & z) = (outer parity) x (-1)^popc(m & s), where bit i of s is
+// parity(generator_i & z): the inner sign is a Walsh function of m.  So a group transforms
+// Re w and Im w once (Walsh-Hadamard, D x 2^D additions each) and every term reads ONE entry
+// of the spectrum.  The x = 0 group (Z strings) is the case xl = 0: w[m] = |a[m]|^2.
+#define QS_PAULI_MAX_D 4
+#define QS_PAULI_MAX_TERMS 32          // accumulators per thread, i.e. terms per pass
+
+struct QsPauliGroup {
+  uint8_t xl;                    // x of the group in generator coordinates (0: Z strings)
+  uint8_t first, count;          // its terms: [first, first + count) of the pass
+  uint8_t parts;                 // bit 0: a term takes Re w, bit 1: a term takes Im w
+};
+
+struct QsPauliPass {
+  uint32_t d;                    // generators = log2 amplitudes per thread
+  uint32_t ngroups, nterms;
+  uint32_t term0;                // row of the pass's first term in the call's partials
+  uint8_t  pivot[QS_PAULI_MAX_D];            // ascending index bits that are zero in every base
+  uint64_t off[1 << QS_PAULI_MAX_D];         // XOR of the generators selected by m
+  QsPauliGroup groups[1 << QS_PAULI_MAX_D];
+  uint64_t z[QS_PAULI_MAX_TERMS];            // index-bit Z mask of each term
+  uint8_t  spec[QS_PAULI_MAX_TERMS];         // s: bit i = parity(generator_i & z)
+  uint8_t  cls[QS_PAULI_MAX_TERMS];          // bit 0: imaginary part of w; bit 1: negated
+};

@@ -90,4 +90,26 @@ int build_plan(int n, const std::vector<Op>& ops, const qsim_plan_options_t& opt
 
 qsim_plan_options_t resolve_options(const qsim_plan_options_t* opt);
 
+// ---- Pauli-sum expectation values (pauli.cpp; descriptors in plan.h) ----------------------
+// Checks of qsim_expect_pauli / _dm: n in [1, 63], masks below 2^n (n_terms == 0 passes).
+int check_pauli_args(const char* who, int n, int64_t n_terms, const uint64_t* x_masks, const uint64_t* z_masks,
+                     const void* out);
+// Reference-qubit masks -> index-bit masks, and popc(x & z) mod 4 of every term.
+void pauli_index_masks(int n, int64_t n_terms, const uint64_t* x_masks, const uint64_t* z_masks,
+                       std::vector<uint64_t>* xi, std::vector<uint64_t>* zi, std::vector<uint8_t>* phase);
+
+// The passes of one call.  Slot s (pass by pass, term by term) holds caller term order[s].
+struct PauliPlan {
+  int d = 0;                                 // generators per pass: min(n, QS_PAULI_MAX_D)
+  std::vector<QsPauliPass> passes;
+  std::vector<int64_t> order;
+};
+// Greedy grouping by X mask: at most one pass per chunk of <= QS_PAULI_MAX_TERMS terms of one
+// non-zero X mask, the Z strings in passes with room (a pass of their own only if none has).
+int plan_pauli(int n, int64_t n_terms, const uint64_t* x_masks, const uint64_t* z_masks, PauliPlan* out);
+// sums: 2 doubles per slot (re, im) -> out[caller term] (real).
+void pauli_finish(const PauliPlan& plan, const double* sums, double* out);
+// sums: 2 doubles per term, times i^phase -> out_re_im.
+void pauli_finish_dm(int64_t n_terms, const std::vector<uint8_t>& phase, const double* sums, double* out_re_im);
+
 }  // namespace qs

@@ -415,6 +415,25 @@ class DeviceState:
                            ket.n_bits)
         return complex(out[0], out[1])
 
+    def expect_pauli(self, x_masks, z_masks) -> np.ndarray:
+        """Expectation values of the Pauli strings ``(x_masks[t], z_masks[t])`` (bit q =
+        reference qubit q, operator i^popc(x & z) X^x Z^z): <P_t> as float64 for a ket,
+        tr(rho P_t) as complex128 for a density matrix (``observables`` builds the masks)."""
+        x = np.ascontiguousarray(x_masks, dtype=np.uint64).reshape(-1)
+        z = np.ascontiguousarray(z_masks, dtype=np.uint64).reshape(-1)
+        if x.shape != z.shape:
+            raise ValueError("x_masks and z_masks must have the same length")
+        lib, be = self.backend.lib, self.backend
+        if self.ndim == 1:
+            out = np.zeros(len(x), dtype=np.float64)
+            _capi.check(lib, lib.qsim_expect_pauli(be.ptr(self.buf), self.n_bits, len(x), x.ctypes.data,
+                                                   z.ctypes.data, _dptr(out), be.stream()))
+            return out
+        out = np.zeros(len(x), dtype=np.complex128)
+        _capi.check(lib, lib.qsim_expect_pauli_dm(be.ptr(self.buf), self.n_bits // 2, len(x), x.ctypes.data,
+                                                  z.ctypes.data, _dptr(out.view(np.float64)), be.stream()))
+        return out
+
 
 def _to_device(x, backend) -> DeviceState:
     return x if isinstance(x, DeviceState) else DeviceState.from_numpy(x, backend)

@@ -252,6 +252,20 @@ def is_hermitian(oper):
 
 
 def expect(oper, state):
+    """<state| oper |state>.  A ``observables.PauliSum`` operator is evaluated on the GPU for a
+    device ket or density matrix, a sharded ket or a host array; a dense operator with a device
+    ket reduces on the GPU too (n <= 20)."""
+    if getattr(oper, "_qsim_pauli_sum", False):
+        from .observables import expect as pauli_expect
+        return pauli_expect(oper, state)
+    if _is_device(state):
+        if state.ndim != 1:
+            raise TypeError("incompatible operator and state vector")
+        from .engine import DeviceState
+        oper = np.asarray(oper)
+        if not (is_qubit_operator(oper) and oper.shape[0] == 1 << state.n_bits):
+            raise TypeError("incompatible operator and state vector")
+        return DeviceState.from_numpy(oper, state.backend).expect_ket(state)
     compatible = is_qubit_operator(oper) and is_qubit_state(state) and oper.shape[0] == state.shape[0]
     if not compatible:
         raise TypeError("incompatible operator and state vector")

@@ -1,0 +1,141 @@
+"""Expectation values of Pauli sums on device states.
+
+The reference evaluates observables only as dense 2^N x 2^N host matrices
+(``numpy_quantum.expect``, DV/numpy_quantum.py:254-264), which stops at a dozen
+qubits.  Here an observable is a sum of Pauli strings, and every string is
+evaluated on the GPU in a read-only pass over the state (``qsim_expect_pauli``):
+strings are grouped by their X/Y support, so one read of the state serves up to
+32 strings whose X masks span at most four dimensions, and an all-Z observable
+costs a single read.  Density matrices (``qsim_expect_pauli_dm``) and sharded
+kets (``sharded.ShardedState.expect_pauli``) take the same masks.
+
+Convention: a string is a pair of masks ``(x, z)`` with bit q for reference
+qubit q; I = (0, 0), X = (1, 0), Z = (0, 1), Y = (1, 1), and the operator is
+``i^popc(x & z) X^x Z^z`` (Z first), so every string is Hermitian.
+"""
+from __future__ import annotations
+
+import numpy as np
+
+from . import numpy_quantum as npq
+from .numpy_quantum import PauliError
+
+_LETTER = "IXYZ"
+_NUMBER = {(0, 0): 0, (1, 0): 1, (1, 1): 2, (0, 1): 3}      # (x bit, z bit) -> Pauli number
+_SINGLE = {0: np.eye(2, dtype=np.complex128), 1: npq.X.astype(np.complex128),
+           2: npq.Y.astype(np.complex128), 3: npq.Z.astype(np.complex128)}
+
+
+class PauliSum:
+    """sum_t c_t P_t over Pauli strings P_t.
+
+    ``terms`` is an iterable of ``(coeff, paulis)``; ``paulis`` is either a string with
+    one letter per qubit, qubit 0 first (``"XIZ"``, as in ``npq.tensor``), or a dict
+    ``{qubit: identifier}`` with anything ``npq.get_pauli_number`` accepts.  A negated
+    identifier ("-x", -3, [0, 0, -1]) folds its sign into the coefficient.  Identical
+    strings are merged (first appearance keeps its place)."""
+
+    _qsim_pauli_sum = True
+
+    def __init__(self, terms):
+        index = {}
+        xs, zs, coeffs = [], [], []
+        nq = 0
+        for item in terms:
+            try:
+                coeff, paulis = item
+            except (TypeError, ValueError):
+                raise PauliError(f"a term must be a pair (coeff, paulis), got {item!r}") from None
+            if isinstance(paulis, str):
+                factors = {q: npq.get_pauli_number(ch) for q, ch in enumerate(paulis)}
+                width = len(paulis)
+            elif isinstance(paulis, dict):
+                factors = {}
+                for q, ident in paulis.items():
+                    if not isinstance(q, (int, np.integer)) or q < 0:
+                        raise PauliError(f"qubit {q!r} is not a non-negative integer")
+                    factors[int(q)] = npq.get_pauli_number(ident)
+                width = max(factors) + 1 if factors else 0
+            else:
+                raise PauliError(f"{paulis!r} is neither a Pauli string nor a {{qubit: Pauli}} dict")
+            c = complex(coeff)
+            x = z = 0
+            for q, number in factors.items():
+                if number < 0:
+                    c, number = -c, -number
+                if number in (1, 2):
+                    x |= 1 << q
+                if number in (2, 3):
+                    z |= 1 << q
+            nq = max(nq, width)
+            key = (x, z)
+            if key in index:
+                coeffs[index[key]] += c
+            else:
+                index[key] = len(xs)
+                xs.append(x)
+                zs.append(z)
+                coeffs.append(c)
+        if nq > 63:
+            raise PauliError("Pauli strings on more than 63 qubits are not supported")
+        self.x_masks = np.array(xs, dtype=np.uint64)
+        self.z_masks = np.array(zs, dtype=np.uint64)
+        self.coeffs = np.array(coeffs, dtype=np.complex128)
+        self.num_qubits = nq
+
+    def __len__(self) -> int:
+        return len(self.coeffs)
+
+    def _letters(self, t: int, n: int):
+        """Pauli numbers (0 = I, 1..3 = X, Y, Z) of term t on qubits 0 .. n-1."""
+        x, z = int(self.x_masks[t]), int(self.z_masks[t])
+        return [_NUMBER[((x >> q) & 1, (z >> q) & 1)] for q in range(n)]
+
+    def __repr__(self) -> str:
+        body = ", ".join(f"({c!r}, {''.join(_LETTER[p] for p in self._letters(t, self.num_qubits))!r})"
+                         for t, c in enumerate(self.coeffs))
+        return f"PauliSum([{body}])"
+
+    def matrix(self, n: int | None = None) -> np.ndarray:
+        """Dense 2^n x 2^n host matrix (qubit 0 is the first Kronecker factor); small n only."""
+        n = self.num_qubits if n is None else int(n)
+        if n < self.num_qubits:
+            raise ValueError(f"the observable acts on {self.num_qubits} qubits, more than n = {n}")
+        out = np.zeros((1 << n, 1 << n), dtype=np.complex128)
+        for t, c in enumerate(self.coeffs):
+            out += c * npq.tensor(*[_SINGLE[p] for p in self._letters(t, n)])
+        return out
+
+
+def _sharded_type():
+    try:
+        from .sharded import ShardedState
+    except ImportError:                      # pragma: no cover - sharded needs nothing optional
+        return ()
+    return ShardedState
+
+
+def expect(observable: PauliSum, state, *, per_term: bool = False):
+    """sum_t c_t <P_t> as a Python complex, or with ``per_term`` the array of <P_t>
+    (real for kets, complex tr(rho P_t) for density matrices).
+
+    ``state``: an ``engine.DeviceState`` (ket or density matrix), a
+    ``sharded.ShardedState`` (collective: every rank calls it and gets the same result) or
+    a host ndarray, which is uploaded to the default CUDA backend first -- there is no
+    CPU path."""
+    if not isinstance(observable, PauliSum):
+        raise TypeError("expect needs a PauliSum observable")
+    from . import engine
+    sharded_type = _sharded_type()
+    if isinstance(state, sharded_type):
+        values = state.expect_pauli(observable.x_masks, observable.z_masks)
+    else:
+        if not isinstance(state, engine.DeviceState):
+            state = engine.DeviceState.from_numpy(np.asarray(state))
+        if observable.num_qubits > state.num_qubits:
+            raise ValueError(f"the observable acts on {observable.num_qubits} qubits, "
+                             f"the state has {state.num_qubits}")
+        values = state.expect_pauli(observable.x_masks, observable.z_masks)
+    if per_term:
+        return values
+    return complex(np.dot(observable.coeffs, values))

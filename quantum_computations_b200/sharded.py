@@ -106,6 +106,7 @@ class ShardedState:
         self._peer = None
         self._p2p = None                          # peers' shards mapped through CUDA IPC (fused exchange)
         self._swap_events = []                    # CUDA event pairs of the fused exchanges (timed lazily)
+        self.is_density = False                   # set by ShardedSimulator(density=True): vec(rho), 2N bits
         # how to view a backend buffer as a torch tensor for the communicator
         self._as_torch = as_torch or (lambda b: b)
 
@@ -159,6 +160,102 @@ class ShardedState:
     def fidelity(self, other: "ShardedState") -> float:
         """|<self|other>|^2 (npq.fidelity, ket-ket branch, DV/numpy_quantum.py:148-161)."""
         return abs(self.inner(other)) ** 2
+
+    # -- observables ---------------------------------------------------------------------------
+    def expect_pauli(self, x_masks, z_masks) -> np.ndarray:
+        """<P_t> of Pauli strings (bit q of the masks = reference qubit q, operator
+        i^popc(x & z) X^x Z^z) as a float64 array; a collective, identical on every rank.
+
+        Z factors on rank qubits become a per-rank sign (the logical value, flip flags
+        included).  X/Y factors must be local: rank qubits in an X support are first traded,
+        in one exchange, against local qubits outside every X support still to evaluate
+        (a string whose X/Y support does not fit in a shard is refused).  Every rank evaluates
+        its shard with ``qsim_expect_pauli`` and the per-term vector is all-reduced once.  The
+        logical state is unchanged; the layout may differ afterwards (``phys`` / ``flip``
+        record it, so ``gather_numpy`` and later schedules see the same state)."""
+        if self.is_density:
+            raise NotImplementedError("Pauli expectation values of a sharded density matrix are not implemented")
+        x = np.ascontiguousarray(x_masks, dtype=np.uint64).reshape(-1)
+        z = np.ascontiguousarray(z_masks, dtype=np.uint64).reshape(-1)
+        if x.shape != z.shape:
+            raise ValueError("x_masks and z_masks must have the same length")
+        n = self.n
+        if len(x) and (int(x.max()) >> n or int(z.max()) >> n):
+            raise ValueError("a Pauli mask has a bit at or above the number of qubits")
+        # logical bit l = n-1-q of reference qubit q
+        xs = [{n - 1 - q for q in range(n) if int(v) >> q & 1} for v in x]
+        zs = [{n - 1 - q for q in range(n) if int(v) >> q & 1} for v in z]
+        values = np.zeros(len(x), dtype=np.float64)
+        remaining = list(range(len(x)))
+        while remaining:
+            is_local = lambda bits: all(self.phys[l] < self.n_local for l in bits)   # noqa: E731
+            chosen = [t for t in remaining if is_local(xs[t])]
+            support = set().union(*[xs[t] for t in chosen])
+            for t in remaining:
+                if t in chosen:
+                    continue
+                wider = support | xs[t]
+                need = [l for l in wider if self.phys[l] >= self.n_local]
+                free = [l for l in range(n) if self.phys[l] < self.n_local and l not in wider]
+                if len(need) <= len(free):
+                    chosen.append(t)
+                    support = wider
+            if not chosen:
+                raise NotImplementedError("a Pauli string's X/Y support is wider than a shard; use fewer ranks")
+            self._localise(support)
+            self._expect_local(sorted(chosen), x, xs, zs, values)
+            done = set(chosen)
+            remaining = [t for t in remaining if t not in done]
+        return self.comm.allreduce_sum(values)
+
+    def expect(self, observable, per_term: bool = False):
+        """``observables.expect`` on this sharded ket (collective)."""
+        from .observables import expect
+        return expect(observable, self, per_term=per_term)
+
+    def _localise(self, support) -> None:
+        """Make the logical bits in ``support`` local with one exchange against the highest
+        local bits outside it.  A bit that arrives complemented (its rank bit carried the flip
+        flag) is put right with an X on the shard, and the flag is cleared, so that the layout
+        tables describe the same logical state as before."""
+        need = sorted((l for l in support if self.phys[l] >= self.n_local), key=lambda l: self.phys[l])
+        if not need:
+            return
+        free = sorted((l for l in range(self.n) if self.phys[l] < self.n_local and l not in support),
+                      key=lambda l: -self.phys[l])
+        pairs = [(self.phys[a], self.phys[b]) for a, b in zip(need, free)]
+        complemented = []
+        for gp, lp in pairs:
+            i = gp - self.n_local
+            if self.flip[i]:
+                complemented.append(lp)            # the arriving bit lands on physical bit lp
+                self.flip[i] = 0
+        self.exchange(pairs)
+        if complemented:
+            x_gate = np.array([[0, 1], [1, 0]], dtype=np.complex128)
+            ops = [([self.n_local - 1 - lp], x_gate) for lp in complemented]
+            engine.Plan(self.backend, self.n_local, ops).execute(self.buf)
+
+    def _expect_local(self, terms, x, xs, zs, values) -> None:
+        """values[t] += this rank's share of <P_t> for terms whose X support is local."""
+        nl = self.n_local
+        lx = np.zeros(len(terms), dtype=np.uint64)
+        lz = np.zeros(len(terms), dtype=np.uint64)
+        sign = np.ones(len(terms))
+        for k, t in enumerate(terms):
+            for l in xs[t]:
+                lx[k] |= np.uint64(1 << (nl - 1 - self.phys[l]))         # shard reference qubit
+            for l in zs[t]:
+                p = self.phys[l]
+                if p < nl:
+                    lz[k] |= np.uint64(1 << (nl - 1 - p))
+                elif self.rank_value(p):
+                    sign[k] = -sign[k]
+        be = self.backend
+        out = np.zeros(len(terms), dtype=np.float64)
+        _capi.check(be.lib, be.lib.qsim_expect_pauli(be.ptr(self.buf), nl, len(terms), lx.ctypes.data, lz.ctypes.data,
+                                                     out.ctypes.data_as(_capi.c_double_p), be.stream()))
+        values[terms] += sign * out
 
     # -- swaps -----------------------------------------------------------------------------------
     import os as _os
@@ -559,6 +656,8 @@ class ShardedSimulator:
         self.density = bool(density)
         if self.density and state.n % 2:
             raise ValueError("a vectorised density matrix has an even number of index bits")
+        if self.density:
+            state.is_density = True
         self.stats = {"segments": 0, "passes": 0, "swaps": 0, "local_gates": 0, "exchange_units": 0.0,
                       "relabels": 0, "carried_common": 0, "carried_signs": 0, "carried_controlled": 0}
         self._schedule = None

@@ -20,7 +20,7 @@ CUDA_LIB = os.path.join(CSRC, "libqsim_b200.so")
 EMU_DIR = os.path.join(ROOT, "tests", "_build")
 EMU_LIB = os.path.join(EMU_DIR, "libqsim_emu.so")
 
-_HEADERS = ["plan.h", "planner.h", "tile_exec.h", "elem_ops.h"]
+_HEADERS = ["plan.h", "planner.h", "tile_exec.h", "elem_ops.h", "backend.h"]
 _HOST_SRCS = ["planner.cpp", "capi_host.cpp", "pauli.cpp"]
 
 

@@ -1,10 +1,12 @@
 // HOST EMULATOR -- TEST INFRASTRUCTURE ONLY.
 //
 // Builds (g++ only, no CUDA) into tests/_build/libqsim_emu.so and exports the
-// same C ABI as libqsim_b200.so, but on HOST pointers.  It runs the very same
-// planner (planner.cpp / capi_host.cpp) and the very same per-thread phase
-// functions (tile_exec.h, elem_ops.h) as the GPU kernels, looping over thread
-// ids where the GPU runs them in parallel.  The CPU test-suite uses it to check
+// same C ABI as libqsim_b200.so, but on HOST pointers.  It links the very same
+// C ABI layer (capi_host.cpp: argument checks, qubit conversion, host lowering),
+// planner (planner.cpp, pauli.cpp) and per-thread phase functions (tile_exec.h,
+// elem_ops.h) as the CUDA library; this file holds only the backend (backend.h),
+// which loops over thread ids where the GPU runs them in parallel, and the
+// functions that have no host equivalent.  The CPU test-suite uses it to check
 // the plan logic and the index arithmetic without a GPU.  The product package
 // never loads it: quantum_computations_b200.engine binds libqsim_b200.so only
 // and raises when that library or a CUDA device is missing.
@@ -12,12 +14,9 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
-#include <string>
-#include <utility>
 #include <vector>
 
-#include "elem_ops.h"
-#include "planner.h"
+#include "backend.h"
 
 namespace {
 
@@ -117,18 +116,24 @@ int emu_generic(const qs::Op& op, qs_c128* state, int n) {
   return QSIM_OK;
 }
 
-int execute_plan(const qsim_plan* p, void* state, int n, void* scratch) {
-  if (!p || !state) return qs::fail(QSIM_ERR_ARG, "qsim_plan_execute: null argument");
+}  // namespace
+
+// =====================================================================================
+// Backend of the compute entry points (backend.h; checks and lowering in capi_host.cpp):
+// the per-thread bodies of the CUDA kernels, looped over the work items
+// =====================================================================================
+namespace qs::dev {
+
+int execute_plan(const qsim_plan& p, qs_c128* state, int n, void*) {
   if (g_ownership_violations)
     return qs::fail(QSIM_ERR_UNSUPPORTED, "emulator: a warp-synchronised step reads another warp's amplitudes");
-  if (n != p->n) return qs::fail(QSIM_ERR_ARG, "qsim_plan_execute: plan was compiled for a different qubit count");
-  for (const qs::PlanItem& it : p->items) {
+  for (const qs::PlanItem& it : p.items) {
     if (it.generic) {
-      int rc = emu_generic(it.op, (qs_c128*)state, n);
+      int rc = emu_generic(it.op, state, n);
       if (rc != QSIM_OK) return rc;
     } else {
       if ((int)it.pass.T > n) return qs::fail(QSIM_ERR_ARG, "pass tile larger than the state");
-      emu_pass(it.pass, (qs_c128*)state, n);
+      emu_pass(it.pass, state, n);
       if (g_ownership_violations)
         return qs::fail(QSIM_ERR_UNSUPPORTED, "emulator: a warp-synchronised step reads another warp's amplitudes");
     }
@@ -136,20 +141,194 @@ int execute_plan(const qsim_plan* p, void* state, int n, void* scratch) {
   return QSIM_OK;
 }
 
-int one_gate(void* state, int n, const int* targets, int k, const double* matrix, void* scratch) {
-  qsim_circuit_t* c = nullptr;
-  int rc = qsim_circuit_create(n, &c);
-  if (rc != QSIM_OK) return rc;
-  rc = qsim_circuit_add_matrix(c, k, targets, matrix);
-  qsim_plan_t* p = nullptr;
-  if (rc == QSIM_OK) rc = qsim_plan_compile(c, nullptr, &p);
-  if (rc == QSIM_OK) rc = execute_plan(p, state, n, scratch);
-  qsim_plan_destroy(p);
-  qsim_circuit_destroy(c);
-  return rc;
+int init_product(qs_c128* state, int n, const ProductAmps& amps, void*) {
+  for (uint64_t i = 0; i < (1ull << n); ++i) state[i] = qs_product_amp(amps.a, n, i);
+  ++g_launches;
+  return QSIM_OK;
 }
 
-}  // namespace
+int measure_probs(const qs_c128* state, int pos, uint64_t pairs, const BraPair& bra0, const BraPair& bra1,
+                  double* out_norm2, void*) {
+  double p0 = 0.0, p1 = 0.0;
+  for (uint64_t r = 0; r < pairs; ++r) {
+    const qs_c128 u = qs_contract(state, pos, r, bra0.b), v = qs_contract(state, pos, r, bra1.b);
+    p0 += u.x * u.x + u.y * u.y;
+    p1 += v.x * v.x + v.y * v.y;
+  }
+  out_norm2[0] = p0;
+  out_norm2[1] = p1;
+  g_launches += 2;
+  return QSIM_OK;
+}
+
+int collapse(const qs_c128* in, qs_c128* out, int pos, const BraPair& bra, double norm, uint64_t count, void*) {
+  for (uint64_t r = 0; r < count; ++r) {
+    qs_c128 v = qs_contract(in, pos, r, bra.b);
+    v.x /= norm; v.y /= norm;
+    out[r] = v;
+  }
+  ++g_launches;
+  return QSIM_OK;
+}
+
+int insert(const qs_c128* in, qs_c128* out, int pos, const BraPair& amp, uint64_t count, void*) {
+  for (uint64_t i = 0; i < count; ++i) out[i] = qs_insert_amp(in, pos, i, amp.b);
+  ++g_launches;
+  return QSIM_OK;
+}
+
+int reduce_norm2(const qs_c128* s, uint64_t n_amps, double* out, void*) {
+  double acc = 0.0;
+  for (uint64_t i = 0; i < n_amps; ++i) acc += s[i].x * s[i].x + s[i].y * s[i].y;
+  *out = acc;
+  g_launches += 2;
+  return QSIM_OK;
+}
+
+int reduce_inner(const qs_c128* u, const qs_c128* v, uint64_t n_amps, double* out_re_im, void*) {
+  double re = 0.0, im = 0.0;
+  for (uint64_t i = 0; i < n_amps; ++i) {
+    re += u[i].x * v[i].x + u[i].y * v[i].y;
+    im += u[i].x * v[i].y - u[i].y * v[i].x;
+  }
+  out_re_im[0] = re;
+  out_re_im[1] = im;
+  g_launches += 2;
+  return QSIM_OK;
+}
+
+int reduce_expect(const qs_c128* k, const qs_c128* r, int n, double* out_re_im, void*) {
+  const uint64_t dim = 1ull << n;
+  double re = 0.0, im = 0.0;
+  for (uint64_t i = 0; i < dim; ++i)
+    for (uint64_t j = 0; j < dim; ++j) {
+      const qs_c128 t = qs_cmul(r[i * dim + j], k[j]);
+      re += k[i].x * t.x + k[i].y * t.y;
+      im += k[i].x * t.y - k[i].y * t.x;
+    }
+  out_re_im[0] = re;
+  out_re_im[1] = im;
+  g_launches += 2;
+  return QSIM_OK;
+}
+
+int reduce_purity(const qs_c128* r, int n, double* out_re_im, void*) {
+  const uint64_t dim = 1ull << n;
+  double re = 0.0, im = 0.0;
+  for (uint64_t i = 0; i < dim; ++i)
+    for (uint64_t j = 0; j < dim; ++j) {
+      const qs_c128 t = qs_cmul(r[i * dim + j], r[j * dim + i]);
+      re += t.x;
+      im += t.y;
+    }
+  out_re_im[0] = re;
+  out_re_im[1] = im;
+  g_launches += 2;
+  return QSIM_OK;
+}
+
+int reduce_trace(const qs_c128* r, int n, double* out_re_im, void*) {
+  const uint64_t dim = 1ull << n;
+  double re = 0.0, im = 0.0;
+  for (uint64_t i = 0; i < dim; ++i) { re += r[i * dim + i].x; im += r[i * dim + i].y; }
+  out_re_im[0] = re;
+  out_re_im[1] = im;
+  g_launches += 2;
+  return QSIM_OK;
+}
+
+// one launch per pass plus the final sum, as in the CUDA library
+int expect_pauli(const qs_c128* s, int n, const PauliPlan& plan, int64_t, double* sums, void*) {
+  const uint64_t count = 1ull << (n - plan.d);
+  for (const QsPauliPass& P : plan.passes) {
+    double acc[QS_PAULI_MAX_TERMS] = {0.0}, wal[2 << QS_PAULI_MAX_D];
+    for (uint64_t o = 0; o < count; ++o) {
+      switch (plan.d) {
+        case 1: qs_pauli_item<1>(P, s, o, acc, wal, 1); break;
+        case 2: qs_pauli_item<2>(P, s, o, acc, wal, 1); break;
+        case 3: qs_pauli_item<3>(P, s, o, acc, wal, 1); break;
+        default: qs_pauli_item<4>(P, s, o, acc, wal, 1); break;
+      }
+    }
+    for (uint32_t t = 0; t < P.nterms; ++t) sums[2 * ((size_t)P.term0 + t)] = acc[t];
+    ++g_launches;
+  }
+  ++g_launches;                              // the final sum
+  return QSIM_OK;
+}
+
+int expect_pauli_dm(const qs_c128* rho, int n, int64_t n_terms, const uint64_t* xi, const uint64_t* zi,
+                    double* sums, void*) {
+  for (int64_t t = 0; t < n_terms; ++t)
+    for (uint64_t c = 0; c < (1ull << n); ++c) {
+      const qs_c128 v = qs_pauli_dm_elem(rho, n, xi[t], zi[t], c);
+      sums[2 * t] += v.x;
+      sums[2 * t + 1] += v.y;
+    }
+  g_launches += 2;
+  return QSIM_OK;
+}
+
+int rb_batch(int nq, int64_t n_seq, const uint16_t* opcodes, const int64_t* offsets, const double* superops,
+             const double* unitaries, const double* rho0, const double* psi0, double* out_fidelity,
+             double* out_purity, double* out_rho, void*) {
+  for (int64_t b = 0; b < n_seq; ++b) {
+    const int64_t lo = offsets[b], hi = offsets[b + 1];
+    if (nq == 2)
+      qs_rb_sequence<4>(opcodes + lo, hi - lo, superops, unitaries, rho0, psi0, out_fidelity + b,
+                        out_purity + b, out_rho ? out_rho + (size_t)b * 2 * 16 : nullptr);
+    else
+      qs_rb_sequence<2>(opcodes + lo, hi - lo, superops, unitaries, rho0, psi0, out_fidelity + b,
+                        out_purity + b, out_rho ? out_rho + (size_t)b * 2 * 4 : nullptr);
+  }
+  ++g_launches;
+  return QSIM_OK;
+}
+
+int traj_batch(int n, int64_t shots, int n_ops, const QsTrajOp* op, const double* matrices, const uint8_t* flips,
+               int64_t flips_per_shot, const qs_c128* psi0, const qs_c128* observable, double* out_fidelity,
+               double* out_prob_sum, qs_c128* out_states, void*) {
+  const uint64_t dim = 1ull << n;
+  std::vector<qs_c128> state(dim);
+  for (int64_t shot = 0; shot < shots; ++shot) {
+    memcpy(state.data(), psi0, sizeof(qs_c128) * dim);
+    const uint8_t* fl = flips + shot * flips_per_shot;
+    for (int o = 0; o < n_ops; ++o) {
+      qs_c128 M[16];
+      qs_traj_rows(op[o], matrices, fl, M);
+      fl += 2 * op[o].k;
+      qs_traj_apply(state.data(), n, op[o], M, 0, 1);
+    }
+    if (out_states) memcpy(out_states + (uint64_t)shot * dim, state.data(), sizeof(qs_c128) * dim);
+    double fr = 0.0, fi = 0.0;
+    for (uint64_t i = 0; i < dim; ++i) {
+      const qs_c128 v = state[i];
+      if (out_prob_sum) out_prob_sum[i] += v.x * v.x + v.y * v.y;
+      if (observable) {
+        const qs_c128 w = observable[i];
+        fr += w.x * v.x + w.y * v.y;
+        fi += w.x * v.y - w.y * v.x;
+      }
+    }
+    if (observable && out_fidelity) out_fidelity[shot] = fr * fr + fi * fi;
+  }
+  ++g_launches;
+  return QSIM_OK;
+}
+
+int swap_pack(const qs_c128* shard, qs_c128* buf, const QsBitSel& sel, uint64_t first, uint64_t count, void*) {
+  for (uint64_t r = 0; r < count; ++r) buf[r] = shard[qs_deposit(first + r, sel)];
+  ++g_launches;
+  return QSIM_OK;
+}
+
+int swap_unpack(qs_c128* shard, const qs_c128* buf, const QsBitSel& sel, uint64_t first, uint64_t count, void*) {
+  for (uint64_t r = 0; r < count; ++r) shard[qs_deposit(first + r, sel)] = buf[r];
+  ++g_launches;
+  return QSIM_OK;
+}
+
+}  // namespace qs::dev
 
 extern "C" {
 
@@ -173,325 +352,6 @@ int qsim_exchange_p2p(void*, void* const*, int, int, const int*, const int*, con
 int qsim_peer_copy(void* dst, const void* src, uint64_t bytes, void*) {
   if (!dst || !src) return qs::fail(QSIM_ERR_ARG, "qsim_peer_copy: null argument");
   memcpy(dst, src, bytes);
-  return QSIM_OK;
-}
-
-int qsim_plan_execute(const qsim_plan_t* p, void* state, int n_qubits, void* scratch, void*) {
-  return execute_plan(p, state, n_qubits, scratch);
-}
-
-int qsim_apply_matrix(void* state, int n_qubits, const int* targets, int k, const double* matrix,
-                      void* scratch, void*) {
-  if (!state || !targets || !matrix) return qs::fail(QSIM_ERR_ARG, "qsim_apply_matrix: null argument");
-  return one_gate(state, n_qubits, targets, k, matrix, scratch);
-}
-
-int qsim_apply_diagonal(void* state, int n_qubits, const int* targets, int k, const double* diag, void*) {
-  if (!state || !targets || !diag) return qs::fail(QSIM_ERR_ARG, "qsim_apply_diagonal: null argument");
-  if (k < 1 || k > QS_MAX_R) return qs::fail(QSIM_ERR_UNSUPPORTED, "qsim_apply_diagonal: k must be in [1, 4]");
-  const int dim = 1 << k;
-  std::vector<double> m(2 * (size_t)dim * dim, 0.0);
-  for (int d = 0; d < dim; ++d) { m[2 * (d * dim + d)] = diag[2 * d]; m[2 * (d * dim + d) + 1] = diag[2 * d + 1]; }
-  return one_gate(state, n_qubits, targets, k, m.data(), nullptr);
-}
-
-int qsim_apply_permutation(void* state, int n_qubits, const int* targets, int k, const int* perm, void*) {
-  if (!state || !targets || !perm) return qs::fail(QSIM_ERR_ARG, "qsim_apply_permutation: null argument");
-  if (k < 1 || k > QS_MAX_R) return qs::fail(QSIM_ERR_UNSUPPORTED, "qsim_apply_permutation: k must be in [1, 4]");
-  const int dim = 1 << k;
-  std::vector<double> m(2 * (size_t)dim * dim, 0.0);
-  std::vector<char> hit(dim, 0);
-  for (int c = 0; c < dim; ++c) {
-    if (perm[c] < 0 || perm[c] >= dim || hit[perm[c]]) return qs::fail(QSIM_ERR_ARG, "qsim_apply_permutation: not a permutation");
-    hit[perm[c]] = 1;
-    m[2 * (perm[c] * dim + c)] = 1.0;
-  }
-  return one_gate(state, n_qubits, targets, k, m.data(), nullptr);
-}
-
-int qsim_apply_superop(void* vec_rho, int n_qubits, const int* targets, int k, const double* superop,
-                       void* scratch, void*) {
-  if (!vec_rho || !targets || !superop) return qs::fail(QSIM_ERR_ARG, "qsim_apply_superop: null argument");
-  if (k < 1 || 2 * k > 10) return qs::fail(QSIM_ERR_UNSUPPORTED, "qsim_apply_superop: k must be in [1, 5]");
-  std::vector<int> t(2 * k);
-  for (int i = 0; i < k; ++i) { t[i] = targets[i]; t[k + i] = targets[i] + n_qubits; }
-  return one_gate(vec_rho, 2 * n_qubits, t.data(), 2 * k, superop, scratch);
-}
-
-int qsim_init_product(void* state, int n_qubits, const double* amps, void*) {
-  if (!state || !amps || n_qubits < 1 || n_qubits > 40) return qs::fail(QSIM_ERR_ARG, "qsim_init_product: bad argument");
-  qs_c128* s = (qs_c128*)state;
-  for (uint64_t i = 0; i < (1ull << n_qubits); ++i) s[i] = qs_product_amp(amps, n_qubits, i);
-  ++g_launches;
-  return QSIM_OK;
-}
-
-int qsim_measure_probs(const void* state, int n_qubits, int qubit, const double* bra0, const double* bra1,
-                       double* out_norm2, void*) {
-  if (!state || !bra0 || !bra1 || !out_norm2) return qs::fail(QSIM_ERR_ARG, "qsim_measure_probs: null argument");
-  if (n_qubits < 1 || qubit < 0 || qubit >= n_qubits) return qs::fail(QSIM_ERR_ARG, "qsim_measure_probs: qubit out of range");
-  const qs_c128* s = (const qs_c128*)state;
-  const int pos = n_qubits - 1 - qubit;
-  double p0 = 0.0, p1 = 0.0;
-  for (uint64_t r = 0; r < (1ull << (n_qubits - 1)); ++r) {
-    const qs_c128 u = qs_contract(s, pos, r, bra0), v = qs_contract(s, pos, r, bra1);
-    p0 += u.x * u.x + u.y * u.y;
-    p1 += v.x * v.x + v.y * v.y;
-  }
-  out_norm2[0] = p0;
-  out_norm2[1] = p1;
-  g_launches += 2;
-  return QSIM_OK;
-}
-
-int qsim_collapse(const void* in, void* out, int n_qubits, int qubit, const double* bra, double norm, void*) {
-  if (!in || !out || !bra) return qs::fail(QSIM_ERR_ARG, "qsim_collapse: null argument");
-  if (n_qubits < 1 || qubit < 0 || qubit >= n_qubits) return qs::fail(QSIM_ERR_ARG, "qsim_collapse: qubit out of range");
-  const int pos = n_qubits - 1 - qubit;
-  qs_c128* o = (qs_c128*)out;
-  for (uint64_t r = 0; r < (1ull << (n_qubits - 1)); ++r) {
-    qs_c128 v = qs_contract((const qs_c128*)in, pos, r, bra);
-    v.x /= norm; v.y /= norm;
-    o[r] = v;
-  }
-  ++g_launches;
-  return QSIM_OK;
-}
-
-int qsim_insert(const void* in, void* out, int n_qubits, int position, const double* amp, void*) {
-  if (!in || !out || !amp) return qs::fail(QSIM_ERR_ARG, "qsim_insert: null argument");
-  if (n_qubits < 0 || position < 0 || position > n_qubits) return qs::fail(QSIM_ERR_ARG, "qsim_insert: position out of range");
-  qs_c128* o = (qs_c128*)out;
-  for (uint64_t i = 0; i < (1ull << (n_qubits + 1)); ++i)
-    o[i] = qs_insert_amp((const qs_c128*)in, n_qubits - position, i, amp);
-  ++g_launches;
-  return QSIM_OK;
-}
-
-int qsim_reduce_norm2(const void* state, uint64_t n_amps, double* out, void*) {
-  if (!state || !out) return qs::fail(QSIM_ERR_ARG, "qsim_reduce_norm2: null argument");
-  const qs_c128* s = (const qs_c128*)state;
-  double acc = 0.0;
-  for (uint64_t i = 0; i < n_amps; ++i) acc += s[i].x * s[i].x + s[i].y * s[i].y;
-  *out = acc;
-  g_launches += 2;
-  return QSIM_OK;
-}
-
-int qsim_reduce_inner(const void* a, const void* b, uint64_t n_amps, double* out_re_im, void*) {
-  if (!a || !b || !out_re_im) return qs::fail(QSIM_ERR_ARG, "qsim_reduce_inner: null argument");
-  const qs_c128 *u = (const qs_c128*)a, *v = (const qs_c128*)b;
-  double re = 0.0, im = 0.0;
-  for (uint64_t i = 0; i < n_amps; ++i) {
-    re += u[i].x * v[i].x + u[i].y * v[i].y;
-    im += u[i].x * v[i].y - u[i].y * v[i].x;
-  }
-  out_re_im[0] = re;
-  out_re_im[1] = im;
-  g_launches += 2;
-  return QSIM_OK;
-}
-
-int qsim_reduce_expect(const void* ket, const void* rho, int n_qubits, double* out_re_im, void*) {
-  if (!ket || !rho || !out_re_im || n_qubits < 0 || n_qubits > 20) return qs::fail(QSIM_ERR_ARG, "qsim_reduce_expect: bad argument");
-  const qs_c128 *k = (const qs_c128*)ket, *r = (const qs_c128*)rho;
-  const uint64_t dim = 1ull << n_qubits;
-  double re = 0.0, im = 0.0;
-  for (uint64_t i = 0; i < dim; ++i)
-    for (uint64_t j = 0; j < dim; ++j) {
-      const qs_c128 t = qs_cmul(r[i * dim + j], k[j]);
-      re += k[i].x * t.x + k[i].y * t.y;
-      im += k[i].x * t.y - k[i].y * t.x;
-    }
-  out_re_im[0] = re;
-  out_re_im[1] = im;
-  g_launches += 2;
-  return QSIM_OK;
-}
-
-int qsim_reduce_purity(const void* rho, int n_qubits, double* out_re_im, void*) {
-  if (!rho || !out_re_im || n_qubits < 0 || n_qubits > 20) return qs::fail(QSIM_ERR_ARG, "qsim_reduce_purity: bad argument");
-  const qs_c128* r = (const qs_c128*)rho;
-  const uint64_t dim = 1ull << n_qubits;
-  double re = 0.0, im = 0.0;
-  for (uint64_t i = 0; i < dim; ++i)
-    for (uint64_t j = 0; j < dim; ++j) {
-      const qs_c128 t = qs_cmul(r[i * dim + j], r[j * dim + i]);
-      re += t.x;
-      im += t.y;
-    }
-  out_re_im[0] = re;
-  out_re_im[1] = im;
-  g_launches += 2;
-  return QSIM_OK;
-}
-
-int qsim_reduce_trace(const void* rho, int n_qubits, double* out_re_im, void*) {
-  if (!rho || !out_re_im || n_qubits < 0 || n_qubits > 20) return qs::fail(QSIM_ERR_ARG, "qsim_reduce_trace: bad argument");
-  const qs_c128* r = (const qs_c128*)rho;
-  const uint64_t dim = 1ull << n_qubits;
-  double re = 0.0, im = 0.0;
-  for (uint64_t i = 0; i < dim; ++i) { re += r[i * dim + i].x; im += r[i * dim + i].y; }
-  out_re_im[0] = re;
-  out_re_im[1] = im;
-  g_launches += 2;
-  return QSIM_OK;
-}
-
-// Pauli expectation values: the same grouping (pauli.cpp) and the same per-thread bodies
-// (elem_ops.h) as the CUDA library; one launch per pass plus the final sum, as there.
-int qsim_expect_pauli(const void* state, int n_qubits, int64_t n_terms, const uint64_t* x_masks,
-                      const uint64_t* z_masks, double* out, void*) {
-  int rc = qs::check_pauli_args("qsim_expect_pauli", n_qubits, n_terms, x_masks, z_masks, out);
-  if (rc != QSIM_OK || n_terms == 0) return rc;
-  if (!state) return qs::fail(QSIM_ERR_ARG, "qsim_expect_pauli: null state");
-  qs::PauliPlan plan;
-  rc = qs::plan_pauli(n_qubits, n_terms, x_masks, z_masks, &plan);
-  if (rc != QSIM_OK) return rc;
-  std::vector<double> sums(2 * (size_t)n_terms, 0.0);
-  const uint64_t count = 1ull << (n_qubits - plan.d);
-  const qs_c128* s = (const qs_c128*)state;
-  for (const QsPauliPass& P : plan.passes) {
-    double acc[QS_PAULI_MAX_TERMS] = {0.0}, wal[2 << QS_PAULI_MAX_D];
-    for (uint64_t o = 0; o < count; ++o) {
-      switch (plan.d) {
-        case 1: qs_pauli_item<1>(P, s, o, acc, wal, 1); break;
-        case 2: qs_pauli_item<2>(P, s, o, acc, wal, 1); break;
-        case 3: qs_pauli_item<3>(P, s, o, acc, wal, 1); break;
-        default: qs_pauli_item<4>(P, s, o, acc, wal, 1); break;
-      }
-    }
-    for (uint32_t t = 0; t < P.nterms; ++t) sums[2 * ((size_t)P.term0 + t)] = acc[t];
-    ++g_launches;
-  }
-  ++g_launches;                              // the final sum
-  qs::pauli_finish(plan, sums.data(), out);
-  return QSIM_OK;
-}
-
-int qsim_expect_pauli_dm(const void* vec_rho, int n_qubits, int64_t n_terms, const uint64_t* x_masks,
-                         const uint64_t* z_masks, double* out_re_im, void*) {
-  int rc = qs::check_pauli_args("qsim_expect_pauli_dm", n_qubits, n_terms, x_masks, z_masks, out_re_im);
-  if (rc != QSIM_OK || n_terms == 0) return rc;
-  if (!vec_rho) return qs::fail(QSIM_ERR_ARG, "qsim_expect_pauli_dm: null state");
-  if (n_qubits > 31) return qs::fail(QSIM_ERR_ARG, "qsim_expect_pauli_dm: n_qubits must be in [1, 31]");
-  std::vector<uint64_t> xi, zi;
-  std::vector<uint8_t> phase;
-  qs::pauli_index_masks(n_qubits, n_terms, x_masks, z_masks, &xi, &zi, &phase);
-  std::vector<double> sums(2 * (size_t)n_terms, 0.0);
-  const qs_c128* rho = (const qs_c128*)vec_rho;
-  for (int64_t t = 0; t < n_terms; ++t)
-    for (uint64_t c = 0; c < (1ull << n_qubits); ++c) {
-      const qs_c128 v = qs_pauli_dm_elem(rho, n_qubits, xi[t], zi[t], c);
-      sums[2 * t] += v.x;
-      sums[2 * t + 1] += v.y;
-    }
-  g_launches += 2;
-  qs::pauli_finish_dm(n_terms, phase, sums.data(), out_re_im);
-  return QSIM_OK;
-}
-
-int qsim_rb_batch(int nq, int64_t n_seq, const uint16_t* opcodes, const int64_t* offsets, int n_opcodes,
-                  const double* superops, const double* unitaries, const double* rho0, const double* psi0,
-                  double* out_fidelity, double* out_purity, double* out_rho, void*) {
-  if (!opcodes || !offsets || !superops || !unitaries || !rho0 || !psi0 || !out_fidelity || !out_purity)
-    return qs::fail(QSIM_ERR_ARG, "qsim_rb_batch: null argument");
-  if (nq < 1 || nq > 2) return qs::fail(QSIM_ERR_UNSUPPORTED, "qsim_rb_batch: nq must be 1 or 2");
-  if (n_seq < 0 || n_opcodes < 1 || n_opcodes > 65536) return qs::fail(QSIM_ERR_ARG, "qsim_rb_batch: bad sizes");
-  for (int64_t b = 0; b < n_seq; ++b) {
-    const int64_t lo = offsets[b], hi = offsets[b + 1];
-    if (nq == 2)
-      qs_rb_sequence<4>(opcodes + lo, hi - lo, superops, unitaries, rho0, psi0, out_fidelity + b,
-                        out_purity + b, out_rho ? out_rho + (size_t)b * 2 * 16 : nullptr);
-    else
-      qs_rb_sequence<2>(opcodes + lo, hi - lo, superops, unitaries, rho0, psi0, out_fidelity + b,
-                        out_purity + b, out_rho ? out_rho + (size_t)b * 2 * 4 : nullptr);
-  }
-  ++g_launches;
-  return QSIM_OK;
-}
-
-int qsim_traj_batch(int n_qubits, int64_t shots, int n_ops, const int32_t* ops, const double* matrices,
-                    const uint8_t* flips, int64_t flips_per_shot, const double* psi0, const double* observable,
-                    double* out_fidelity, double* out_prob_sum, double* out_states, void*) {
-  if (!ops || !matrices || !flips || !psi0) return qs::fail(QSIM_ERR_ARG, "qsim_traj_batch: null argument");
-  if (n_qubits < 1 || n_qubits > 12) return qs::fail(QSIM_ERR_UNSUPPORTED, "qsim_traj_batch: 1 <= n_qubits <= 12");
-  if (shots < 0 || n_ops < 0 || flips_per_shot < 0) return qs::fail(QSIM_ERR_ARG, "qsim_traj_batch: bad sizes");
-  const uint64_t dim = 1ull << n_qubits;
-  const QsTrajOp* op = (const QsTrajOp*)ops;
-  std::vector<qs_c128> state(dim);
-  for (int64_t shot = 0; shot < shots; ++shot) {
-    memcpy(state.data(), psi0, sizeof(qs_c128) * dim);
-    const uint8_t* fl = flips + shot * flips_per_shot;
-    for (int o = 0; o < n_ops; ++o) {
-      qs_c128 M[16];
-      qs_traj_rows(op[o], matrices, fl, M);
-      fl += 2 * op[o].k;
-      qs_traj_apply(state.data(), n_qubits, op[o], M, 0, 1);
-    }
-    if (out_states) memcpy(out_states + 2 * (uint64_t)shot * dim, state.data(), sizeof(qs_c128) * dim);
-    double fr = 0.0, fi = 0.0;
-    for (uint64_t i = 0; i < dim; ++i) {
-      const qs_c128 v = state[i];
-      if (out_prob_sum) out_prob_sum[i] += v.x * v.x + v.y * v.y;
-      if (observable) {
-        const double wx = observable[2 * i], wy = observable[2 * i + 1];
-        fr += wx * v.x + wy * v.y;
-        fi += wx * v.y - wy * v.x;
-      }
-    }
-    if (observable && out_fidelity) out_fidelity[shot] = fr * fr + fi * fi;
-  }
-  ++g_launches;
-  return QSIM_OK;
-}
-
-static int swap_select(const char* who, int n_local, int nbits, const int* local_qubits, const int* bit_values,
-                       uint64_t first, uint64_t count, QsBitSel* sel) {
-  if (n_local < 1 || nbits < 1 || nbits > 8 || nbits > n_local || !local_qubits || !bit_values)
-    return qs::fail(QSIM_ERR_ARG, std::string(who) + ": bad bit list");
-  sel->k = nbits;
-  for (int i = 0; i < nbits; ++i) {
-    if (local_qubits[i] < 0 || local_qubits[i] >= n_local || (bit_values[i] | 1) != 1)
-      return qs::fail(QSIM_ERR_ARG, std::string(who) + ": bad qubit or bit");
-    sel->pos[i] = n_local - 1 - local_qubits[i];
-    sel->val[i] = bit_values[i];
-  }
-  for (int i = 1; i < nbits; ++i)
-    for (int j = i; j > 0 && sel->pos[j] < sel->pos[j - 1]; --j) {
-      std::swap(sel->pos[j], sel->pos[j - 1]);
-      std::swap(sel->val[j], sel->val[j - 1]);
-    }
-  for (int i = 1; i < nbits; ++i)
-    if (sel->pos[i] == sel->pos[i - 1]) return qs::fail(QSIM_ERR_ARG, std::string(who) + ": repeated qubit");
-  if (first + count > (1ull << (n_local - nbits)))
-    return qs::fail(QSIM_ERR_ARG, std::string(who) + ": chunk out of range");
-  return QSIM_OK;
-}
-
-int qsim_swap_pack(const void* shard, void* sendbuf, int n_local, int nbits, const int* local_qubits,
-                   const int* bit_values, uint64_t first, uint64_t count, void*) {
-  if (!shard || !sendbuf) return qs::fail(QSIM_ERR_ARG, "qsim_swap_pack: null argument");
-  QsBitSel sel;
-  const int rc = swap_select("qsim_swap_pack", n_local, nbits, local_qubits, bit_values, first, count, &sel);
-  if (rc != QSIM_OK) return rc;
-  const qs_c128* s = (const qs_c128*)shard;
-  qs_c128* b = (qs_c128*)sendbuf;
-  for (uint64_t r = 0; r < count; ++r) b[r] = s[qs_deposit(first + r, sel)];
-  ++g_launches;
-  return QSIM_OK;
-}
-
-int qsim_swap_unpack(void* shard, const void* recvbuf, int n_local, int nbits, const int* local_qubits,
-                     const int* bit_values, uint64_t first, uint64_t count, void*) {
-  if (!shard || !recvbuf) return qs::fail(QSIM_ERR_ARG, "qsim_swap_unpack: null argument");
-  QsBitSel sel;
-  const int rc = swap_select("qsim_swap_unpack", n_local, nbits, local_qubits, bit_values, first, count, &sel);
-  if (rc != QSIM_OK) return rc;
-  qs_c128* s = (qs_c128*)shard;
-  const qs_c128* b = (const qs_c128*)recvbuf;
-  for (uint64_t r = 0; r < count; ++r) s[qs_deposit(first + r, sel)] = b[r];
-  ++g_launches;
   return QSIM_OK;
 }
 

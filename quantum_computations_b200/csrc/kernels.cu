@@ -1,4 +1,5 @@
-// sm_100a kernels and the device-facing half of the C ABI (include/qsim_b200.h).
+// sm_100a kernels, the CUDA backend of the compute entry points (backend.h) and the peer, IPC and
+// exchange functions of the C ABI (include/qsim_b200.h).
 //
 // Almost everything here is memory-bound complex128 work: TMA-staged 2^T-amplitude
 // tiles in shared memory so that many gates apply per HBM pass, 16-byte (128-bit)
@@ -22,8 +23,7 @@
 #include <utility>
 #include <vector>
 
-#include "elem_ops.h"
-#include "planner.h"
+#include "backend.h"
 
 namespace {
 
@@ -62,6 +62,13 @@ DevCtx g_ctx[kMaxDevices];
     if (e_ != cudaSuccess)                                                             \
       return qs::fail(QSIM_ERR_CUDA, std::string(#call) + ": " + cudaGetErrorString(e_)); \
   } while (0)
+
+// Counts `n` kernel launches and reports a launch that failed.
+int launched(int n = 1) {
+  g_launches.fetch_add(n, std::memory_order_relaxed);
+  QS_CUDA(cudaGetLastError());
+  return QSIM_OK;
+}
 
 // The device a buffer lives on, made current for the lifetime of this object (the caller's
 // current device is restored afterwards: torch keeps its own idea of it).
@@ -366,17 +373,12 @@ int launch_pass(DevCtx* ctx, const QsPass& P, qs_c128* state, int n, cudaStream_
   CUtensorMap map;
   make_tma_geom(P, state, n, &geom, &map);
   variants[vi]<<<(unsigned)grid, threads, smem, stream>>>(state, P, map, geom, ntiles);
-  g_launches.fetch_add(1, std::memory_order_relaxed);
-  QS_CUDA(cudaGetLastError());
-  return QSIM_OK;
+  return launched();
 }
 
 // =====================================================================================
 // Simple streaming kernels
 // =====================================================================================
-// the 2 x n single-qubit amplitudes travel as a kernel parameter (no allocation, no copy)
-struct ProductAmps { double a[4 * 40]; };
-
 __global__ void k_init_product(qs_c128* state, int n, const __grid_constant__ ProductAmps amps, uint64_t count) {
   for (uint64_t i = blockIdx.x * (uint64_t)blockDim.x + threadIdx.x; i < count;
        i += (uint64_t)gridDim.x * blockDim.x)
@@ -412,8 +414,6 @@ __global__ void __launch_bounds__(256) k_init_product_big(qs_c128* state, int n,
     for (uint32_t o1 = 0; o1 < 256; ++o1) dst[(uint64_t)o1 << 8] = qs_cmul(pl, t1[o1]);
   }
 }
-
-struct BraPair { double b[4]; };
 
 __global__ void k_collapse(const qs_c128* __restrict__ in, qs_c128* __restrict__ out, int pos,
                            BraPair bra, double norm, uint64_t count) {
@@ -632,8 +632,8 @@ int reduce_to_host(DevCtx* ctx, F f, uint64_t count, double* out2, cudaStream_t 
   std::lock_guard<std::mutex> guard(ctx->reduce_lock);
   k_reduce<F><<<(unsigned)blocks, kReduceThreads, 0, stream>>>(f, count, ctx->d_partials);
   k_reduce_final<<<1, kReduceThreads, 0, stream>>>(ctx->d_partials, (int)blocks, ctx->d_out);
-  g_launches.fetch_add(2, std::memory_order_relaxed);
-  QS_CUDA(cudaGetLastError());
+  int rc = launched(2);
+  if (rc != QSIM_OK) return rc;
   QS_CUDA(cudaMemcpyAsync(ctx->h_out, ctx->d_out, 2 * sizeof(double), cudaMemcpyDeviceToHost, stream));
   QS_CUDA(cudaStreamSynchronize(stream));
   out2[0] = ctx->h_out[0];
@@ -747,15 +747,17 @@ int pauli_scratch(DevCtx* ctx, size_t terms, size_t blocks) {
   return QSIM_OK;
 }
 
-// Final sum of a call's partials and the one download; synchronises the stream.
-int pauli_sums_to_host(DevCtx* ctx, int64_t n_terms, int nblocks, cudaStream_t stream) {
+// Final sum of a call's partials and the one download into `sums` (2 * n_terms doubles; the
+// caller holds reduce_lock, which guards the pinned buffer too); synchronises the stream.
+int pauli_sums_to_host(DevCtx* ctx, int64_t n_terms, int nblocks, double* sums, cudaStream_t stream) {
   const unsigned grid = (unsigned)std::min<int64_t>(n_terms, 65535);
   k_pauli_final<<<grid, kReduceThreads, 0, stream>>>(ctx->d_pauli_partials, nblocks, n_terms, ctx->d_pauli_sums);
-  g_launches.fetch_add(1, std::memory_order_relaxed);
-  QS_CUDA(cudaGetLastError());
+  const int rc = launched();
+  if (rc != QSIM_OK) return rc;
   QS_CUDA(cudaMemcpyAsync(ctx->h_pauli_sums, ctx->d_pauli_sums, sizeof(double) * 2 * n_terms, cudaMemcpyDeviceToHost,
                           stream));
   QS_CUDA(cudaStreamSynchronize(stream));
+  memcpy(sums, ctx->h_pauli_sums, sizeof(double) * 2 * n_terms);
   return QSIM_OK;
 }
 
@@ -968,38 +970,7 @@ int run_dense_block(DevCtx* ctx, const qs::PlanItem& it, qs_c128* state, int n, 
   uint64_t grid = (uint64_t)ctx->sms * (uint64_t)occ;
   if (grid > ntiles) grid = ntiles;
   k_dense_block<<<(unsigned)grid, threads, smem, stream>>>(state, (const double*)it.dev_mat.get(), G, ntiles);
-  g_launches.fetch_add(1, std::memory_order_relaxed);
-  QS_CUDA(cudaGetLastError());
-  return QSIM_OK;
-}
-
-int execute_plan(const qsim_plan* p, void* state, int n, void* scratch, void* stream) {
-  if (!p || !state) return qs::fail(QSIM_ERR_ARG, "qsim_plan_execute: null argument");
-  if (n != p->n) return qs::fail(QSIM_ERR_ARG, "qsim_plan_execute: plan was compiled for a different qubit count");
-  Bound bound;
-  int rc = bind_device(state, &bound);
-  DevCtx* ctx = bound.ctx;
-  if (rc != QSIM_OK) return rc;
-  cudaStream_t st = (cudaStream_t)stream;
-  for (const qs::PlanItem& it : p->items) {
-    rc = it.generic ? run_dense_block(ctx, it, (qs_c128*)state, n, bound.device, st)
-                    : launch_pass(ctx, it.pass, (qs_c128*)state, n, st);
-    if (rc != QSIM_OK) return rc;
-  }
-  return QSIM_OK;
-}
-
-int one_gate(void* state, int n, const int* targets, int k, const double* matrix, void* scratch, void* stream) {
-  qsim_circuit_t* c = nullptr;
-  int rc = qsim_circuit_create(n, &c);
-  if (rc != QSIM_OK) return rc;
-  rc = qsim_circuit_add_matrix(c, k, targets, matrix);
-  qsim_plan_t* p = nullptr;
-  if (rc == QSIM_OK) rc = qsim_plan_compile(c, nullptr, &p);
-  if (rc == QSIM_OK) rc = execute_plan(p, state, n, scratch, stream);
-  qsim_plan_destroy(p);
-  qsim_circuit_destroy(c);
-  return rc;
+  return launched();
 }
 
 }  // namespace
@@ -1122,9 +1093,7 @@ int qsim_exchange_p2p(void* shard, void* const* peer_shards, int n_local, int nb
   else if (U == 4) k_exchange_p2p<4><<<(unsigned)blocks, 256, 0, st>>>((qs_c128*)shard, G);
   else if (U == 2) k_exchange_p2p<2><<<(unsigned)blocks, 256, 0, st>>>((qs_c128*)shard, G);
   else k_exchange_p2p<1><<<(unsigned)blocks, 256, 0, st>>>((qs_c128*)shard, G);
-  g_launches.fetch_add(1, std::memory_order_relaxed);
-  QS_CUDA(cudaGetLastError());
-  return QSIM_OK;
+  return launched();
 }
 
 int qsim_peer_copy(void* dst, const void* src, uint64_t bytes, void* stream) {
@@ -1133,231 +1102,154 @@ int qsim_peer_copy(void* dst, const void* src, uint64_t bytes, void* stream) {
   return QSIM_OK;
 }
 
-int qsim_plan_execute(const qsim_plan_t* p, void* state, int n_qubits, void* scratch, void* stream) {
-  return execute_plan(p, state, n_qubits, scratch, stream);
-}
+}  // extern "C"
 
-int qsim_apply_matrix(void* state, int n_qubits, const int* targets, int k, const double* matrix,
-                      void* scratch, void* stream) {
-  if (!state || !targets || !matrix) return qs::fail(QSIM_ERR_ARG, "qsim_apply_matrix: null argument");
-  return one_gate(state, n_qubits, targets, k, matrix, scratch, stream);
-}
+// =====================================================================================
+// Backend of the compute entry points (backend.h; checks and lowering in capi_host.cpp)
+// =====================================================================================
+namespace qs::dev {
 
-int qsim_apply_diagonal(void* state, int n_qubits, const int* targets, int k, const double* diag, void* stream) {
-  if (!state || !targets || !diag) return qs::fail(QSIM_ERR_ARG, "qsim_apply_diagonal: null argument");
-  if (k < 1 || k > QS_MAX_R) return qs::fail(QSIM_ERR_UNSUPPORTED, "qsim_apply_diagonal: k must be in [1, 4]");
-  const int dim = 1 << k;
-  std::vector<double> m(2 * (size_t)dim * dim, 0.0);
-  for (int d = 0; d < dim; ++d) { m[2 * (d * dim + d)] = diag[2 * d]; m[2 * (d * dim + d) + 1] = diag[2 * d + 1]; }
-  return one_gate(state, n_qubits, targets, k, m.data(), nullptr, stream);
-}
-
-int qsim_apply_permutation(void* state, int n_qubits, const int* targets, int k, const int* perm, void* stream) {
-  if (!state || !targets || !perm) return qs::fail(QSIM_ERR_ARG, "qsim_apply_permutation: null argument");
-  if (k < 1 || k > QS_MAX_R) return qs::fail(QSIM_ERR_UNSUPPORTED, "qsim_apply_permutation: k must be in [1, 4]");
-  const int dim = 1 << k;
-  std::vector<double> m(2 * (size_t)dim * dim, 0.0);
-  std::vector<char> hit(dim, 0);
-  for (int c = 0; c < dim; ++c) {
-    if (perm[c] < 0 || perm[c] >= dim || hit[perm[c]]) return qs::fail(QSIM_ERR_ARG, "qsim_apply_permutation: not a permutation");
-    hit[perm[c]] = 1;
-    m[2 * (perm[c] * dim + c)] = 1.0;
-  }
-  return one_gate(state, n_qubits, targets, k, m.data(), nullptr, stream);
-}
-
-int qsim_apply_superop(void* vec_rho, int n_qubits, const int* targets, int k, const double* superop,
-                       void* scratch, void* stream) {
-  if (!vec_rho || !targets || !superop) return qs::fail(QSIM_ERR_ARG, "qsim_apply_superop: null argument");
-  if (k < 1 || 2 * k > 10) return qs::fail(QSIM_ERR_UNSUPPORTED, "qsim_apply_superop: k must be in [1, 5]");
-  std::vector<int> t(2 * k);
-  for (int i = 0; i < k; ++i) { t[i] = targets[i]; t[k + i] = targets[i] + n_qubits; }
-  return one_gate(vec_rho, 2 * n_qubits, t.data(), 2 * k, superop, scratch, stream);
-}
-
-int qsim_init_product(void* state, int n_qubits, const double* amps, void* stream) {
-  if (!state || !amps || n_qubits < 1 || n_qubits > 40) return qs::fail(QSIM_ERR_ARG, "qsim_init_product: bad argument");
+int execute_plan(const qsim_plan& p, qs_c128* state, int n, void* stream) {
   Bound bound;
   int rc = bind_device(state, &bound);
   DevCtx* ctx = bound.ctx;
   if (rc != QSIM_OK) return rc;
   cudaStream_t st = (cudaStream_t)stream;
-  ProductAmps pa;
-  memset(&pa, 0, sizeof(pa));
-  memcpy(pa.a, amps, sizeof(double) * 4 * n_qubits);
-  const uint64_t count = 1ull << n_qubits;
-  if (n_qubits >= 16) {
+  for (const qs::PlanItem& it : p.items) {
+    rc = it.generic ? run_dense_block(ctx, it, state, n, bound.device, st) : launch_pass(ctx, it.pass, state, n, st);
+    if (rc != QSIM_OK) return rc;
+  }
+  return QSIM_OK;
+}
+
+int init_product(qs_c128* state, int n, const ProductAmps& amps, void* stream) {
+  Bound bound;
+  int rc = bind_device(state, &bound);
+  DevCtx* ctx = bound.ctx;
+  if (rc != QSIM_OK) return rc;
+  cudaStream_t st = (cudaStream_t)stream;
+  const uint64_t count = 1ull << n;
+  if (n >= 16) {
     uint64_t blocks = count >> 16;
     if (blocks > (uint64_t)ctx->sms * 8) blocks = (uint64_t)ctx->sms * 8;
-    k_init_product_big<<<(unsigned)blocks, 256, 0, st>>>((qs_c128*)state, n_qubits, pa);
+    k_init_product_big<<<(unsigned)blocks, 256, 0, st>>>(state, n, amps);
   } else {
-    k_init_product<<<stream_grid(ctx, count, 256), 256, 0, st>>>((qs_c128*)state, n_qubits, pa, count);
+    k_init_product<<<stream_grid(ctx, count, 256), 256, 0, st>>>(state, n, amps, count);
   }
-  g_launches.fetch_add(1, std::memory_order_relaxed);
-  QS_CUDA(cudaGetLastError());
-  return QSIM_OK;
+  return launched();
 }
 
-int qsim_measure_probs(const void* state, int n_qubits, int qubit, const double* bra0, const double* bra1,
-                       double* out_norm2, void* stream) {
-  if (!state || !bra0 || !bra1 || !out_norm2) return qs::fail(QSIM_ERR_ARG, "qsim_measure_probs: null argument");
-  if (n_qubits < 1 || qubit < 0 || qubit >= n_qubits) return qs::fail(QSIM_ERR_ARG, "qsim_measure_probs: qubit out of range");
+int measure_probs(const qs_c128* state, int pos, uint64_t pairs, const BraPair& bra0, const BraPair& bra1,
+                  double* out_norm2, void* stream) {
   Bound bound;
   int rc = bind_device(state, &bound);
   DevCtx* ctx = bound.ctx;
   if (rc != QSIM_OK) return rc;
-  FnMeasure f;
-  f.a = (const qs_c128*)state;
-  f.pos = n_qubits - 1 - qubit;
-  memcpy(f.b0.b, bra0, sizeof(f.b0.b));
-  memcpy(f.b1.b, bra1, sizeof(f.b1.b));
-  return reduce_to_host(ctx, f, 1ull << (n_qubits - 1), out_norm2, (cudaStream_t)stream);
+  FnMeasure f{state, pos, bra0, bra1};
+  return reduce_to_host(ctx, f, pairs, out_norm2, (cudaStream_t)stream);
 }
 
-int qsim_collapse(const void* in, void* out, int n_qubits, int qubit, const double* bra, double norm, void* stream) {
-  if (!in || !out || !bra) return qs::fail(QSIM_ERR_ARG, "qsim_collapse: null argument");
-  if (n_qubits < 1 || qubit < 0 || qubit >= n_qubits) return qs::fail(QSIM_ERR_ARG, "qsim_collapse: qubit out of range");
+int collapse(const qs_c128* in, qs_c128* out, int pos, const BraPair& bra, double norm, uint64_t count,
+             void* stream) {
   Bound bound;
   int rc = bind_device(in, &bound);
   DevCtx* ctx = bound.ctx;
   if (rc != QSIM_OK) return rc;
-  BraPair b;
-  memcpy(b.b, bra, sizeof(b.b));
-  const uint64_t count = 1ull << (n_qubits - 1);
-  k_collapse<<<stream_grid(ctx, count, 256), 256, 0, (cudaStream_t)stream>>>(
-      (const qs_c128*)in, (qs_c128*)out, n_qubits - 1 - qubit, b, norm, count);
-  g_launches.fetch_add(1, std::memory_order_relaxed);
-  QS_CUDA(cudaGetLastError());
-  return QSIM_OK;
+  k_collapse<<<stream_grid(ctx, count, 256), 256, 0, (cudaStream_t)stream>>>(in, out, pos, bra, norm, count);
+  return launched();
 }
 
-int qsim_insert(const void* in, void* out, int n_qubits, int position, const double* amp, void* stream) {
-  if (!in || !out || !amp) return qs::fail(QSIM_ERR_ARG, "qsim_insert: null argument");
-  if (n_qubits < 0 || position < 0 || position > n_qubits) return qs::fail(QSIM_ERR_ARG, "qsim_insert: position out of range");
+int insert(const qs_c128* in, qs_c128* out, int pos, const BraPair& amp, uint64_t count, void* stream) {
   Bound bound;
   int rc = bind_device(in, &bound);
   DevCtx* ctx = bound.ctx;
   if (rc != QSIM_OK) return rc;
-  BraPair a;
-  memcpy(a.b, amp, sizeof(a.b));
-  const uint64_t count = 1ull << (n_qubits + 1);
-  // the new register has n+1 qubits; reference position p is index bit (n+1)-1-p
-  k_insert<<<stream_grid(ctx, count, 256), 256, 0, (cudaStream_t)stream>>>(
-      (const qs_c128*)in, (qs_c128*)out, n_qubits - position, a, count);
-  g_launches.fetch_add(1, std::memory_order_relaxed);
-  QS_CUDA(cudaGetLastError());
-  return QSIM_OK;
+  k_insert<<<stream_grid(ctx, count, 256), 256, 0, (cudaStream_t)stream>>>(in, out, pos, amp, count);
+  return launched();
 }
 
-int qsim_reduce_norm2(const void* state, uint64_t n_amps, double* out, void* stream) {
-  if (!state || !out) return qs::fail(QSIM_ERR_ARG, "qsim_reduce_norm2: null argument");
+int reduce_norm2(const qs_c128* state, uint64_t n_amps, double* out, void* stream) {
   Bound bound;
   int rc = bind_device(state, &bound);
   DevCtx* ctx = bound.ctx;
   if (rc != QSIM_OK) return rc;
-  FnNorm2 f{(const qs_c128*)state};
+  FnNorm2 f{state};
   double r[2];
   rc = reduce_to_host(ctx, f, n_amps, r, (cudaStream_t)stream);
   if (rc == QSIM_OK) *out = r[0];
   return rc;
 }
 
-int qsim_reduce_inner(const void* a, const void* b, uint64_t n_amps, double* out_re_im, void* stream) {
-  if (!a || !b || !out_re_im) return qs::fail(QSIM_ERR_ARG, "qsim_reduce_inner: null argument");
+int reduce_inner(const qs_c128* a, const qs_c128* b, uint64_t n_amps, double* out_re_im, void* stream) {
   Bound bound;
   int rc = bind_device(a, &bound);
   DevCtx* ctx = bound.ctx;
   if (rc != QSIM_OK) return rc;
-  FnInner f{(const qs_c128*)a, (const qs_c128*)b};
+  FnInner f{a, b};
   return reduce_to_host(ctx, f, n_amps, out_re_im, (cudaStream_t)stream);
 }
 
-int qsim_reduce_expect(const void* ket, const void* rho, int n_qubits, double* out_re_im, void* stream) {
-  if (!ket || !rho || !out_re_im || n_qubits < 0 || n_qubits > 20) return qs::fail(QSIM_ERR_ARG, "qsim_reduce_expect: bad argument");
+int reduce_expect(const qs_c128* ket, const qs_c128* rho, int n, double* out_re_im, void* stream) {
   Bound bound;
   int rc = bind_device(rho, &bound);
   DevCtx* ctx = bound.ctx;
   if (rc != QSIM_OK) return rc;
-  FnExpect f{(const qs_c128*)ket, (const qs_c128*)rho, n_qubits};
-  return reduce_to_host(ctx, f, 1ull << (2 * n_qubits), out_re_im, (cudaStream_t)stream);
+  FnExpect f{ket, rho, n};
+  return reduce_to_host(ctx, f, 1ull << (2 * n), out_re_im, (cudaStream_t)stream);
 }
 
-int qsim_reduce_purity(const void* rho, int n_qubits, double* out_re_im, void* stream) {
-  if (!rho || !out_re_im || n_qubits < 0 || n_qubits > 20) return qs::fail(QSIM_ERR_ARG, "qsim_reduce_purity: bad argument");
+int reduce_purity(const qs_c128* rho, int n, double* out_re_im, void* stream) {
   Bound bound;
   int rc = bind_device(rho, &bound);
   DevCtx* ctx = bound.ctx;
   if (rc != QSIM_OK) return rc;
-  FnPurity f{(const qs_c128*)rho, n_qubits};
-  return reduce_to_host(ctx, f, 1ull << (2 * n_qubits), out_re_im, (cudaStream_t)stream);
+  FnPurity f{rho, n};
+  return reduce_to_host(ctx, f, 1ull << (2 * n), out_re_im, (cudaStream_t)stream);
 }
 
-int qsim_reduce_trace(const void* rho, int n_qubits, double* out_re_im, void* stream) {
-  if (!rho || !out_re_im || n_qubits < 0 || n_qubits > 20) return qs::fail(QSIM_ERR_ARG, "qsim_reduce_trace: bad argument");
+int reduce_trace(const qs_c128* rho, int n, double* out_re_im, void* stream) {
   Bound bound;
   int rc = bind_device(rho, &bound);
   DevCtx* ctx = bound.ctx;
   if (rc != QSIM_OK) return rc;
-  FnTrace f{(const qs_c128*)rho, n_qubits};
-  return reduce_to_host(ctx, f, 1ull << n_qubits, out_re_im, (cudaStream_t)stream);
+  FnTrace f{rho, n};
+  return reduce_to_host(ctx, f, 1ull << n, out_re_im, (cudaStream_t)stream);
 }
 
-int qsim_expect_pauli(const void* state, int n_qubits, int64_t n_terms, const uint64_t* x_masks,
-                      const uint64_t* z_masks, double* out, void* stream) {
-  int rc = qs::check_pauli_args("qsim_expect_pauli", n_qubits, n_terms, x_masks, z_masks, out);
-  if (rc != QSIM_OK || n_terms == 0) return rc;
-  if (!state) return qs::fail(QSIM_ERR_ARG, "qsim_expect_pauli: null state");
-  qs::PauliPlan plan;
-  try {
-    rc = qs::plan_pauli(n_qubits, n_terms, x_masks, z_masks, &plan);
-  } catch (const std::bad_alloc&) {
-    rc = qs::fail(QSIM_ERR_NOMEM, "out of host memory while grouping the Pauli terms");
-  }
-  if (rc != QSIM_OK) return rc;
+int expect_pauli(const qs_c128* state, int n, const PauliPlan& plan, int64_t n_terms, double* sums, void* stream) {
   Bound bound;
-  rc = bind_device(state, &bound);
+  int rc = bind_device(state, &bound);
   DevCtx* ctx = bound.ctx;
   if (rc != QSIM_OK) return rc;
-  const uint64_t count = 1ull << (n_qubits - plan.d);
+  const uint64_t count = 1ull << (n - plan.d);
   uint64_t blocks = (count + kPauliThreads - 1) / kPauliThreads;
   blocks = std::min<uint64_t>(blocks, (uint64_t)ctx->sms * kPauliBlocksPerSM);
   const cudaStream_t st = (cudaStream_t)stream;
   std::lock_guard<std::mutex> guard(ctx->reduce_lock);
   rc = pauli_scratch(ctx, (size_t)n_terms, (size_t)blocks);
   if (rc != QSIM_OK) return rc;
-  const qs_c128* s = (const qs_c128*)state;
   for (const QsPauliPass& P : plan.passes) {
     switch (plan.d) {
-      case 1: launch_pauli_pass<1>(P, s, count, (unsigned)blocks, ctx->d_pauli_partials, st); break;
-      case 2: launch_pauli_pass<2>(P, s, count, (unsigned)blocks, ctx->d_pauli_partials, st); break;
-      case 3: launch_pauli_pass<3>(P, s, count, (unsigned)blocks, ctx->d_pauli_partials, st); break;
-      default: launch_pauli_pass<4>(P, s, count, (unsigned)blocks, ctx->d_pauli_partials, st); break;
+      case 1: launch_pauli_pass<1>(P, state, count, (unsigned)blocks, ctx->d_pauli_partials, st); break;
+      case 2: launch_pauli_pass<2>(P, state, count, (unsigned)blocks, ctx->d_pauli_partials, st); break;
+      case 3: launch_pauli_pass<3>(P, state, count, (unsigned)blocks, ctx->d_pauli_partials, st); break;
+      default: launch_pauli_pass<4>(P, state, count, (unsigned)blocks, ctx->d_pauli_partials, st); break;
     }
-    g_launches.fetch_add(1, std::memory_order_relaxed);
-    QS_CUDA(cudaGetLastError());
+    rc = launched();
+    if (rc != QSIM_OK) return rc;
   }
-  rc = pauli_sums_to_host(ctx, n_terms, (int)blocks, st);
-  if (rc != QSIM_OK) return rc;
-  qs::pauli_finish(plan, ctx->h_pauli_sums, out);
-  return QSIM_OK;
+  return pauli_sums_to_host(ctx, n_terms, (int)blocks, sums, st);
 }
 
-int qsim_expect_pauli_dm(const void* vec_rho, int n_qubits, int64_t n_terms, const uint64_t* x_masks,
-                         const uint64_t* z_masks, double* out_re_im, void* stream) {
-  int rc = qs::check_pauli_args("qsim_expect_pauli_dm", n_qubits, n_terms, x_masks, z_masks, out_re_im);
-  if (rc != QSIM_OK || n_terms == 0) return rc;
-  if (!vec_rho) return qs::fail(QSIM_ERR_ARG, "qsim_expect_pauli_dm: null state");
-  if (n_qubits > 31) return qs::fail(QSIM_ERR_ARG, "qsim_expect_pauli_dm: n_qubits must be in [1, 31]");
-  std::vector<uint64_t> xi, zi;
-  std::vector<uint8_t> phase;
-  qs::pauli_index_masks(n_qubits, n_terms, x_masks, z_masks, &xi, &zi, &phase);
-  std::vector<uint64_t> masks(2 * (size_t)n_terms);
+int expect_pauli_dm(const qs_c128* rho, int n, int64_t n_terms, const uint64_t* xi, const uint64_t* zi,
+                    double* sums, void* stream) {
+  std::vector<uint64_t> masks(2 * (size_t)n_terms);     // upload format of k_pauli_expect_dm: [x, z] per term
   for (int64_t t = 0; t < n_terms; ++t) { masks[2 * t] = xi[t]; masks[2 * t + 1] = zi[t]; }
   Bound bound;
-  rc = bind_device(vec_rho, &bound);
+  int rc = bind_device(rho, &bound);
   DevCtx* ctx = bound.ctx;
   if (rc != QSIM_OK) return rc;
-  const uint64_t dim = 1ull << n_qubits;
+  const uint64_t dim = 1ull << n;
   const unsigned bx = (unsigned)std::min<uint64_t>((dim + kReduceThreads - 1) / kReduceThreads, kPauliDmBlocks);
   const unsigned by = (unsigned)std::min<int64_t>(n_terms, 65535);
   const cudaStream_t st = (cudaStream_t)stream;
@@ -1365,27 +1257,18 @@ int qsim_expect_pauli_dm(const void* vec_rho, int n_qubits, int64_t n_terms, con
   rc = pauli_scratch(ctx, (size_t)n_terms, (size_t)bx);
   if (rc != QSIM_OK) return rc;
   QS_CUDA(cudaMemcpyAsync(ctx->d_pauli_masks, masks.data(), sizeof(uint64_t) * masks.size(), cudaMemcpyHostToDevice, st));
-  k_pauli_expect_dm<<<dim3(bx, by), kReduceThreads, 0, st>>>((const qs_c128*)vec_rho, n_qubits, ctx->d_pauli_masks,
-                                                            n_terms, ctx->d_pauli_partials);
-  g_launches.fetch_add(1, std::memory_order_relaxed);
-  QS_CUDA(cudaGetLastError());
-  rc = pauli_sums_to_host(ctx, n_terms, (int)bx, st);
+  k_pauli_expect_dm<<<dim3(bx, by), kReduceThreads, 0, st>>>(rho, n, ctx->d_pauli_masks, n_terms,
+                                                             ctx->d_pauli_partials);
+  rc = launched();
   if (rc != QSIM_OK) return rc;
-  qs::pauli_finish_dm(n_terms, phase, ctx->h_pauli_sums, out_re_im);
-  return QSIM_OK;
+  return pauli_sums_to_host(ctx, n_terms, (int)bx, sums, st);
 }
 
-int qsim_rb_batch(int nq, int64_t n_seq, const uint16_t* opcodes, const int64_t* offsets, int n_opcodes,
-                  const double* superops, const double* unitaries, const double* rho0, const double* psi0,
-                  double* out_fidelity, double* out_purity, double* out_rho, void* stream) {
-  if (!opcodes || !offsets || !superops || !unitaries || !rho0 || !psi0 || !out_fidelity || !out_purity)
-    return qs::fail(QSIM_ERR_ARG, "qsim_rb_batch: null argument");
-  if (nq < 1 || nq > 2) return qs::fail(QSIM_ERR_UNSUPPORTED, "qsim_rb_batch: nq must be 1 or 2");
-  if (n_seq < 0 || n_opcodes < 1 || n_opcodes > 65536) return qs::fail(QSIM_ERR_ARG, "qsim_rb_batch: bad sizes");
-  if (n_seq == 0) return QSIM_OK;
+int rb_batch(int nq, int64_t n_seq, const uint16_t* opcodes, const int64_t* offsets, const double* superops,
+             const double* unitaries, const double* rho0, const double* psi0, double* out_fidelity,
+             double* out_purity, double* out_rho, void* stream) {
   Bound bound;
   int rc = bind_device(out_fidelity, &bound);
-  DevCtx* ctx = bound.ctx;
   if (rc != QSIM_OK) return rc;
   const unsigned blocks = (unsigned)((n_seq + 127) / 128);
   cudaStream_t st = (cudaStream_t)stream;
@@ -1395,94 +1278,47 @@ int qsim_rb_batch(int nq, int64_t n_seq, const uint16_t* opcodes, const int64_t*
   else
     k_rb_batch<2><<<blocks, 128, 0, st>>>(n_seq, opcodes, offsets, superops, unitaries, rho0, psi0,
                                          out_fidelity, out_purity, out_rho);
-  g_launches.fetch_add(1, std::memory_order_relaxed);
-  QS_CUDA(cudaGetLastError());
-  return QSIM_OK;
+  return launched();
 }
 
-int qsim_traj_batch(int n_qubits, int64_t shots, int n_ops, const int32_t* ops, const double* matrices,
-                    const uint8_t* flips, int64_t flips_per_shot, const double* psi0, const double* observable,
-                    double* out_fidelity, double* out_prob_sum, double* out_states, void* stream) {
-  if (!ops || !matrices || !flips || !psi0) return qs::fail(QSIM_ERR_ARG, "qsim_traj_batch: null argument");
-  if (n_qubits < 1 || n_qubits > 12) return qs::fail(QSIM_ERR_UNSUPPORTED, "qsim_traj_batch: 1 <= n_qubits <= 12");
-  if (shots < 0 || n_ops < 0 || flips_per_shot < 0) return qs::fail(QSIM_ERR_ARG, "qsim_traj_batch: bad sizes");
-  if (shots == 0) return QSIM_OK;
+int traj_batch(int n, int64_t shots, int n_ops, const QsTrajOp* ops, const double* matrices, const uint8_t* flips,
+               int64_t flips_per_shot, const qs_c128* psi0, const qs_c128* observable, double* out_fidelity,
+               double* out_prob_sum, qs_c128* out_states, void* stream) {
   Bound bound;
   int rc = bind_device(psi0, &bound);
   if (rc != QSIM_OK) return rc;
-  const int smem = (int)(sizeof(qs_c128) << n_qubits);
+  const int smem = (int)(sizeof(qs_c128) << n);
   if (smem > 48 * 1024) QS_CUDA(cudaFuncSetAttribute(k_traj_batch, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
   int occ = 0;
   QS_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_traj_batch, 256, smem));
   if (occ < 1) return qs::fail(QSIM_ERR_CUDA, "trajectory batch does not fit on an SM");
   int64_t grid = (int64_t)bound.ctx->sms * occ;
   if (grid > shots) grid = shots;
-  k_traj_batch<<<(unsigned)grid, 256, smem, (cudaStream_t)stream>>>(
-      n_qubits, shots, n_ops, (const QsTrajOp*)ops, matrices, flips, flips_per_shot, (const qs_c128*)psi0,
-      (const qs_c128*)observable, out_fidelity, out_prob_sum, (qs_c128*)out_states);
-  g_launches.fetch_add(1, std::memory_order_relaxed);
-  QS_CUDA(cudaGetLastError());
-  return QSIM_OK;
+  k_traj_batch<<<(unsigned)grid, 256, smem, (cudaStream_t)stream>>>(n, shots, n_ops, ops, matrices, flips,
+                                                                    flips_per_shot, psi0, observable, out_fidelity,
+                                                                    out_prob_sum, out_states);
+  return launched();
 }
 
-// fills `sel` (positions ascending) from reference-style local qubit numbers
-static int swap_select(const char* who, int n_local, int nbits, const int* local_qubits, const int* bit_values,
-                       uint64_t first, uint64_t count, QsBitSel* sel) {
-  if (n_local < 1 || nbits < 1 || nbits > 8 || nbits > n_local || !local_qubits || !bit_values)
-    return qs::fail(QSIM_ERR_ARG, std::string(who) + ": bad bit list");
-  sel->k = nbits;
-  for (int i = 0; i < nbits; ++i) {
-    if (local_qubits[i] < 0 || local_qubits[i] >= n_local || (bit_values[i] | 1) != 1)
-      return qs::fail(QSIM_ERR_ARG, std::string(who) + ": bad qubit or bit");
-    sel->pos[i] = n_local - 1 - local_qubits[i];
-    sel->val[i] = bit_values[i];
-  }
-  for (int i = 1; i < nbits; ++i)                 // insertion sort by position
-    for (int j = i; j > 0 && sel->pos[j] < sel->pos[j - 1]; --j) {
-      std::swap(sel->pos[j], sel->pos[j - 1]);
-      std::swap(sel->val[j], sel->val[j - 1]);
-    }
-  for (int i = 1; i < nbits; ++i)
-    if (sel->pos[i] == sel->pos[i - 1]) return qs::fail(QSIM_ERR_ARG, std::string(who) + ": repeated qubit");
-  if (first + count > (1ull << (n_local - nbits)))
-    return qs::fail(QSIM_ERR_ARG, std::string(who) + ": chunk out of range");
-  return QSIM_OK;
-}
-
-int qsim_swap_pack(const void* shard, void* sendbuf, int n_local, int nbits, const int* local_qubits,
-                   const int* bit_values, uint64_t first, uint64_t count, void* stream) {
-  if (!shard || !sendbuf) return qs::fail(QSIM_ERR_ARG, "qsim_swap_pack: null argument");
-  QsBitSel sel;
-  int rc = swap_select("qsim_swap_pack", n_local, nbits, local_qubits, bit_values, first, count, &sel);
-  if (rc != QSIM_OK) return rc;
+int swap_pack(const qs_c128* shard, qs_c128* buf, const QsBitSel& sel, uint64_t first, uint64_t count, void* stream) {
   Bound bound;
-  rc = bind_device(shard, &bound);
+  int rc = bind_device(shard, &bound);
   DevCtx* ctx = bound.ctx;
   if (rc != QSIM_OK) return rc;
   if (count == 0) return QSIM_OK;
-  k_swap_pack<<<stream_grid(ctx, count, 256), 256, 0, (cudaStream_t)stream>>>(
-      (const qs_c128*)shard, (qs_c128*)sendbuf, sel, first, count);
-  g_launches.fetch_add(1, std::memory_order_relaxed);
-  QS_CUDA(cudaGetLastError());
-  return QSIM_OK;
+  k_swap_pack<<<stream_grid(ctx, count, 256), 256, 0, (cudaStream_t)stream>>>(shard, buf, sel, first, count);
+  return launched();
 }
 
-int qsim_swap_unpack(void* shard, const void* recvbuf, int n_local, int nbits, const int* local_qubits,
-                     const int* bit_values, uint64_t first, uint64_t count, void* stream) {
-  if (!shard || !recvbuf) return qs::fail(QSIM_ERR_ARG, "qsim_swap_unpack: null argument");
-  QsBitSel sel;
-  int rc = swap_select("qsim_swap_unpack", n_local, nbits, local_qubits, bit_values, first, count, &sel);
-  if (rc != QSIM_OK) return rc;
+int swap_unpack(qs_c128* shard, const qs_c128* buf, const QsBitSel& sel, uint64_t first, uint64_t count,
+                void* stream) {
   Bound bound;
-  rc = bind_device(shard, &bound);
+  int rc = bind_device(shard, &bound);
   DevCtx* ctx = bound.ctx;
   if (rc != QSIM_OK) return rc;
   if (count == 0) return QSIM_OK;
-  k_swap_unpack<<<stream_grid(ctx, count, 256), 256, 0, (cudaStream_t)stream>>>(
-      (qs_c128*)shard, (const qs_c128*)recvbuf, sel, first, count);
-  g_launches.fetch_add(1, std::memory_order_relaxed);
-  QS_CUDA(cudaGetLastError());
-  return QSIM_OK;
+  k_swap_unpack<<<stream_grid(ctx, count, 256), 256, 0, (cudaStream_t)stream>>>(shard, buf, sel, first, count);
+  return launched();
 }
 
-}  // extern "C"
+}  // namespace qs::dev

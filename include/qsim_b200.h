@@ -156,6 +156,35 @@ int qsim_expect_pauli(const void* state, int n_qubits, int64_t n_terms, const ui
 int qsim_expect_pauli_dm(const void* vec_rho, int n_qubits, int64_t n_terms, const uint64_t* x_masks,
                          const uint64_t* z_masks, double* out_re_im, void* stream);
 
+/* ---- measurement statistics: marginal probabilities and shot sampling -------------------
+ * Qubits are the reference's (qubit q is index bit n-1-q).  A marginal over qubits[0..k) has
+ * 2^k bins; bit k-1-j of the bin number is the value of qubits[j], so qubits[0] is the most
+ * significant bit (the marginal over qubits 0..19 of a 30-qubit ket is bench.py's
+ * `state_marginal`).  The probability of basis index i is |psi_i|^2 for a ket and Re rho[i, i]
+ * for the vec of an N-qubit density matrix.  The qubits must be distinct, 0 <= k <= n_qubits,
+ * 1 <= n_qubits <= 40 (N <= 31 for the _dm variants); anything else is QSIM_ERR_ARG.  Fixed grids
+ * and fixed summation / scan trees (no floating-point atomics): repeated calls on the same state
+ * give bit-identical marginals and identical outcomes. */
+/* out: DEVICE array of 2^k doubles, the raw sums (not normalised).  Does not synchronise. */
+int qsim_marginal_probs(const void* state, int n_qubits, int k, const int* qubits, double* out, void* stream);
+int qsim_marginal_probs_dm(const void* vec_rho, int n_qubits, int k, const int* qubits, double* out,
+                           void* stream);
+/* Inverse-CDF sampling of full basis indices.  For the caller's uniform u in [0, 1) (DEVICE array
+ * `uniforms`, `shots` doubles) the outcome is the smallest index i with cdf(i) > u * total, where
+ * total is the mass the call computed (a ket need not be normalised) and cdf uses the library's
+ * fixed summation order; an index with probability 0 is never drawn (a uniform that rounding
+ * places past the last nonzero probability takes that index).  For a density matrix a negative
+ * diagonal entry counts as 0.  out: DEVICE array of `shots` basis indices.  *total (host) gets the
+ * mass sampled from; returning it synchronises the stream.  A total <= 0 (or not finite) is
+ * QSIM_ERR_ARG; shots == 0 returns at once; shots must be below 2^31.  workspace: DEVICE buffer of
+ * at least qsim_sample_workspace_bytes(n_qubits, shots) bytes (N for the _dm variant), owned by
+ * the caller; a shorter one is QSIM_ERR_ARG. */
+int qsim_sample_workspace_bytes(int n_qubits, int64_t shots, uint64_t* out_bytes);
+int qsim_sample(const void* state, int n_qubits, int64_t shots, const double* uniforms, uint64_t* out,
+                double* total, void* workspace, uint64_t workspace_bytes, void* stream);
+int qsim_sample_dm(const void* vec_rho, int n_qubits, int64_t shots, const double* uniforms, uint64_t* out,
+                   double* total, void* workspace, uint64_t workspace_bytes, void* stream);
+
 /* ---- batched tiny-circuit executor (replaces the sample loop of
  *      PAPER/randomised_benchmarking.py:65-75) --------------------------------------
  * B independent registers of nq <= 2 qubits kept as density matrices (dim = 2^nq).

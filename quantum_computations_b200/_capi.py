@@ -78,6 +78,13 @@ SIGNATURES = {
     "qsim_expect_pauli": (C.c_int, [C.c_void_p, C.c_int, C.c_int64, C.c_void_p, C.c_void_p, c_double_p, C.c_void_p]),
     "qsim_expect_pauli_dm": (C.c_int, [C.c_void_p, C.c_int, C.c_int64, C.c_void_p, C.c_void_p, c_double_p,
                                        C.c_void_p]),
+    "qsim_marginal_probs": (C.c_int, [C.c_void_p, C.c_int, C.c_int, c_int_p, C.c_void_p, C.c_void_p]),
+    "qsim_marginal_probs_dm": (C.c_int, [C.c_void_p, C.c_int, C.c_int, c_int_p, C.c_void_p, C.c_void_p]),
+    "qsim_sample_workspace_bytes": (C.c_int, [C.c_int, C.c_int64, C.POINTER(C.c_uint64)]),
+    "qsim_sample": (C.c_int, [C.c_void_p, C.c_int, C.c_int64, C.c_void_p, C.c_void_p, c_double_p, C.c_void_p,
+                              C.c_uint64, C.c_void_p]),
+    "qsim_sample_dm": (C.c_int, [C.c_void_p, C.c_int, C.c_int64, C.c_void_p, C.c_void_p, c_double_p, C.c_void_p,
+                                 C.c_uint64, C.c_void_p]),
     "qsim_rb_batch": (C.c_int, [C.c_int, C.c_int64, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p,
                                 C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "qsim_traj_batch": (C.c_int, [C.c_int, C.c_int64, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64,

@@ -31,6 +31,12 @@ int expect_pauli(const qs_c128* state, int n, const PauliPlan& plan, int64_t n_t
 // xi, zi: index-bit masks per term; sums: 2 * n_terms doubles (re, im per term)
 int expect_pauli_dm(const qs_c128* rho, int n, int64_t n_terms, const uint64_t* xi, const uint64_t* zi,
                     double* sums, void* stream);
+// out: 2^G.k doubles (device memory for the CUDA library)
+int marginal_probs(const QsProbSrc& src, const QsMargGeom& G, double* out, void* stream);
+// n index bits; ws: the caller's workspace laid out by qs_sample_layout(n, shots); *total gets the
+// mass sampled from (the caller refuses a total that is not positive and finite)
+int sample(const QsProbSrc& src, int n, int64_t shots, const double* uniforms, uint64_t* out, double* total,
+           unsigned char* ws, void* stream);
 int rb_batch(int nq, int64_t n_seq, const uint16_t* opcodes, const int64_t* offsets, const double* superops,
              const double* unitaries, const double* rho0, const double* psi0, double* out_fidelity,
              double* out_purity, double* out_rho, void* stream);

@@ -3,6 +3,7 @@
 // libqsim_b200.so (CUDA) and the host emulator of the tests.  Each compute entry point checks
 // its arguments, turns reference qubits into index bits (qubit q of n is index bit n-1-q), does
 // any lowering on the host and hands the rest to the backend (backend.h).
+#include <algorithm>
 #include <cmath>
 #include <cstring>
 #include <new>
@@ -56,13 +57,100 @@ int swap_select(const char* who, int n_local, int nbits, const int* local_qubits
   return QSIM_OK;
 }
 
+// Checks a marginal's arguments and lays out its pass (elem_ops.h, QsMargGeom): lanes take index
+// bits 0..4; of the summed bits above them, the lowest are serial and the highest `gs` number the
+// partials, gs chosen so that about 2^15 warp tasks exist and bins x partials stay within
+// 2^QS_MARG_PARTIALS_LOG2 (k >= 20: no partials, the pass writes `out`).
+int marginal_geom(const char* who, int n, int max_n, int k, const int* qubits, QsMargGeom* G) {
+  const std::string w(who);
+  if (n < 1 || n > max_n) return qs::fail(QSIM_ERR_ARG, w + ": n_qubits must be in [1, " + std::to_string(max_n) + "]");
+  if (k < 0 || k > n) return qs::fail(QSIM_ERR_ARG, w + ": k must be in [0, n_qubits]");
+  int binpos[64];
+  for (int b = 0; b < 64; ++b) binpos[b] = -1;
+  for (int j = 0; j < k; ++j) {
+    if (qubits[j] < 0 || qubits[j] >= n) return qs::fail(QSIM_ERR_ARG, w + ": qubit out of range");
+    const int bit = n - 1 - qubits[j];
+    if (binpos[bit] >= 0) return qs::fail(QSIM_ERR_ARG, w + ": qubits must be distinct");
+    binpos[bit] = k - 1 - j;                   // qubits[0] is the most significant bin bit
+  }
+  memset(G, 0, sizeof(*G));
+  const int lane_log2 = n < 5 ? n : 5;
+  G->n = n;
+  G->k = k;
+  G->lanes = 1 << lane_log2;
+  int k_hi = 0, hs = 0, high_summed[64];
+  for (int b = lane_log2; b < n; ++b) {
+    if (binpos[b] >= 0) ++k_hi;
+    else high_summed[hs++] = b;
+  }
+  int gs = std::min(hs, std::min(std::max(0, 15 - k_hi), 14));
+  if (k + gs > QS_MARG_PARTIALS_LOG2) gs = std::max(0, QS_MARG_PARTIALS_LOG2 - k);
+  G->gs_bits = gs;
+  for (int i = 0; i < hs - gs; ++i) G->rmask |= 1ull << high_summed[i];
+  for (int b = lane_log2; b < n; ++b)
+    if (!(G->rmask >> b & 1)) G->gmask |= 1ull << b;
+  G->nserial = 1ull << (hs - gs);
+  G->ntasks = 1ull << (n - lane_log2 - (hs - gs));
+  for (int b = 0; b < lane_log2; ++b)
+    if (binpos[b] < 0) G->lane_sum |= 1u << b;
+  for (int l = 0; l < G->lanes; ++l)
+    for (int b = 0; b < lane_log2; ++b)
+      if (binpos[b] >= 0 && (l >> b & 1)) G->lane_slot[l] += 1ull << (binpos[b] + gs);
+  uint64_t contrib[64] = {0};                  // slot contribution of task bit b
+  for (int b = lane_log2, g = 0; b < n; ++b) {
+    if (binpos[b] >= 0) contrib[b] = 1ull << (binpos[b] + gs);
+    else if (!(G->rmask >> b & 1)) contrib[b] = 1ull << g++;
+  }
+  for (int t = 0; t < QS_MARG_TAB_BYTES; ++t)
+    for (int v = 0; v < 256; ++v)
+      for (int i = 0; i < 8; ++i)
+        if (v >> i & 1 && 5 + 8 * t + i < 64) G->tab[t][v] += contrib[5 + 8 * t + i];
+  return QSIM_OK;
+}
+
+int marginal(const char* who, const void* state, int n, int max_n, int k, const int* qubits, double* out, bool dm,
+             void* stream) {
+  if (!state || !out || (k > 0 && !qubits)) return qs::fail(QSIM_ERR_ARG, std::string(who) + ": null argument");
+  QsMargGeom G;
+  const int rc = marginal_geom(who, n, max_n, k, qubits, &G);
+  if (rc != QSIM_OK) return rc;
+  const QsProbSrc src{(const qs_c128*)state, dm ? (1ull << n) + 1ull : 1ull, dm ? 1 : 0};
+  return qs::dev::marginal_probs(src, G, out, stream);
+}
+
+int sample_bytes(const char* who, int n, int max_n, int64_t shots, uint64_t* bytes) {
+  const std::string w(who);
+  if (n < 1 || n > max_n) return qs::fail(QSIM_ERR_ARG, w + ": n_qubits must be in [1, " + std::to_string(max_n) + "]");
+  if (shots < 0 || shots >= (1ll << 31)) return qs::fail(QSIM_ERR_ARG, w + ": shots must be in [0, 2^31)");
+  *bytes = qs_sample_layout(n, (uint64_t)shots).bytes;
+  return QSIM_OK;
+}
+
+int sample(const char* who, const void* state, int n, int max_n, int64_t shots, const double* uniforms, uint64_t* out,
+           double* total, void* workspace, uint64_t workspace_bytes, bool dm, void* stream) {
+  uint64_t need = 0;
+  int rc = sample_bytes(who, n, max_n, shots, &need);
+  if (rc != QSIM_OK || shots == 0) return rc;
+  const std::string w(who);
+  if (!state || !uniforms || !out || !total || !workspace) return qs::fail(QSIM_ERR_ARG, w + ": null argument");
+  if (workspace_bytes < need)
+    return qs::fail(QSIM_ERR_ARG, w + ": workspace too small (" + std::to_string(need) + " bytes needed)");
+  const QsProbSrc src{(const qs_c128*)state, dm ? (1ull << n) + 1ull : 1ull, dm ? 1 : 0};
+  double t = 0.0;
+  rc = qs::dev::sample(src, n, shots, uniforms, out, &t, (unsigned char*)workspace, stream);
+  if (rc != QSIM_OK) return rc;
+  if (!(t > 0.0) || !std::isfinite(t)) return qs::fail(QSIM_ERR_ARG, w + ": the state has no probability mass");
+  *total = t;
+  return QSIM_OK;
+}
+
 }  // namespace
 
 extern "C" {
 
 const char* qsim_last_error(void) { return qs::last_error(); }
 
-int qsim_version(void) { return 101; }
+int qsim_version(void) { return 102; }
 
 int qsim_circuit_create(int n_qubits, qsim_circuit_t** out) {
   if (!out) return qs::fail(QSIM_ERR_ARG, "qsim_circuit_create: out is null");
@@ -322,6 +410,31 @@ int qsim_expect_pauli_dm(const void* vec_rho, int n_qubits, int64_t n_terms, con
   if (rc != QSIM_OK) return rc;
   qs::pauli_finish_dm(n_terms, phase, sums.data(), out_re_im);
   return QSIM_OK;
+}
+
+int qsim_marginal_probs(const void* state, int n_qubits, int k, const int* qubits, double* out, void* stream) {
+  return marginal("qsim_marginal_probs", state, n_qubits, 40, k, qubits, out, false, stream);
+}
+
+int qsim_marginal_probs_dm(const void* vec_rho, int n_qubits, int k, const int* qubits, double* out, void* stream) {
+  return marginal("qsim_marginal_probs_dm", vec_rho, n_qubits, 31, k, qubits, out, true, stream);
+}
+
+int qsim_sample_workspace_bytes(int n_qubits, int64_t shots, uint64_t* out_bytes) {
+  if (!out_bytes) return qs::fail(QSIM_ERR_ARG, "qsim_sample_workspace_bytes: null argument");
+  return sample_bytes("qsim_sample_workspace_bytes", n_qubits, 40, shots, out_bytes);
+}
+
+int qsim_sample(const void* state, int n_qubits, int64_t shots, const double* uniforms, uint64_t* out, double* total,
+                void* workspace, uint64_t workspace_bytes, void* stream) {
+  return sample("qsim_sample", state, n_qubits, 40, shots, uniforms, out, total, workspace, workspace_bytes, false,
+                stream);
+}
+
+int qsim_sample_dm(const void* vec_rho, int n_qubits, int64_t shots, const double* uniforms, uint64_t* out,
+                   double* total, void* workspace, uint64_t workspace_bytes, void* stream) {
+  return sample("qsim_sample_dm", vec_rho, n_qubits, 31, shots, uniforms, out, total, workspace, workspace_bytes, true,
+                stream);
 }
 
 int qsim_rb_batch(int nq, int64_t n_seq, const uint16_t* opcodes, const int64_t* offsets, int n_opcodes,

@@ -2,6 +2,8 @@
 // (grid-stride loops in kernels.cu) and the host emulator of the CPU tests.
 // Bit convention: reference qubit q of an n-qubit register is index bit n-1-q.
 #pragma once
+#include <cmath>
+
 #include "tile_exec.h"
 
 QS_HD qs_c128 qs_cmul(qs_c128 a, qs_c128 b) {
@@ -290,4 +292,192 @@ QS_HD qs_c128 qs_pauli_dm_elem(const qs_c128* __restrict__ rho, int N, uint64_t 
   qs_c128 v = rho[(c << N) | (c ^ x)];
   if (qs_par64(c & z)) { v.x = -v.x; v.y = -v.y; }
   return v;
+}
+
+// ---- measurement statistics (qsim_marginal_probs / qsim_sample and their _dm variants) ---------
+// The probability of basis index i: |a[i]|^2 for a ket (stride 1), Re a[i * stride] for the vec of
+// a density matrix (stride 2^N + 1 walks the diagonal).
+struct QsProbSrc { const qs_c128* a; uint64_t stride; int dm; };
+QS_HD double qs_prob(const QsProbSrc& s, uint64_t i) {
+  const qs_c128 v = s.a[i * s.stride];
+  return s.dm ? v.x : v.x * v.x + v.y * v.y;
+}
+// what sampling draws from: a negative diagonal entry (rounding) counts as 0
+QS_HD double qs_prob_clamped(const QsProbSrc& s, uint64_t i) {
+  const double p = qs_prob(s, i);
+  return p > 0.0 ? p : 0.0;
+}
+struct QsProbFn {
+  QsProbSrc s;
+  QS_HD double operator()(uint64_t i) const { return qs_prob(s, i); }
+};
+
+// Bits of v deposited, lowest first, into the set bits of mask.
+QS_HD uint64_t qs_deposit_mask(uint64_t v, uint64_t mask) {
+  uint64_t out = 0;
+  for (int b = 0; b < 64 && v; ++b)
+    if (mask >> b & 1ull) { out |= (v & 1ull) << b; v >>= 1; }
+  return out;
+}
+
+// Geometry of the marginal pass (built on the host, capi_host.cpp).  A warp task reads 32 lanes x
+// nserial probabilities: index bits 0..4 are the lane number whatever they are (every warp load
+// covers 512 contiguous bytes of a ket), the serial bits (rmask) are summed in registers and the
+// task bits (gmask) number the tasks.  Lane bits that are summed bits reduce by a shuffle-xor tree
+// (lane_sum); lane bits that are bin bits stay in separate lanes.  A task writes one value per bin
+// of its lanes, into slot lane_slot[lane] + slot(task), slot(task) being the task bits looked up
+// byte by byte in tab.  gs_bits == 0: the slot is the bin and the pass writes `out` itself.
+// Otherwise a slot is (bin << gs_bits | g), g = the task's summed task bits, and a final kernel
+// sums the 2^gs_bits partials of every bin in a fixed tree (qs_marg_final_ref).
+constexpr int QS_MARG_TAB_BYTES = 5;         // task bits 5 .. 44
+constexpr int QS_MARG_PARTIALS_LOG2 = 20;    // bins x partials per bin when gs_bits > 0
+struct QsMargGeom {
+  int32_t n, k, gs_bits, lanes;              // lanes = 2^min(n, 5)
+  uint32_t lane_sum, pad;
+  uint64_t rmask, gmask, nserial, ntasks;
+  uint64_t lane_slot[32];
+  uint64_t tab[QS_MARG_TAB_BYTES][256];
+};
+
+// Lane `lane`'s sum over the serial bits of the task at `base` (its task bits deposited): serial
+// element e (ascending index) goes to accumulator e & 7, eight loads in flight, and the eight
+// accumulators are added in a fixed tree.
+template <class P>
+QS_HD double qs_marg_lane(const QsMargGeom& G, const P& prob, uint64_t base, uint32_t lane) {
+  double acc[8] = {0.0, 0.0, 0.0, 0.0, 0.0, 0.0, 0.0, 0.0};
+  const uint64_t rm = G.rmask;
+  uint64_t s = 0;                             // next serial bits: submasks of rm in ascending order
+  if (G.nserial >= 8) {
+    for (uint64_t e = 0; e < G.nserial; e += 8) {
+      uint64_t idx[8];
+#pragma unroll
+      for (int u = 0; u < 8; ++u) { idx[u] = base | s | lane; s = (s - rm) & rm; }
+      double p[8];
+#pragma unroll
+      for (int u = 0; u < 8; ++u) p[u] = prob(idx[u]);
+#pragma unroll
+      for (int u = 0; u < 8; ++u) acc[u] += p[u];
+    }
+  } else {
+#pragma unroll
+    for (int u = 0; u < 8; ++u)
+      if ((uint64_t)u < G.nserial) { acc[u] += prob(base | s | lane); s = (s - rm) & rm; }
+  }
+  return ((acc[0] + acc[1]) + (acc[2] + acc[3])) + ((acc[4] + acc[5]) + (acc[6] + acc[7]));
+}
+
+QS_HD uint64_t qs_marg_task_slot(const QsMargGeom& G, uint64_t base) {
+  const uint64_t t = base >> 5;
+  uint64_t slot = 0;
+  for (int b = 0; b < QS_MARG_TAB_BYTES; ++b) slot += G.tab[b][(t >> (8 * b)) & 255u];
+  return slot;
+}
+
+// Inverse-CDF step of one level: the smallest s in [0, K) with X(s) > *t (binary search over the
+// level's inclusive scan X), and *t becomes the target inside s.  An s with mass(s) == 0 can only
+// come from rounding between differently ordered sums: then the next s with nonzero mass is taken
+// and the target becomes 0 (its first nonzero entry).  With no such s (the target at or past the
+// end of the scan, by rounding) the last s with nonzero mass is taken and the target becomes +inf
+// (its last nonzero entry).  The parent has nonzero mass, so one of its parts has.
+template <class FX, class FM>
+QS_HD int qs_cdf_pick(const FX& X, const FM& mass, int K, double* t) {
+  int lo = 0, hi = K;
+  while (lo < hi) {
+    const int mid = (lo + hi) >> 1;
+    if (X(mid) > *t) hi = mid;
+    else lo = mid + 1;
+  }
+  if (lo < K && mass(lo) > 0.0) {
+    if (lo > 0) *t = *t - X(lo - 1);           // >= 0: X(lo - 1) <= *t
+    return lo;
+  }
+  if (lo < K)
+    for (int r = lo + 1; r < K; ++r)
+      if (mass(r) > 0.0) { *t = 0.0; return r; }
+  for (int r = K - 1; r >= 0; --r)
+    if (mass(r) > 0.0) { *t = HUGE_VAL; return r; }
+  *t = HUGE_VAL;
+  return K - 1;
+}
+
+// Sampling: 256 amplitudes per sub-tile, 256 sub-tiles per chunk, up to 1024 shots per work item
+// of the resolving kernel.  The caller's workspace (byte offsets, 256-aligned) holds per sub-tile
+// and per chunk the masses, the chunk scan and the total, per chunk the shot counts, bucket ends and
+// work-item offsets, and per shot its chunk, its target inside the chunk and its bucketed order.
+constexpr int QS_SUB_LOG2 = 8, QS_CHUNK_LOG2 = 16, QS_SAMPLE_ITEM = 1024;
+struct QsSampleLayout {
+  uint64_t nchunks, sub_mass, chunk_mass, chunk_incl, total, counts, ends, items, shot_chunk, shot_t, order,
+      bytes;
+};
+inline QsSampleLayout qs_sample_layout(int n, uint64_t shots) {
+  QsSampleLayout L;
+  L.nchunks = n > QS_CHUNK_LOG2 ? 1ull << (n - QS_CHUNK_LOG2) : 1ull;
+  uint64_t off = 0;
+  auto take = [&off](uint64_t bytes) { const uint64_t at = off; off += (bytes + 255ull) & ~255ull; return at; };
+  L.sub_mass = take(8 * (L.nchunks << (QS_CHUNK_LOG2 - QS_SUB_LOG2)));
+  L.chunk_mass = take(8 * L.nchunks);
+  L.chunk_incl = take(8 * L.nchunks);
+  L.total = take(8);
+  L.counts = take(4 * L.nchunks);
+  L.ends = take(4 * L.nchunks);
+  L.items = take(4 * (L.nchunks + 1));
+  L.shot_chunk = take(4 * shots);
+  L.shot_t = take(8 * shots);
+  L.order = take(4 * shots);
+  L.bytes = off;
+  return L;
+}
+
+// ---- host reference of the kernels' summation orders (the emulator runs these) ------------------
+// Kogge-Stone inclusive scan of 32 values: what __shfl_up_sync gives lane by lane.
+inline void qs_ks32(double* x) {
+  for (int d = 1; d < 32; d <<= 1) {
+    double o[32];
+    for (int l = 0; l < 32; ++l) o[l] = x[l];
+    for (int l = d; l < 32; ++l) x[l] = o[l] + o[l - d];
+  }
+}
+
+// The library's inclusive scan of v[0 .. count) by `threads` threads (a multiple of 32, <= 1024):
+// thread r sums its segment [r * seg, (r + 1) * seg) serially (seg = ceil(count / threads)), the
+// thread totals are scanned by a Kogge-Stone tree inside each warp and the warp totals by the same
+// tree, and element i of segment r is excl(r) + its serial prefix, with
+// excl(r) = (warp's exclusive part) + (lane's exclusive part).
+inline void qs_scan_ref(const double* v, uint64_t count, int threads, double* incl) {
+  const uint64_t seg = (count + threads - 1) / threads;
+  double li[1024], wt[32];
+  for (int r = 0; r < threads; ++r) {
+    double s = 0.0;
+    for (uint64_t e = 0; e < seg; ++e)
+      if (r * seg + e < count) s += v[r * seg + e];
+    li[r] = s;
+  }
+  for (int w = 0; w < threads / 32; ++w) qs_ks32(li + 32 * w);
+  for (int w = 0; w < 32; ++w) wt[w] = w < threads / 32 ? li[32 * w + 31] : 0.0;
+  qs_ks32(wt);
+  for (int r = 0; r < threads; ++r) {
+    const int w = r >> 5, l = r & 31;
+    const double ex = (w ? wt[w - 1] : 0.0) + (l ? li[r - 1] : 0.0);
+    double s = 0.0;
+    for (uint64_t e = 0; e < seg; ++e)
+      if (r * seg + e < count) { s += v[r * seg + e]; incl[r * seg + e] = ex + s; }
+  }
+}
+
+// out[bin] of the final marginal kernel: thread r of 256 sums the partials r, r + 256, ... serially,
+// a shuffle-xor tree (16, 8, 4, 2, 1) combines each warp, and the 8 warp sums go in a fixed tree.
+inline double qs_marg_final_ref(const double* row, uint64_t count) {
+  double v[256], w[8];
+  for (int r = 0; r < 256; ++r) {
+    double s = 0.0;
+    for (uint64_t i = r; i < count; i += 256) s += row[i];
+    v[r] = s;
+  }
+  for (int off = 16; off > 0; off >>= 1) {
+    double o[256];
+    for (int r = 0; r < 256; ++r) o[r] = v[r];
+    for (int r = 0; r < 256; ++r) v[r] = o[r] + o[r ^ off];
+  }
+  for (int i = 0; i < 8; ++i) w[i] = v[32 * i];
+  return ((w[0] + w[1]) + (w[2] + w[3])) + ((w[4] + w[5]) + (w[6] + w[7]));
 }

@@ -269,6 +269,93 @@ int expect_pauli_dm(const qs_c128* rho, int n, int64_t n_terms, const uint64_t* 
   return QSIM_OK;
 }
 
+// The warp tasks of k_marginal one after the other, lane by lane, in the kernel's summation order
+// (the lane shuffle tree and the final sum as qs_marg_final_ref): bit-identical to the GPU.
+int marginal_probs(const QsProbSrc& src, const QsMargGeom& G, double* out, void*) {
+  const QsProbFn prob{src};
+  std::vector<double> partials;
+  if (G.gs_bits) partials.assign((size_t)1 << (G.k + G.gs_bits), 0.0);
+  double* dst = G.gs_bits ? partials.data() : out;
+  uint64_t base = 0;
+  for (uint64_t t = 0; t < G.ntasks; ++t) {
+    double v[32];
+    for (uint32_t l = 0; l < 32; ++l) v[l] = l < (uint32_t)G.lanes ? qs_marg_lane(G, prob, base, l) : 0.0;
+    for (int b = 0; b < 5; ++b)
+      if (G.lane_sum >> b & 1) {
+        double o[32];
+        for (int l = 0; l < 32; ++l) o[l] = v[l];
+        for (int l = 0; l < 32; ++l) v[l] = o[l] + o[l ^ (1 << b)];
+      }
+    const uint64_t slot = qs_marg_task_slot(G, base);
+    for (uint32_t l = 0; l < (uint32_t)G.lanes; ++l)
+      if ((l & G.lane_sum) == 0) dst[G.lane_slot[l] + slot] = v[l];
+    base = ((base | ~G.gmask) + 1) & G.gmask;
+  }
+  ++g_launches;
+  if (G.gs_bits) {
+    for (uint64_t b = 0; b < (1ull << G.k); ++b)
+      out[b] = qs_marg_final_ref(partials.data() + (b << G.gs_bits), 1ull << G.gs_bits);
+    ++g_launches;
+  }
+  return QSIM_OK;
+}
+
+// The six kernels of the CUDA sampler as host loops, with the same scans (qs_scan_ref) and the
+// same inverse-CDF steps (qs_cdf_pick): the same uniforms give the same outcomes.  The bucketing of
+// the shots by chunk and sub-tile only orders the work, so the loops here go shot by shot.
+int sample(const QsProbSrc& src, int n, int64_t shots, const double* uniforms, uint64_t* out, double* total,
+           unsigned char* ws, void*) {
+  const QsSampleLayout L = qs_sample_layout(n, (uint64_t)shots);
+  const uint64_t n_amps = 1ull << n, subs = 1ull << (QS_CHUNK_LOG2 - QS_SUB_LOG2);
+  double* sub_mass = (double*)(ws + L.sub_mass);
+  double* chunk_mass = (double*)(ws + L.chunk_mass);
+  double* chunk_incl = (double*)(ws + L.chunk_incl);
+  double* shot_t = (double*)(ws + L.shot_t);
+  uint32_t* shot_chunk = (uint32_t*)(ws + L.shot_chunk);
+  auto sub_probs = [&](uint64_t c, uint64_t s, double* p) {
+    for (int e = 0; e < 256; ++e) {
+      const uint64_t i = (c << QS_CHUNK_LOG2) | (s << QS_SUB_LOG2) | (uint64_t)e;
+      p[e] = i < n_amps ? qs_prob_clamped(src, i) : 0.0;
+    }
+  };
+  double p[256], incl[256];
+  for (uint64_t c = 0; c < L.nchunks; ++c) {             // k_sample_masses
+    for (uint64_t s = 0; s < subs; ++s) {
+      sub_probs(c, s, p);
+      qs_scan_ref(p, 256, 32, incl);
+      sub_mass[c * subs + s] = incl[255];
+    }
+    qs_scan_ref(sub_mass + c * subs, subs, 32, incl);
+    chunk_mass[c] = incl[255];
+  }
+  qs_scan_ref(chunk_mass, L.nchunks, 1024, chunk_incl);   // k_sample_scan
+  const double tot = chunk_incl[L.nchunks - 1];
+  *total = tot;
+  g_launches += 6;
+  if (!(tot > 0.0) || !std::isfinite(tot)) return QSIM_OK;
+  const int K = (int)L.nchunks;
+  for (int64_t i = 0; i < shots; ++i) {                    // k_sample_locate
+    double t = uniforms[i] * tot;
+    shot_chunk[i] = (uint32_t)qs_cdf_pick([&](int c) { return chunk_incl[c]; }, [&](int c) { return chunk_mass[c]; },
+                                          K, &t);
+    shot_t[i] = t;
+  }
+  uint64_t cached = ~0ull;
+  double sub_incl[256];
+  for (int64_t i = 0; i < shots; ++i) {                    // k_sample_resolve
+    const uint64_t c = shot_chunk[i];
+    const double* sm = sub_mass + c * subs;
+    if (c != cached) { qs_scan_ref(sm, subs, 32, sub_incl); cached = c; }
+    double t = shot_t[i];
+    const int s = qs_cdf_pick([&](int j) { return sub_incl[j]; }, [&](int j) { return sm[j]; }, 256, &t);
+    sub_probs(c, (uint64_t)s, p);
+    qs_scan_ref(p, 256, 32, incl);
+    const int j = qs_cdf_pick([&](int e) { return incl[e]; }, [&](int e) { return p[e]; }, 256, &t);
+    out[i] = (c << QS_CHUNK_LOG2) | ((uint64_t)s << QS_SUB_LOG2) | (uint64_t)j;
+  }
+  return QSIM_OK;
+}
+
 int rb_batch(int nq, int64_t n_seq, const uint16_t* opcodes, const int64_t* offsets, const double* superops,
              const double* unitaries, const double* rho0, const double* psi0, double* out_fidelity,
              double* out_purity, double* out_rho, void*) {

@@ -46,6 +46,11 @@ struct DevCtx {
   double* h_pauli_sums = nullptr;       // pinned [terms][2]
   uint64_t* d_pauli_masks = nullptr;    // [terms][2] (density matrices: x, z)
   size_t pauli_partials_cap = 0, pauli_terms_cap = 0;
+  // partials of the marginals with few bins (2^QS_MARG_PARTIALS_LOG2 doubles, allocated at the first
+  // such call).  A marginal does not synchronise: the next one waits on the device for marg_done.
+  std::mutex marg_lock;
+  double* d_marg_partials = nullptr;
+  cudaEvent_t marg_done = nullptr;
   std::mutex occ_lock;
   int occ[12] = {0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0};   // resident CTAs/SM of the k_tile_pass variants at the last smem size
   int occ_smem = -1;
@@ -768,6 +773,341 @@ void launch_pauli_pass(const QsPauliPass& P, const qs_c128* state, uint64_t coun
 }
 
 // =====================================================================================
+// Marginal probabilities (elem_ops.h, QsMargGeom): one read-only pass, then a fixed-tree final sum
+// =====================================================================================
+constexpr int kMargThreads = 256;
+constexpr int kMargWarpsPerSM = 64;
+
+// Warp w takes the tasks [w * per_warp, (w + 1) * per_warp): each lane sums its serial elements
+// (qs_marg_lane), the summed lane bits reduce by shuffles, and the lanes that stand for a bin
+// write it to dst (out, or the partials).
+__global__ void __launch_bounds__(kMargThreads)
+k_marginal(const __grid_constant__ QsMargGeom G, QsProbSrc src, double* __restrict__ dst, uint64_t per_warp) {
+  const uint32_t lane = threadIdx.x & 31u;
+  const uint64_t warp = (blockIdx.x * (uint64_t)kMargThreads + threadIdx.x) >> 5;
+  const uint64_t t0 = warp * per_warp;
+  if (t0 >= G.ntasks) return;
+  const uint64_t t1 = t0 + per_warp < G.ntasks ? t0 + per_warp : G.ntasks;
+  const bool active = lane < (uint32_t)G.lanes;
+  const bool writer = active && (lane & G.lane_sum) == 0u;
+  const uint64_t lslot = G.lane_slot[lane];
+  const QsProbFn prob{src};
+  uint64_t base = qs_deposit_mask(t0, G.gmask);
+#pragma unroll 2
+  for (uint64_t t = t0; t < t1; ++t) {
+    double v = active ? qs_marg_lane(G, prob, base, lane) : 0.0;
+#pragma unroll
+    for (int b = 0; b < 5; ++b)
+      if (G.lane_sum >> b & 1u) v += __shfl_xor_sync(0xffffffffu, v, 1 << b);
+    if (writer) dst[lslot + qs_marg_task_slot(G, base)] = v;
+    base = ((base | ~G.gmask) + 1ull) & G.gmask;
+  }
+}
+
+// out[b] = the 2^gs_bits partials of bin b in the tree of qs_marg_final_ref.
+__global__ void __launch_bounds__(256)
+k_marg_final(const double* __restrict__ partials, int gs_bits, uint64_t bins, double* __restrict__ out) {
+  __shared__ double w[8];
+  const uint64_t per = 1ull << gs_bits;
+  for (uint64_t b = blockIdx.x; b < bins; b += gridDim.x) {
+    const double* row = partials + (b << gs_bits);
+    double s = 0.0;
+    for (uint64_t i = threadIdx.x; i < per; i += 256) s += row[i];
+#pragma unroll
+    for (int off = 16; off > 0; off >>= 1) s += __shfl_xor_sync(0xffffffffu, s, off);
+    if ((threadIdx.x & 31u) == 0) w[threadIdx.x >> 5] = s;
+    __syncthreads();
+    if (threadIdx.x == 0) out[b] = ((w[0] + w[1]) + (w[2] + w[3])) + ((w[4] + w[5]) + (w[6] + w[7]));
+    __syncthreads();
+  }
+}
+
+// =====================================================================================
+// Shot sampling: two-level inverse CDF (elem_ops.h: layout, qs_scan_ref orders, qs_cdf_pick)
+// =====================================================================================
+// Kogge-Stone inclusive scan over the lanes (qs_ks32).
+__device__ __forceinline__ double warp_ks32(double x) {
+  const int lane = threadIdx.x & 31;
+#pragma unroll
+  for (int d = 1; d < 32; d <<= 1) {
+    const double y = __shfl_up_sync(0xffffffffu, x, d);
+    if (lane >= d) x = x + y;
+  }
+  return x;
+}
+
+// qs_scan_ref(v, 256, 32): v[e] is at v[e + (e >> 3)] (padded: lane l reads its eight values
+// without bank conflicts); incl[m] = inclusive value of element 8 * lane + m.
+__device__ __forceinline__ void warp_scan256(const double* v, double incl[8]) {
+  const int lane = threadIdx.x & 31;
+  double s = 0.0;
+#pragma unroll
+  for (int m = 0; m < 8; ++m) { s += v[9 * lane + m]; incl[m] = s; }
+  const double li = warp_ks32(s);
+  double ex = __shfl_up_sync(0xffffffffu, li, 1);
+  ex = 0.0 + (lane ? ex : 0.0);
+#pragma unroll
+  for (int m = 0; m < 8; ++m) incl[m] = ex + incl[m];
+}
+
+// The 256 probabilities of sub-tile (c, s) into the warp's padded buffer (coalesced loads).
+__device__ __forceinline__ void load_sub(const QsProbSrc& src, uint64_t n_amps, uint64_t c, uint64_t s, double* pb) {
+  const int lane = threadIdx.x & 31;
+  const uint64_t base = (c << QS_CHUNK_LOG2) | (s << QS_SUB_LOG2);
+  double p[8];
+#pragma unroll
+  for (int m = 0; m < 8; ++m) {
+    const uint64_t i = base + (uint64_t)(32 * m + lane);
+    p[m] = i < n_amps ? qs_prob_clamped(src, i) : 0.0;
+  }
+#pragma unroll
+  for (int m = 0; m < 8; ++m) {
+    const int e = 32 * m + lane;
+    pb[e + (e >> 3)] = p[m];
+  }
+  __syncwarp();
+}
+
+// Pass 1: every sub-tile's mass and every chunk's mass (the totals of their qs_scan_ref scans).
+__global__ void __launch_bounds__(256)
+k_sample_masses(QsProbSrc src, uint64_t n_amps, uint64_t nchunks, double* __restrict__ sub_mass,
+                double* __restrict__ chunk_mass) {
+  __shared__ double pb[8][288];
+  __shared__ double sm[288];
+  const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
+  double incl[8];
+  for (uint64_t c = blockIdx.x; c < nchunks; c += gridDim.x) {
+    for (int s = w; s < 256; s += 8) {
+      load_sub(src, n_amps, c, (uint64_t)s, pb[w]);
+      warp_scan256(pb[w], incl);
+      if (lane == 31) { sub_mass[(c << 8) + s] = incl[7]; sm[s + (s >> 3)] = incl[7]; }
+      __syncwarp();
+    }
+    __syncthreads();
+    if (w == 0) {
+      warp_scan256(sm, incl);
+      if (lane == 31) chunk_mass[c] = incl[7];
+    }
+    __syncthreads();
+  }
+}
+
+// Pass 2 (one CTA of 1024): the chunk scan qs_scan_ref(chunk_mass, nchunks, 1024) and the total.
+__global__ void __launch_bounds__(1024)
+k_sample_scan(const double* __restrict__ cm, uint64_t count, double* __restrict__ incl, double* __restrict__ total) {
+  __shared__ double wt[32];
+  const int r = threadIdx.x, lane = r & 31, w = r >> 5;
+  const uint64_t seg = (count + 1023) / 1024;
+  double s = 0.0;
+  for (uint64_t e = 0; e < seg; ++e)
+    if (r * seg + e < count) s += cm[r * seg + e];
+  const double li = warp_ks32(s);
+  if (lane == 31) wt[w] = li;
+  __syncthreads();
+  if (w == 0) {
+    const double x = warp_ks32(wt[lane]);
+    wt[lane] = x;
+  }
+  __syncthreads();
+  double lex = __shfl_up_sync(0xffffffffu, li, 1);
+  const double ex = (w ? wt[w - 1] : 0.0) + (lane ? lex : 0.0);
+  s = 0.0;
+  for (uint64_t e = 0; e < seg; ++e) {
+    const uint64_t i = r * seg + e;
+    if (i < count) {
+      s += cm[i];
+      incl[i] = ex + s;
+      if (i == count - 1) *total = ex + s;
+    }
+  }
+}
+
+__device__ __forceinline__ bool sample_total_ok(double t) { return t > 0.0 && t < HUGE_VAL; }
+
+// atomicAdd(counter, 1) for every calling lane, one atomic per distinct counter in the warp: a
+// concentrated distribution sends all shots to one counter, and same-address atomics serialise.
+// Returns the lane's old value (its slot).
+__device__ __forceinline__ uint32_t warp_claim(uint32_t* counter) {
+  const unsigned peers = __match_any_sync(__activemask(), (unsigned long long)counter);
+  const int lane = threadIdx.x & 31, leader = __ffs(peers) - 1;
+  uint32_t base = 0;
+  if (lane == leader) base = atomicAdd(counter, (uint32_t)__popc(peers));
+  base = __shfl_sync(peers, base, leader);
+  return base + (uint32_t)__popc(peers & ((1u << lane) - 1u));
+}
+
+// Pass 3: every shot's chunk (first inverse-CDF level) and its target inside it; shot counts per chunk.
+__global__ void __launch_bounds__(256)
+k_sample_locate(const double* __restrict__ u, uint64_t shots, const double* __restrict__ chunk_incl,
+                const double* __restrict__ chunk_mass, int nchunks, const double* __restrict__ total,
+                uint32_t* __restrict__ shot_chunk, double* __restrict__ shot_t, uint32_t* __restrict__ counts) {
+  const double tot = *total;
+  if (!sample_total_ok(tot)) return;         // refused on the host
+  for (uint64_t i = blockIdx.x * (uint64_t)blockDim.x + threadIdx.x; i < shots; i += (uint64_t)gridDim.x * blockDim.x) {
+    double t = u[i] * tot;
+    const int c = qs_cdf_pick([&](int j) { return chunk_incl[j]; }, [&](int j) { return chunk_mass[j]; }, nchunks, &t);
+    shot_chunk[i] = (uint32_t)c;
+    shot_t[i] = t;
+    warp_claim(counts + c);                   // integer counts: exact in any order
+  }
+}
+
+// Exclusive block scan of one unsigned value per thread (blockDim.x a multiple of 32); *sum = the total.
+__device__ __forceinline__ uint32_t block_exscan_u32(uint32_t v, uint32_t* wt, uint32_t* sum) {
+  const int lane = threadIdx.x & 31, w = threadIdx.x >> 5, nw = blockDim.x >> 5;
+  uint32_t x = v;
+#pragma unroll
+  for (int d = 1; d < 32; d <<= 1) {
+    const uint32_t y = __shfl_up_sync(0xffffffffu, x, d);
+    if (lane >= d) x += y;
+  }
+  if (lane == 31) wt[w] = x;
+  __syncthreads();
+  if (w == 0) {
+    uint32_t z = lane < nw ? wt[lane] : 0u;
+#pragma unroll
+    for (int d = 1; d < 32; d <<= 1) {
+      const uint32_t y = __shfl_up_sync(0xffffffffu, z, d);
+      if (lane >= d) z += y;
+    }
+    if (lane < nw) wt[lane] = z;
+  }
+  __syncthreads();
+  const uint32_t ex = (w ? wt[w - 1] : 0u) + x - v;
+  *sum = wt[nw - 1];
+  __syncthreads();
+  return ex;
+}
+
+// Pass 4 (one CTA of 1024): bucket starts per chunk (written to `ends`, which the scatter advances
+// to the bucket ends) and work-item offsets (ceil(count / QS_SAMPLE_ITEM) items per chunk).
+__global__ void __launch_bounds__(1024)
+k_sample_offsets(const uint32_t* __restrict__ counts, uint64_t nchunks, uint32_t* __restrict__ ends,
+                 uint32_t* __restrict__ items) {
+  __shared__ uint32_t wt[32];
+  const int r = threadIdx.x;
+  const uint64_t seg = (nchunks + 1023) / 1024;
+  uint32_t a = 0, b = 0;
+  for (uint64_t e = 0; e < seg; ++e)
+    if (r * seg + e < nchunks) {
+      const uint32_t c = counts[r * seg + e];
+      a += c;
+      b += (c + QS_SAMPLE_ITEM - 1) / QS_SAMPLE_ITEM;
+    }
+  uint32_t tot_a, tot_b;
+  uint32_t xa = block_exscan_u32(a, wt, &tot_a);
+  uint32_t xb = block_exscan_u32(b, wt, &tot_b);
+  for (uint64_t e = 0; e < seg; ++e) {
+    const uint64_t i = r * seg + e;
+    if (i < nchunks) {
+      const uint32_t c = counts[i];
+      ends[i] = xa;
+      items[i] = xb;
+      xa += c;
+      xb += (c + QS_SAMPLE_ITEM - 1) / QS_SAMPLE_ITEM;
+    }
+  }
+  if (r == 0) items[nchunks] = tot_b;
+}
+
+// Pass 5: the shots bucketed by chunk (the order inside a bucket does not matter: every outcome is a
+// function of its own uniform).
+__global__ void __launch_bounds__(256)
+k_sample_scatter(uint64_t shots, const uint32_t* __restrict__ shot_chunk, uint32_t* __restrict__ ends,
+                 uint32_t* __restrict__ order) {
+  for (uint64_t i = blockIdx.x * (uint64_t)blockDim.x + threadIdx.x; i < shots; i += (uint64_t)gridDim.x * blockDim.x)
+    order[warp_claim(ends + shot_chunk[i])] = (uint32_t)i;
+}
+
+struct ResolveSmem {
+  double sm[288];                       // the chunk's sub-tile masses (padded)
+  double sincl[256];                    // their scan
+  double pb[8][288];                    // per warp: a sub-tile's probabilities (padded)
+  double ib[8][256];                    // per warp: their scan
+  double tl[QS_SAMPLE_ITEM];            // per shot slot: target inside its sub-tile
+  uint32_t shot[QS_SAMPLE_ITEM];
+  uint16_t bucket[QS_SAMPLE_ITEM];      // shot slots bucketed by sub-tile
+  uint8_t sub[QS_SAMPLE_ITEM];
+  uint32_t cnt[256], start[257], wt[32];
+};
+
+// Pass 6: work item = up to QS_SAMPLE_ITEM shots of one chunk.  The shots find their sub-tile
+// (second level, from the stored sub-tile masses), are bucketed by it in shared memory, and only the
+// sub-tiles that hold shots are read again: each is scanned by one warp, which then resolves its
+// shots by binary search.  Heavy chunks (a basis state, GHZ) simply have many work items.
+__global__ void __launch_bounds__(256)
+k_sample_resolve(QsProbSrc src, uint64_t n_amps, uint64_t nchunks, const double* __restrict__ sub_mass,
+                 const uint32_t* __restrict__ counts, const uint32_t* __restrict__ ends,
+                 const uint32_t* __restrict__ items, const uint32_t* __restrict__ order,
+                 const double* __restrict__ shot_t, uint64_t* __restrict__ out) {
+  extern __shared__ __align__(16) unsigned char qs_resolve_smem[];
+  ResolveSmem& S = *reinterpret_cast<ResolveSmem*>(qs_resolve_smem);
+  const int tid = threadIdx.x, lane = tid & 31, w = tid >> 5;
+  const uint32_t n_items = items[nchunks];
+  double incl[8];
+  for (uint32_t item = blockIdx.x; item < n_items; item += gridDim.x) {
+    uint64_t lo = 0, hi = nchunks;          // the chunk: the last c with items[c] <= item
+    while (hi - lo > 1) {
+      const uint64_t mid = (lo + hi) >> 1;
+      if (items[mid] <= item) lo = mid;
+      else hi = mid;
+    }
+    const uint64_t c = lo;
+    const uint32_t j0 = (item - items[c]) * QS_SAMPLE_ITEM;
+    const uint32_t first = ends[c] - counts[c] + j0;
+    const uint32_t len = min((uint32_t)QS_SAMPLE_ITEM, counts[c] - j0);
+    S.sm[tid + (tid >> 3)] = sub_mass[(c << 8) + tid];
+    S.cnt[tid] = 0;
+    __syncthreads();
+    if (w == 0) {
+      warp_scan256(S.sm, incl);
+#pragma unroll
+      for (int m = 0; m < 8; ++m) S.sincl[8 * lane + m] = incl[m];
+    }
+    __syncthreads();
+    for (uint32_t q = tid; q < len; q += 256) {
+      const uint32_t i = order[first + q];
+      double t = shot_t[i];
+      const int s = qs_cdf_pick([&](int j) { return S.sincl[j]; }, [&](int j) { return S.sm[j + (j >> 3)]; }, 256, &t);
+      S.shot[q] = i;
+      S.tl[q] = t;
+      S.sub[q] = (uint8_t)s;
+      warp_claim(&S.cnt[s]);
+    }
+    __syncthreads();
+    {
+      uint32_t total;
+      const uint32_t ex = block_exscan_u32(S.cnt[tid], S.wt, &total);
+      S.start[tid] = ex;
+      if (tid == 0) S.start[256] = total;
+      S.cnt[tid] = ex;                       // from here on: bucket cursors
+    }
+    __syncthreads();
+    for (uint32_t q = tid; q < len; q += 256) S.bucket[warp_claim(&S.cnt[S.sub[q]])] = (uint16_t)q;
+    __syncthreads();
+    for (int s = w; s < 256; s += 8) {
+      const uint32_t b0 = S.start[s], b1 = S.start[s + 1];
+      if (b0 == b1) continue;
+      load_sub(src, n_amps, c, (uint64_t)s, S.pb[w]);
+      warp_scan256(S.pb[w], incl);
+#pragma unroll
+      for (int m = 0; m < 8; ++m) S.ib[w][8 * lane + m] = incl[m];
+      __syncwarp();
+      const double* ib = S.ib[w];
+      const double* pb = S.pb[w];
+      for (uint32_t q = b0 + lane; q < b1; q += 32) {
+        const uint32_t slot = S.bucket[q];
+        double t = S.tl[slot];
+        const int j = qs_cdf_pick([&](int e) { return ib[e]; }, [&](int e) { return pb[e + (e >> 3)]; }, 256, &t);
+        out[S.shot[slot]] = (c << QS_CHUNK_LOG2) | ((uint64_t)s << QS_SUB_LOG2) | (uint64_t)j;
+      }
+      __syncwarp();
+    }
+    __syncthreads();
+  }
+}
+
+// =====================================================================================
 // Batched tiny-circuit executor
 // =====================================================================================
 template <int DIM>
@@ -1262,6 +1602,78 @@ int expect_pauli_dm(const qs_c128* rho, int n, int64_t n_terms, const uint64_t* 
   rc = launched();
   if (rc != QSIM_OK) return rc;
   return pauli_sums_to_host(ctx, n_terms, (int)bx, sums, st);
+}
+
+int marginal_probs(const QsProbSrc& src, const QsMargGeom& G, double* out, void* stream) {
+  Bound bound;
+  int rc = bind_device(src.a, &bound);
+  DevCtx* ctx = bound.ctx;
+  if (rc != QSIM_OK) return rc;
+  const cudaStream_t st = (cudaStream_t)stream;
+  const uint64_t warps = std::min<uint64_t>(G.ntasks, (uint64_t)ctx->sms * kMargWarpsPerSM);
+  const uint64_t blocks = (warps + kMargThreads / 32 - 1) / (kMargThreads / 32);
+  const uint64_t slots = blocks * (kMargThreads / 32);
+  const uint64_t per_warp = (G.ntasks + slots - 1) / slots;
+  if (G.gs_bits == 0) {
+    k_marginal<<<(unsigned)blocks, kMargThreads, 0, st>>>(G, src, out, per_warp);
+    return launched();
+  }
+  std::lock_guard<std::mutex> guard(ctx->marg_lock);
+  if (!ctx->marg_done) QS_CUDA(cudaEventCreateWithFlags(&ctx->marg_done, cudaEventDisableTiming));
+  if (!ctx->d_marg_partials) QS_CUDA(cudaMalloc(&ctx->d_marg_partials, sizeof(double) << QS_MARG_PARTIALS_LOG2));
+  QS_CUDA(cudaStreamWaitEvent(st, ctx->marg_done, 0));     // the previous marginal's final sum has read them
+  k_marginal<<<(unsigned)blocks, kMargThreads, 0, st>>>(G, src, ctx->d_marg_partials, per_warp);
+  const uint64_t bins = 1ull << G.k;
+  const unsigned grid = (unsigned)std::min<uint64_t>(bins, (uint64_t)ctx->sms * 8);
+  k_marg_final<<<grid, 256, 0, st>>>(ctx->d_marg_partials, G.gs_bits, bins, out);
+  rc = launched(2);
+  if (rc != QSIM_OK) return rc;
+  QS_CUDA(cudaEventRecord(ctx->marg_done, st));
+  return QSIM_OK;
+}
+
+int sample(const QsProbSrc& src, int n, int64_t shots, const double* uniforms, uint64_t* out, double* total,
+           unsigned char* ws, void* stream) {
+  Bound bound;
+  int rc = bind_device(src.a, &bound);
+  DevCtx* ctx = bound.ctx;
+  if (rc != QSIM_OK) return rc;
+  const cudaStream_t st = (cudaStream_t)stream;
+  const QsSampleLayout L = qs_sample_layout(n, (uint64_t)shots);
+  double* sub_mass = (double*)(ws + L.sub_mass);
+  double* chunk_mass = (double*)(ws + L.chunk_mass);
+  double* chunk_incl = (double*)(ws + L.chunk_incl);
+  double* d_total = (double*)(ws + L.total);
+  uint32_t* counts = (uint32_t*)(ws + L.counts);
+  uint32_t* ends = (uint32_t*)(ws + L.ends);
+  uint32_t* items = (uint32_t*)(ws + L.items);
+  uint32_t* shot_chunk = (uint32_t*)(ws + L.shot_chunk);
+  double* shot_t = (double*)(ws + L.shot_t);
+  uint32_t* order = (uint32_t*)(ws + L.order);
+  const uint64_t n_amps = 1ull << n, nchunks = L.nchunks;
+  const int smem = (int)sizeof(ResolveSmem);
+  QS_CUDA(cudaFuncSetAttribute(k_sample_resolve, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+  int occ = 0;
+  QS_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_sample_resolve, 256, smem));
+  if (occ < 1) return qs::fail(QSIM_ERR_CUDA, "sample resolve kernel does not fit on an SM");
+  QS_CUDA(cudaMemsetAsync(counts, 0, sizeof(uint32_t) * nchunks, st));
+  const unsigned shot_grid = stream_grid(ctx, (uint64_t)shots, 256);
+  k_sample_masses<<<(unsigned)std::min<uint64_t>(nchunks, (uint64_t)ctx->sms * 8), 256, 0, st>>>(
+      src, n_amps, nchunks, sub_mass, chunk_mass);
+  k_sample_scan<<<1, 1024, 0, st>>>(chunk_mass, nchunks, chunk_incl, d_total);
+  k_sample_locate<<<shot_grid, 256, 0, st>>>(uniforms, (uint64_t)shots, chunk_incl, chunk_mass, (int)nchunks, d_total,
+                                             shot_chunk, shot_t, counts);
+  k_sample_offsets<<<1, 1024, 0, st>>>(counts, nchunks, ends, items);
+  k_sample_scatter<<<shot_grid, 256, 0, st>>>((uint64_t)shots, shot_chunk, ends, order);
+  k_sample_resolve<<<(unsigned)(ctx->sms * occ), 256, smem, st>>>(src, n_amps, nchunks, sub_mass, counts, ends, items,
+                                                                  order, shot_t, out);
+  rc = launched(6);
+  if (rc != QSIM_OK) return rc;
+  std::lock_guard<std::mutex> guard(ctx->reduce_lock);      // guards the pinned word
+  QS_CUDA(cudaMemcpyAsync(ctx->h_out, d_total, sizeof(double), cudaMemcpyDeviceToHost, st));
+  QS_CUDA(cudaStreamSynchronize(st));
+  *total = ctx->h_out[0];
+  return QSIM_OK;
 }
 
 int rb_batch(int nq, int64_t n_seq, const uint16_t* opcodes, const int64_t* offsets, const double* superops,

@@ -435,6 +435,82 @@ class DeviceState:
         return out
 
 
+    # -- measurement statistics ------------------------------------------------------------------
+    def probabilities(self, qubits=None, *, device: bool = False):
+        """Marginal distribution over ``qubits`` (default: all qubits): 2^k float64 entries, bit
+        k-1-j of the entry number is the value of ``qubits[j]`` (``qubits[0]`` most significant).
+        |psi_i|^2 for a ket, Re rho[i, i] for a density matrix, not normalised.  ``device=True``
+        returns the device array instead of a NumPy copy."""
+        n = self.num_qubits
+        q = _qubit_list(qubits, n)
+        out = marginal_probs(self.backend, self.buf, n, q, self.ndim == 2)
+        return out if device else self.backend.download(out)
+
+    def sample(self, shots: int, qubits=None, *, rng=None) -> np.ndarray:
+        """``shots`` measurement outcomes over ``qubits`` (default: all) as int64, ``qubits[0]``
+        the most significant bit.  Uniforms come from ``rng.random(shots)`` on the host (``rng``: a
+        ``np.random.Generator``, a seed, or None for ``default_rng()``); full basis indices are
+        drawn by inverse-CDF sampling on the device (``qsim_sample``) and projected on the qubits.
+        The state is left unchanged."""
+        n = self.num_qubits
+        q = _qubit_list(qubits, n)
+        gen = rng if isinstance(rng, np.random.Generator) else np.random.default_rng(rng)
+        u = gen.random(int(shots))
+        idx, _total = sample_indices(self.backend, self.buf, n, u, self.ndim == 2)
+        return project_outcomes(idx, n, q)
+
+
+def _qubit_list(qubits, n: int) -> list:
+    q = list(range(n)) if qubits is None else [int(v) for v in qubits]
+    if any(not 0 <= v < n for v in q):
+        raise ValueError("qubit out of range")
+    if len(set(q)) != len(q):
+        raise ValueError("qubits must be distinct")
+    return q
+
+
+def marginal_probs(backend, buf, n: int, qubits, dm: bool = False):
+    """``qsim_marginal_probs`` (``_dm``) of the buffer over reference qubits ``qubits`` of an
+    n-qubit register: a new device array of 2^len(qubits) doubles."""
+    q = np.ascontiguousarray(qubits, dtype=np.int32)
+    out = backend.zeros(1 << len(q), np.float64)
+    fn = backend.lib.qsim_marginal_probs_dm if dm else backend.lib.qsim_marginal_probs
+    _capi.check(backend.lib, fn(backend.ptr(buf), n, len(q), q.ctypes.data_as(_capi.c_int_p), backend.ptr(out),
+                                backend.stream()))
+    return out
+
+
+def sample_indices(backend, buf, n: int, uniforms: np.ndarray, dm: bool = False):
+    """``qsim_sample`` (``_dm``) with the host uniforms uploaded: (int64 basis indices on the host,
+    the total mass sampled from)."""
+    u = np.ascontiguousarray(uniforms, dtype=np.float64).reshape(-1)
+    shots = len(u)
+    if shots == 0:
+        return np.zeros(0, dtype=np.int64), 0.0
+    lib = backend.lib
+    need = C.c_uint64()
+    _capi.check(lib, lib.qsim_sample_workspace_bytes(n, shots, C.byref(need)))
+    ws = backend.zeros(int(need.value), np.uint8)
+    du = backend.upload(u)
+    out = backend.zeros(shots, np.int64)                 # uint64 indices < 2^40: the same bits
+    total = C.c_double()
+    fn = lib.qsim_sample_dm if dm else lib.qsim_sample
+    _capi.check(lib, fn(backend.ptr(buf), n, shots, backend.ptr(du), backend.ptr(out), C.byref(total),
+                        backend.ptr(ws), need.value, backend.stream()))
+    return np.asarray(backend.download(out), dtype=np.int64), float(total.value)
+
+
+def project_outcomes(indices: np.ndarray, n: int, qubits) -> np.ndarray:
+    """Basis indices of an n-qubit register -> outcomes over ``qubits`` (``qubits[0]`` the MSB)."""
+    k = len(qubits)
+    if list(qubits) == list(range(n)):
+        return indices
+    out = np.zeros(len(indices), dtype=np.int64)
+    for j, q in enumerate(qubits):
+        out |= ((indices >> (n - 1 - q)) & 1) << (k - 1 - j)
+    return out
+
+
 def _to_device(x, backend) -> DeviceState:
     return x if isinstance(x, DeviceState) else DeviceState.from_numpy(x, backend)
 

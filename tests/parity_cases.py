@@ -301,7 +301,8 @@ def check_random_vs_oracle(backend, trials, n_range, tile_range, seed):
 
 def check_edge_cases(backend):
     """The corners: empty and diagonal-only circuits, registers of one qubit, gates on the
-    whole register, gates wider than a step (in-place dense-block kernel, k = 5 .. 8),
+    whole register, gates wider than a step (in-place dense-block kernel, k = 5 .. 10; from
+    k = 9 on its tile needs more than 48 KiB of shared memory),
     cancelling CZ pairs, reversed / scattered targets, empty and zero-length RB batches."""
     rng = np.random.default_rng(99)
 
@@ -360,7 +361,8 @@ def check_edge_cases(backend):
     # ... on registers with many tiles; targets on the lowest index bits (qubits n-1, n-2, n-3), on the
     # highest, scattered; the same plan executed twice (the device copy of the matrix is reused)
     for k, n, idx in ((5, 12, [11, 10, 9, 0, 4]), (5, 13, [0, 1, 2, 3, 4]), (6, 12, None), (7, 12, None),
-                      (8, 11, None), (5, 5, None), (6, 7, [6, 5, 4, 3, 2, 1])):
+                      (8, 11, None), (5, 5, None), (6, 7, [6, 5, 4, 3, 2, 1]), (9, 12, None),
+                      (9, 9, [8, 7, 6, 5, 4, 3, 2, 1, 0]), (10, 13, None), (10, 11, [0, 1, 2, 3, 4, 5, 6, 7, 8, 9])):
         psi = rand_state(n)
         if idx is None:
             idx = [int(q) for q in rng.permutation(n)[:k]]

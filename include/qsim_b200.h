@@ -156,6 +156,23 @@ int qsim_expect_pauli(const void* state, int n_qubits, int64_t n_terms, const ui
 int qsim_expect_pauli_dm(const void* vec_rho, int n_qubits, int64_t n_terms, const uint64_t* x_masks,
                          const uint64_t* z_masks, double* out_re_im, void* stream);
 
+/* ---- Pauli-string rotations (Trotterised evolution under a Pauli sum) ------------------
+ * state <- R_{n_rot-1} ... R_1 R_0 state, in place, with R_t = exp(-i angles[t]/2 P_t) and P_t the
+ * string (x_masks[t], z_masks[t]) in the convention of qsim_expect_pauli.  Masks and angles are
+ * HOST arrays of n_rot.  The rotations are applied in caller order (never reordered); runs of
+ * consecutive rotations whose X masks span at most 4 dimensions share one read and one write of
+ * the state (up to 32 rotations per pass).  Angle-0 rotations are skipped; x = z = 0 is the global
+ * phase exp(-i angle/2).  Null pointers, masks at or above n_qubits, n_qubits outside [1, 63] and a
+ * non-finite angle are QSIM_ERR_ARG; n_rot == 0 does nothing.  Allocates nothing and does not
+ * synchronise. */
+int qsim_apply_pauli_rotations(void* state, int n_qubits, int64_t n_rot, const uint64_t* x_masks,
+                               const uint64_t* z_masks, const double* angles, void* stream);
+/* rho <- U rho U^dagger, U = R_{n_rot-1} ... R_0, on the row-major vec of an N-qubit density matrix
+ * (N <= 31): each rotation acts on the row qubits with its angle and, conjugated, on the column
+ * qubits in the same pass. */
+int qsim_apply_pauli_rotations_dm(void* vec_rho, int n_qubits, int64_t n_rot, const uint64_t* x_masks,
+                                  const uint64_t* z_masks, const double* angles, void* stream);
+
 /* ---- measurement statistics: marginal probabilities and shot sampling -------------------
  * Qubits are the reference's (qubit q is index bit n-1-q).  A marginal over qubits[0..k) has
  * 2^k bins; bit k-1-j of the bin number is the value of qubits[j], so qubits[0] is the most

@@ -31,6 +31,8 @@ int expect_pauli(const qs_c128* state, int n, const PauliPlan& plan, int64_t n_t
 // xi, zi: index-bit masks per term; sums: 2 * n_terms doubles (re, im per term)
 int expect_pauli_dm(const qs_c128* rho, int n, int64_t n_terms, const uint64_t* xi, const uint64_t* zi,
                     double* sums, void* stream);
+// n index bits (2N for a density matrix); one launch per pass, in place, no allocation, no synchronisation
+int apply_pauli_rotations(qs_c128* state, int n, const PauliRotPlan& plan, void* stream);
 // out: 2^G.k doubles (device memory for the CUDA library)
 int marginal_probs(const QsProbSrc& src, const QsMargGeom& G, double* out, void* stream);
 // n index bits; ws: the caller's workspace laid out by qs_sample_layout(n, shots); *total gets the

@@ -144,6 +144,25 @@ int sample(const char* who, const void* state, int n, int max_n, int64_t shots, 
   return QSIM_OK;
 }
 
+int pauli_rotations(const char* who, void* state, int n, int64_t n_rot, const uint64_t* x_masks,
+                    const uint64_t* z_masks, const double* angles, bool dm, void* stream) {
+  int rc = qs::check_pauli_args(who, n, n_rot, x_masks, z_masks, angles);
+  if (rc != QSIM_OK || n_rot == 0) return rc;
+  const std::string w(who);
+  if (!state) return qs::fail(QSIM_ERR_ARG, w + ": null state");
+  if (dm && n > 31) return qs::fail(QSIM_ERR_ARG, w + ": n_qubits must be in [1, 31]");
+  for (int64_t t = 0; t < n_rot; ++t)
+    if (!std::isfinite(angles[t])) return qs::fail(QSIM_ERR_ARG, w + ": non-finite angle");
+  qs::PauliRotPlan plan;
+  try {
+    rc = qs::plan_pauli_rotations(n, n_rot, x_masks, z_masks, angles, dm, &plan);
+  } catch (const std::bad_alloc&) {
+    rc = qs::fail(QSIM_ERR_NOMEM, "out of host memory while packing the Pauli rotations");
+  }
+  if (rc != QSIM_OK || plan.passes.empty()) return rc;
+  return qs::dev::apply_pauli_rotations((qs_c128*)state, dm ? 2 * n : n, plan, stream);
+}
+
 }  // namespace
 
 extern "C" {
@@ -410,6 +429,18 @@ int qsim_expect_pauli_dm(const void* vec_rho, int n_qubits, int64_t n_terms, con
   if (rc != QSIM_OK) return rc;
   qs::pauli_finish_dm(n_terms, phase, sums.data(), out_re_im);
   return QSIM_OK;
+}
+
+int qsim_apply_pauli_rotations(void* state, int n_qubits, int64_t n_rot, const uint64_t* x_masks,
+                               const uint64_t* z_masks, const double* angles, void* stream) {
+  return pauli_rotations("qsim_apply_pauli_rotations", state, n_qubits, n_rot, x_masks, z_masks, angles, false,
+                         stream);
+}
+
+int qsim_apply_pauli_rotations_dm(void* vec_rho, int n_qubits, int64_t n_rot, const uint64_t* x_masks,
+                                  const uint64_t* z_masks, const double* angles, void* stream) {
+  return pauli_rotations("qsim_apply_pauli_rotations_dm", vec_rho, n_qubits, n_rot, x_masks, z_masks, angles, true,
+                         stream);
 }
 
 int qsim_marginal_probs(const void* state, int n_qubits, int k, const int* qubits, double* out, void* stream) {

@@ -286,6 +286,57 @@ QS_HD void qs_pauli_item(const QsPauliPass& P, const qs_c128* __restrict__ state
   }
 }
 
+// One work item (outer index o) of a rotation pass, in place: the 2^D amplitudes base ^ off[m]
+// are loaded once, every rotation of the pass updates all of them from b[m] = a[m ^ xl] (the same
+// uniform conditional swaps as qs_pauli_item), and they are stored back to the same addresses.
+//     a[m] <- c a[m] + s kappa sigma(m) b[m],   sigma(m) = (-1)^(par(base & z) + popc((m ^ xl) & spec))
+// kappa = i^cls is a swap and / or a negation of b's components, never a multiplication.
+template <int D>
+QS_HD void qs_pauli_rot_item(const QsPauliRotPass& P, qs_c128* __restrict__ state, uint64_t o) {
+  uint64_t base = o;
+#pragma unroll
+  for (int i = 0; i < D; ++i) base = qs_insert_bit(base, P.pivot[i], 0);
+  qs_c128 a[1 << D];
+#pragma unroll
+  for (int m = 0; m < (1 << D); ++m) a[m] = state[base ^ P.off[m]];
+  for (uint32_t r = 0; r < P.nrot; ++r) {
+    const uint32_t xl = P.xl[r], spec = P.spec[r], cls = P.cls[r];
+    const double c = P.c[r];
+    const double s = (qs_par64(base & P.z[r]) ^ (cls >> 1)) ? -P.s[r] : P.s[r];
+    qs_c128 b[1 << D];
+#pragma unroll
+    for (int m = 0; m < (1 << D); ++m) b[m] = a[m];
+#pragma unroll
+    for (int k = 0; k < D; ++k) {
+      if ((xl >> k) & 1) {
+#pragma unroll
+        for (int m = 0; m < (1 << D); ++m)
+          if (!((m >> k) & 1)) {
+            const qs_c128 tmp = b[m];
+            b[m] = b[m | (1 << k)];
+            b[m | (1 << k)] = tmp;
+          }
+      }
+    }
+    if (cls & 1u) {                        // times i
+#pragma unroll
+      for (int m = 0; m < (1 << D); ++m) {
+        const double t = b[m].x;
+        b[m].x = -b[m].y;
+        b[m].y = t;
+      }
+    }
+#pragma unroll
+    for (int m = 0; m < (1 << D); ++m) {
+      const double sm = qs_par64(((uint32_t)m ^ xl) & spec) ? -s : s;
+      a[m].x = c * a[m].x + sm * b[m].x;
+      a[m].y = c * a[m].y + sm * b[m].y;
+    }
+  }
+#pragma unroll
+  for (int m = 0; m < (1 << D); ++m) state[base ^ P.off[m]] = a[m];
+}
+
 // Density matrix: entry c of tr(rho X^x Z^z) = sum_c (-1)^popc(c & z) rho[c, c ^ x] (the phase
 // i^popc(x & z) is applied by the host).  rho is the row-major vec of an N-qubit matrix.
 QS_HD qs_c128 qs_pauli_dm_elem(const qs_c128* __restrict__ rho, int N, uint64_t x, uint64_t z, uint64_t c) {

@@ -257,6 +257,23 @@ int expect_pauli(const qs_c128* s, int n, const PauliPlan& plan, int64_t, double
   return QSIM_OK;
 }
 
+// one launch per pass, as in the CUDA library
+int apply_pauli_rotations(qs_c128* s, int n, const PauliRotPlan& plan, void*) {
+  const uint64_t count = 1ull << (n - plan.d);
+  for (const QsPauliRotPass& P : plan.passes) {
+    for (uint64_t o = 0; o < count; ++o) {
+      switch (plan.d) {
+        case 1: qs_pauli_rot_item<1>(P, s, o); break;
+        case 2: qs_pauli_rot_item<2>(P, s, o); break;
+        case 3: qs_pauli_rot_item<3>(P, s, o); break;
+        default: qs_pauli_rot_item<4>(P, s, o); break;
+      }
+    }
+    ++g_launches;
+  }
+  return QSIM_OK;
+}
+
 int expect_pauli_dm(const qs_c128* rho, int n, int64_t n_terms, const uint64_t* xi, const uint64_t* zi,
                     double* sums, void*) {
   for (int64_t t = 0; t < n_terms; ++t)

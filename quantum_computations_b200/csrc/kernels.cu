@@ -773,6 +773,21 @@ void launch_pauli_pass(const QsPauliPass& P, const qs_c128* state, uint64_t coun
 }
 
 // =====================================================================================
+// Pauli-string rotations (plan.h, elem_ops.h, pauli.cpp): one in-place pass per run of rotations
+// =====================================================================================
+// D = 4 takes 222 registers, so two 128-thread CTAs are resident per SM; measured (DESIGN.md section 5),
+// one CTA per SM is 1.3x slower and 2, 4 or 8 are equal
+constexpr int kRotThreads = 128;
+constexpr int kRotBlocksPerSM = 4;
+
+template <int D>
+__global__ void __launch_bounds__(kRotThreads)
+k_pauli_rotate(qs_c128* __restrict__ state, const __grid_constant__ QsPauliRotPass P, uint64_t count) {
+  for (uint64_t o = blockIdx.x * (uint64_t)kRotThreads + threadIdx.x; o < count; o += (uint64_t)gridDim.x * kRotThreads)
+    qs_pauli_rot_item<D>(P, state, o);
+}
+
+// =====================================================================================
 // Marginal probabilities (elem_ops.h, QsMargGeom): one read-only pass, then a fixed-tree final sum
 // =====================================================================================
 constexpr int kMargThreads = 256;
@@ -1602,6 +1617,29 @@ int expect_pauli_dm(const qs_c128* rho, int n, int64_t n_terms, const uint64_t* 
   rc = launched();
   if (rc != QSIM_OK) return rc;
   return pauli_sums_to_host(ctx, n_terms, (int)bx, sums, st);
+}
+
+int apply_pauli_rotations(qs_c128* state, int n, const PauliRotPlan& plan, void* stream) {
+  Bound bound;
+  int rc = bind_device(state, &bound);
+  DevCtx* ctx = bound.ctx;
+  if (rc != QSIM_OK) return rc;
+  const uint64_t count = 1ull << (n - plan.d);
+  const int per_sm = qs::dev_knob("QSIM_ROT_BLOCKS_PER_SM", kRotBlocksPerSM);
+  const unsigned blocks = (unsigned)std::min<uint64_t>((count + kRotThreads - 1) / kRotThreads,
+                                                       (uint64_t)ctx->sms * per_sm);
+  const cudaStream_t st = (cudaStream_t)stream;
+  for (const QsPauliRotPass& P : plan.passes) {
+    switch (plan.d) {
+      case 1: k_pauli_rotate<1><<<blocks, kRotThreads, 0, st>>>(state, P, count); break;
+      case 2: k_pauli_rotate<2><<<blocks, kRotThreads, 0, st>>>(state, P, count); break;
+      case 3: k_pauli_rotate<3><<<blocks, kRotThreads, 0, st>>>(state, P, count); break;
+      default: k_pauli_rotate<4><<<blocks, kRotThreads, 0, st>>>(state, P, count); break;
+    }
+    rc = launched();
+    if (rc != QSIM_OK) return rc;
+  }
+  return QSIM_OK;
 }
 
 int marginal_probs(const QsProbSrc& src, const QsMargGeom& G, double* out, void* stream) {

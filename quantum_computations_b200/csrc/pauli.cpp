@@ -1,8 +1,9 @@
-// Host half of the Pauli-sum expectation values (qsim_expect_pauli / _dm): argument checks,
-// the reference-qubit -> index-bit conversion and the packing of the terms into Pauli passes.
-// Shared verbatim by libqsim_b200.so and the host emulator, so the CPU tests check the very
-// grouping the GPU runs.
+// Host half of the Pauli-sum expectation values (qsim_expect_pauli / _dm) and of the Pauli-string
+// rotations (qsim_apply_pauli_rotations / _dm): argument checks, the reference-qubit -> index-bit
+// conversion and the packing of the terms into Pauli passes.  Shared verbatim by libqsim_b200.so
+// and the host emulator, so the CPU tests check the very grouping the GPU runs.
 #include <algorithm>
+#include <cmath>
 #include <cstring>
 #include <map>
 
@@ -205,6 +206,88 @@ int plan_pauli(int n, int64_t n_terms, const uint64_t* x_masks, const uint64_t* 
     }
     P.nterms = t;
     term0 += t;
+    out->passes.push_back(P);
+  }
+  return QSIM_OK;
+}
+
+int plan_pauli_rotations(int n, int64_t n_rot, const uint64_t* x_masks, const uint64_t* z_masks, const double* angles,
+                         bool dm, PauliRotPlan* out) {
+  // the rotations on the register, in caller order; a unit is what must share a pass (for a density
+  // matrix the row and the column half of one caller rotation: they commute, and one pass holds both)
+  struct Rot { uint64_t x, z; double theta; int cls; };
+  const int nreg = dm ? 2 * n : n;
+  std::vector<Rot> rots;
+  std::vector<size_t> unit_end;
+  for (int64_t t = 0; t < n_rot; ++t) {
+    if (angles[t] == 0.0) continue;                    // the identity
+    const int c = popc64(x_masks[t] & z_masks[t]) & 3;
+    const int cls = (c + 3) & 3;                       // -i i^c
+    rots.push_back({to_index_bits(x_masks[t], nreg), to_index_bits(z_masks[t], nreg), angles[t], cls});
+    // column half: conj(exp(-i theta/2 P)) = exp(+i theta/2 conj(P)) and conj(P) = (-1)^c P
+    if (dm)
+      rots.push_back({to_index_bits(x_masks[t] << n, nreg), to_index_bits(z_masks[t] << n, nreg),
+                      (c & 1) ? angles[t] : -angles[t], cls});
+    unit_end.push_back(rots.size());
+  }
+  const int d = std::min(nreg, QS_PAULI_MAX_D);
+  out->d = d;
+  out->passes.clear();
+
+  // Greedy in caller order: a unit joins the open pass if the cap allows and its X masks lie in the
+  // span or fit as further generators; otherwise it opens the next pass.
+  struct Draft { Span span; size_t first, last; };
+  std::vector<Draft> drafts;
+  size_t begin = 0;
+  for (size_t end : unit_end) {
+    bool fits = !drafts.empty() && end - drafts.back().first <= QS_PAULI_ROT_MAX;
+    Span grown;
+    if (fits) {
+      grown = drafts.back().span;
+      for (size_t r = begin; r < end && fits; ++r)
+        if (!grown.contains(rots[r].x)) {
+          if (grown.d < d) grown.add(rots[r].x);
+          else fits = false;
+        }
+    }
+    if (fits) {
+      drafts.back().span = grown;
+      drafts.back().last = end;
+    } else {
+      Draft dr;
+      for (size_t r = begin; r < end; ++r)
+        if (!dr.span.contains(rots[r].x)) dr.span.add(rots[r].x);
+      dr.first = begin;
+      dr.last = end;
+      drafts.push_back(dr);
+    }
+    begin = end;
+  }
+
+  // descriptors: spans padded and pivots chosen as in plan_pauli
+  for (Draft& p : drafts) {
+    for (int b = nreg - 1; p.span.d < d && b >= 0; --b)
+      if (!p.span.contains(1ull << b)) p.span.add(1ull << b);
+    QsPauliRotPass P;
+    memset(&P, 0, sizeof(P));
+    P.d = (uint32_t)d;
+    int piv[QS_PAULI_MAX_D];
+    for (int i = 0; i < d; ++i) piv[i] = p.span.piv[i];
+    std::sort(piv, piv + d);
+    for (int i = 0; i < d; ++i) P.pivot[i] = (uint8_t)piv[i];
+    for (int m = 0; m < (1 << d); ++m) P.off[m] = p.span.off(m);
+    for (size_t r = p.first; r < p.last; ++r) {
+      const Rot& R = rots[r];
+      const uint32_t k = P.nrot++;
+      P.xl[k] = (uint8_t)p.span.coords(R.x);
+      P.z[k] = R.z;
+      uint32_t spec = 0;
+      for (int i = 0; i < d; ++i) spec |= (uint32_t)(popc64(P.off[1 << i] & R.z) & 1) << i;
+      P.spec[k] = (uint8_t)spec;
+      P.cls[k] = (uint8_t)R.cls;
+      P.c[k] = std::cos(0.5 * R.theta);
+      P.s[k] = std::sin(0.5 * R.theta);
+    }
     out->passes.push_back(P);
   }
   return QSIM_OK;

@@ -218,3 +218,27 @@ struct QsPauliPass {
   uint8_t  spec[QS_PAULI_MAX_TERMS];         // s: bit i = parity(generator_i & z)
   uint8_t  cls[QS_PAULI_MAX_TERMS];          // bit 0: imaginary part of w; bit 1: negated
 };
+
+// ---- Pauli-string rotations (qsim_apply_pauli_rotations / _dm) ------------------------------
+// One *rotation pass* applies R_r = exp(-i theta_r / 2 P_r) = c_r - i s_r P_r for a contiguous run
+// of rotations, in caller order, with one read and one write of the state.  The thread layout is
+// the Pauli pass's (d, pivot, off as in QsPauliPass): every X mask of the run is off[xl] for some
+// xl, so P pairs amplitude m with m ^ xl inside the thread's registers, and
+//     (P a)[m] = i^popc(x & z) (-1)^(par(base & z) + popc((m ^ xl) & spec)) a[m ^ xl].
+// The caller's factor -i i^popc(x & z) is kappa = i^cls.  Rotations of one pass run in a loop, so
+// the cap only bounds the descriptor; DESIGN.md section 3.2.3 gives the measurement behind it.
+#define QS_PAULI_ROT_MAX 32
+
+struct QsPauliRotPass {
+  uint32_t d;                                // generators = log2 amplitudes per thread
+  uint32_t nrot;
+  uint8_t  pivot[QS_PAULI_MAX_D];            // ascending index bits that are zero in every base
+  uint64_t off[1 << QS_PAULI_MAX_D];         // XOR of the generators selected by m
+  uint64_t z[QS_PAULI_ROT_MAX];              // index-bit Z mask of each rotation
+  double   c[QS_PAULI_ROT_MAX];              // cos(theta / 2)
+  double   s[QS_PAULI_ROT_MAX];              // sin(theta / 2)
+  uint8_t  xl[QS_PAULI_ROT_MAX];             // X mask in generator coordinates
+  uint8_t  spec[QS_PAULI_ROT_MAX];           // bit i = parity(generator_i & z)
+  uint8_t  cls[QS_PAULI_ROT_MAX];            // kappa = -i i^popc(x & z) = i^cls
+};
+static_assert(sizeof(QsPauliRotPass) <= 4096, "QsPauliRotPass is a kernel parameter");

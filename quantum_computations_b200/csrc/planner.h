@@ -107,6 +107,17 @@ struct PauliPlan {
 // Greedy grouping by X mask: at most one pass per chunk of <= QS_PAULI_MAX_TERMS terms of one
 // non-zero X mask, the Z strings in passes with room (a pass of their own only if none has).
 int plan_pauli(int n, int64_t n_terms, const uint64_t* x_masks, const uint64_t* z_masks, PauliPlan* out);
+// The rotation passes of one qsim_apply_pauli_rotations(_dm) call, in caller order.
+struct PauliRotPlan {
+  int d = 0;                                 // generators per pass: min(register bits, QS_PAULI_MAX_D)
+  std::vector<QsPauliRotPass> passes;
+};
+// Greedy in caller order, never reordered: a rotation joins the open pass while the cap allows and
+// its X mask is in the span or the span has room; angle-0 rotations are skipped.  dm: n is N and
+// every rotation becomes its row half and its conjugated column half on the 2N-bit vec of rho,
+// always in one pass.
+int plan_pauli_rotations(int n, int64_t n_rot, const uint64_t* x_masks, const uint64_t* z_masks, const double* angles,
+                         bool dm, PauliRotPlan* out);
 // sums: 2 doubles per slot (re, im) -> out[caller term] (real).
 void pauli_finish(const PauliPlan& plan, const double* sums, double* out);
 // sums: 2 doubles per term, times i^phase -> out_re_im.

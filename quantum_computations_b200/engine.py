@@ -434,6 +434,22 @@ class DeviceState:
                                                   z.ctypes.data, _dptr(out.view(np.float64)), be.stream()))
         return out
 
+    def apply_pauli_rotations(self, x_masks, z_masks, angles) -> "DeviceState":
+        """In place: state <- R_{k-1} ... R_0 state with R_t = exp(-i angles[t]/2 P_t) and P_t the
+        string ``(x_masks[t], z_masks[t])`` (convention of ``expect_pauli``), in that order; a
+        density matrix becomes U rho U^dagger.  Returns ``self``."""
+        x = np.ascontiguousarray(x_masks, dtype=np.uint64).reshape(-1)
+        z = np.ascontiguousarray(z_masks, dtype=np.uint64).reshape(-1)
+        a = np.ascontiguousarray(angles, dtype=np.float64).reshape(-1)
+        if x.shape != z.shape or x.shape != a.shape:
+            raise ValueError("x_masks, z_masks and angles must have the same length")
+        lib, be = self.backend.lib, self.backend
+        fn, n = (lib.qsim_apply_pauli_rotations, self.n_bits) if self.ndim == 1 else \
+            (lib.qsim_apply_pauli_rotations_dm, self.n_bits // 2)
+        _capi.check(lib, fn(be.ptr(self.buf), n, len(x), x.ctypes.data, z.ctypes.data, a.ctypes.data, be.stream()))
+        self.host_dtype = np.dtype(np.complex128)
+        return self
+
 
     # -- measurement statistics ------------------------------------------------------------------
     def probabilities(self, qubits=None, *, device: bool = False):

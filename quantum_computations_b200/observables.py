@@ -9,6 +9,11 @@ strings are grouped by their X/Y support, so one read of the state serves up to
 costs a single read.  Density matrices (``qsim_expect_pauli_dm``) and sharded
 kets (``sharded.ShardedState.expect_pauli``) take the same masks.
 
+The same masks drive evolution: ``evolve`` applies a Trotterised exp(-i H t) for a
+``PauliSum`` H as a list of rotations exp(-i theta/2 P) (``apply_pauli_rotations`` of a
+device or sharded state, ``qsim_apply_pauli_rotations``), up to 32 rotations per read
+and write of the state.
+
 Convention: a string is a pair of masks ``(x, z)`` with bit q for reference
 qubit q; I = (0, 0), X = (1, 0), Z = (0, 1), Y = (1, 1), and the operator is
 ``i^popc(x & z) X^x Z^z`` (Z first), so every string is Hermitian.
@@ -139,3 +144,48 @@ def expect(observable: PauliSum, state, *, per_term: bool = False):
     if per_term:
         return values
     return complex(np.dot(observable.coeffs, values))
+
+
+def trotter_rotations(hamiltonian: PauliSum, time: float, steps: int = 1, order: int = 1):
+    """The rotation list ``(x_masks, z_masks, angles)`` of a Trotterised exp(-i H time): ``steps``
+    first-order steps (terms in the sum's order, angle 2 c_t time / steps) or symmetric second-order
+    (Strang) steps (every term but the last at half the angle, forward then backward).  Adjacent
+    rotations about the same string are merged, which is exact."""
+    if not isinstance(hamiltonian, PauliSum):
+        raise TypeError("evolve needs a PauliSum Hamiltonian")
+    if order not in (1, 2):
+        raise ValueError("order must be 1 or 2")
+    steps = int(steps)
+    if steps < 1:
+        raise ValueError("steps must be at least 1")
+    if np.any(hamiltonian.coeffs.imag != 0):
+        raise ValueError("the Hamiltonian has a coefficient with a nonzero imaginary part (not Hermitian)")
+    full = 2.0 * hamiltonian.coeffs.real * (float(time) / steps)
+    terms = list(range(len(hamiltonian)))
+    if order == 1:
+        one = [(t, full[t]) for t in terms]
+    else:
+        one = [(t, 0.5 * full[t]) for t in terms[:-1]] + [(t, full[t]) for t in terms[-1:]] + \
+              [(t, 0.5 * full[t]) for t in reversed(terms[:-1])]
+    merged = []
+    for t, angle in one * steps:
+        if merged and merged[-1][0] == t:
+            merged[-1][1] += angle
+        else:
+            merged.append([t, angle])
+    index = np.array([t for t, _ in merged], dtype=np.int64)
+    return (hamiltonian.x_masks[index], hamiltonian.z_masks[index],
+            np.array([a for _, a in merged], dtype=np.float64))
+
+
+def evolve(hamiltonian: PauliSum, state, time: float, *, steps: int = 1, order: int = 1):
+    """Trotterised exp(-i H time) applied in place to ``state`` (an ``engine.DeviceState`` ket or
+    density matrix, or a ``sharded.ShardedState``, collectively); returns the state.  H must have
+    real coefficients.  The identity term is kept as a global phase, so a ket matches
+    ``expm(-1j * H * time)`` including its phase when the terms commute.  All rotations go to
+    ``apply_pauli_rotations`` in one call (see ``trotter_rotations``)."""
+    x, z, angles = trotter_rotations(hamiltonian, time, steps, order)
+    if not isinstance(state, _sharded_type()) and hamiltonian.num_qubits > state.num_qubits:
+        raise ValueError(f"the Hamiltonian acts on {hamiltonian.num_qubits} qubits, "
+                         f"the state has {state.num_qubits}")
+    return state.apply_pauli_rotations(x, z, angles)

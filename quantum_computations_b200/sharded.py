@@ -213,6 +213,67 @@ class ShardedState:
         from .observables import expect
         return expect(observable, self, per_term=per_term)
 
+    def apply_pauli_rotations(self, x_masks, z_masks, angles) -> "ShardedState":
+        """In place, collective: the ket becomes R_{k-1} ... R_0 |psi> with R_t = exp(-i angles[t]/2 P_t)
+        (``engine.DeviceState.apply_pauli_rotations``).  Returns ``self``.
+
+        The rotations are cut, in order, into runs whose joint X/Y support fits in a shard; each run
+        is made local with one exchange (``_localise``) and applied with one
+        ``qsim_apply_pauli_rotations`` call.  A Z factor on a rank qubit acts as the scalar (-1)^v on
+        this shard, v its logical value (flip flags included), so it leaves the shard's mask and
+        negates the angle where v = 1.  A string whose X/Y support does not fit in a shard is refused.
+        The layout may differ afterwards (``phys`` / ``flip`` record it)."""
+        if self.is_density:
+            raise NotImplementedError("Pauli rotations of a sharded density matrix are not implemented")
+        x = np.ascontiguousarray(x_masks, dtype=np.uint64).reshape(-1)
+        z = np.ascontiguousarray(z_masks, dtype=np.uint64).reshape(-1)
+        a = np.ascontiguousarray(angles, dtype=np.float64).reshape(-1)
+        if x.shape != z.shape or x.shape != a.shape:
+            raise ValueError("x_masks, z_masks and angles must have the same length")
+        n = self.n
+        if len(x) and (int(x.max()) >> n or int(z.max()) >> n):
+            raise ValueError("a Pauli mask has a bit at or above the number of qubits")
+        if not np.all(np.isfinite(a)):
+            raise ValueError("non-finite angle")
+        xs = [{n - 1 - q for q in range(n) if int(v) >> q & 1} for v in x]
+        zs = [{n - 1 - q for q in range(n) if int(v) >> q & 1} for v in z]
+        if any(len(s) > self.n_local for s in xs):
+            raise NotImplementedError("a Pauli string's X/Y support is wider than a shard; use fewer ranks")
+        start = 0
+        while start < len(x):
+            support, end = set(xs[start]), start + 1
+            while end < len(x):
+                wider = support | xs[end]
+                need = [l for l in wider if self.phys[l] >= self.n_local]
+                free = [l for l in range(n) if self.phys[l] < self.n_local and l not in wider]
+                if len(need) > len(free):
+                    break
+                support, end = wider, end + 1
+            self._localise(support)
+            self._rotate_local(range(start, end), xs, zs, a)
+            start = end
+        return self
+
+    def _rotate_local(self, run, xs, zs, angles) -> None:
+        """The rotations ``run`` (X supports local) on this shard, Z factors on rank qubits as signs."""
+        nl = self.n_local
+        run = list(run)
+        lx = np.zeros(len(run), dtype=np.uint64)
+        lz = np.zeros(len(run), dtype=np.uint64)
+        la = np.array(angles[run], dtype=np.float64)
+        for k, t in enumerate(run):
+            for l in xs[t]:
+                lx[k] |= np.uint64(1 << (nl - 1 - self.phys[l]))         # shard reference qubit
+            for l in zs[t]:
+                p = self.phys[l]
+                if p < nl:
+                    lz[k] |= np.uint64(1 << (nl - 1 - p))
+                elif self.rank_value(p):
+                    la[k] = -la[k]
+        be = self.backend
+        _capi.check(be.lib, be.lib.qsim_apply_pauli_rotations(be.ptr(self.buf), nl, len(run), lx.ctypes.data,
+                                                              lz.ctypes.data, la.ctypes.data, be.stream()))
+
     def _localise(self, support) -> None:
         """Make the logical bits in ``support`` local with one exchange against the highest
         local bits outside it.  A bit that arrives complemented (its rank bit carried the flip

@@ -173,6 +173,35 @@ int qsim_apply_pauli_rotations(void* state, int n_qubits, int64_t n_rot, const u
 int qsim_apply_pauli_rotations_dm(void* vec_rho, int n_qubits, int64_t n_rot, const uint64_t* x_masks,
                                   const uint64_t* z_masks, const double* angles, void* stream);
 
+/* ---- H|psi> for a Pauli sum, and adjoint gradients over Pauli rotations -----------------
+ * out <- sum_t c_t P_t in, out of place, with c_t = (coeffs_re_im[2t], coeffs_re_im[2t+1]) and P_t
+ * the string (x_masks[t], z_masks[t]) in the convention of qsim_expect_pauli; masks and coefficients
+ * are HOST arrays.  Terms are grouped by X mask as for qsim_expect_pauli: one read of `in` and one
+ * read-modify-write of `out` per pass of up to 32 terms.  n_terms == 0 writes zeros.  in == out,
+ * null pointers, masks at or above n_qubits, n_qubits outside [1, 63] and a non-finite coefficient
+ * are QSIM_ERR_ARG.  The vec of an N-qubit density matrix with 2N qubits and masks on qubits
+ * 0..N-1 (the row qubits) gives vec(H rho).  Allocates nothing and does not synchronise. */
+int qsim_apply_pauli_sum(const void* in, void* out, int n_qubits, int64_t n_terms, const uint64_t* x_masks,
+                         const uint64_t* z_masks, const double* coeffs_re_im, void* stream);
+/* out <- out + sum_t c_t P_t in: the same passes, every one adding to out (no extra buffer and no
+ * extra pass for a sum taken in parts); n_terms == 0 leaves out unchanged.  Same checks. */
+int qsim_accumulate_pauli_sum(const void* in, void* out, int n_qubits, int64_t n_terms, const uint64_t* x_masks,
+                              const uint64_t* z_masks, const double* coeffs_re_im, void* stream);
+/* The backward sweep of the adjoint method over U = R_{n_rot-1} ... R_0, the rotation list of
+ * qsim_apply_pauli_rotations.  On entry psi = U psi0 and lam is any state; on return psi holds psi0
+ * (within rounding), lam holds U^dagger lam and out[t] = Im<lam_t|P_t|psi_t>, both states taken just
+ * after R_t.  With lam = H psi, out[t] = d<H>/d theta_t.  The sweep runs the rotations in reverse
+ * order with up to 32 per read and write of both states (X masks spanning at most 3 dimensions);
+ * angle-0 rotations are kept.  out: HOST array of n_rot doubles; fixed summation trees, so two calls
+ * on the same inputs give bit-identical results.  psi == lam is QSIM_ERR_ARG, the other checks are
+ * those of qsim_apply_pauli_rotations; n_rot == 0 does nothing.  Synchronises the stream. */
+int qsim_pauli_rotations_adjoint(void* psi, void* lam, int n_qubits, int64_t n_rot, const uint64_t* x_masks,
+                                 const uint64_t* z_masks, const double* angles, double* out, void* stream);
+/* The same on the row-major vecs of N-qubit density matrices (N <= 31): psi = U rho0 U^dagger,
+ * out[t] = d Re<<lam|rho>>/d theta_t with <<A|B>> = tr(A^dagger B). */
+int qsim_pauli_rotations_adjoint_dm(void* psi, void* lam, int n_qubits, int64_t n_rot, const uint64_t* x_masks,
+                                    const uint64_t* z_masks, const double* angles, double* out, void* stream);
+
 /* ---- measurement statistics: marginal probabilities and shot sampling -------------------
  * Qubits are the reference's (qubit q is index bit n-1-q).  A marginal over qubits[0..k) has
  * 2^k bins; bit k-1-j of the bin number is the value of qubits[j], so qubits[0] is the most

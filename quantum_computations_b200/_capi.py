@@ -82,6 +82,14 @@ SIGNATURES = {
                                              C.c_void_p]),
     "qsim_apply_pauli_rotations_dm": (C.c_int, [C.c_void_p, C.c_int, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p,
                                                 C.c_void_p]),
+    "qsim_apply_pauli_sum": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int64, C.c_void_p, C.c_void_p,
+                                       C.c_void_p, C.c_void_p]),
+    "qsim_accumulate_pauli_sum": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int64, C.c_void_p, C.c_void_p,
+                                            C.c_void_p, C.c_void_p]),
+    "qsim_pauli_rotations_adjoint": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int64, C.c_void_p, C.c_void_p,
+                                               C.c_void_p, C.c_void_p, C.c_void_p]),
+    "qsim_pauli_rotations_adjoint_dm": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int64, C.c_void_p,
+                                                  C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "qsim_marginal_probs": (C.c_int, [C.c_void_p, C.c_int, C.c_int, c_int_p, C.c_void_p, C.c_void_p]),
     "qsim_marginal_probs_dm": (C.c_int, [C.c_void_p, C.c_int, C.c_int, c_int_p, C.c_void_p, C.c_void_p]),
     "qsim_sample_workspace_bytes": (C.c_int, [C.c_int, C.c_int64, C.POINTER(C.c_uint64)]),

@@ -33,6 +33,12 @@ int expect_pauli_dm(const qs_c128* rho, int n, int64_t n_terms, const uint64_t* 
                     double* sums, void* stream);
 // n index bits (2N for a density matrix); one launch per pass, in place, no allocation, no synchronisation
 int apply_pauli_rotations(qs_c128* state, int n, const PauliRotPlan& plan, void* stream);
+// out <- sum_t c_t P_t in (or out + ..., as the plan's passes say), n index bits, one launch per pass;
+// no allocation, no synchronisation
+int apply_pauli_sum(const qs_c128* in, qs_c128* out, int n, const PauliApplyPlan& plan, void* stream);
+// the sweep of an adjoint plan on psi and lam (n index bits), one launch per pass plus the final sum;
+// sums: 2 doubles per rotation slot of `plan`; synchronises the stream
+int pauli_rotations_adjoint(qs_c128* psi, qs_c128* lam, int n, const PauliRotPlan& plan, double* sums, void* stream);
 // out: 2^G.k doubles (device memory for the CUDA library)
 int marginal_probs(const QsProbSrc& src, const QsMargGeom& G, double* out, void* stream);
 // n index bits; ws: the caller's workspace laid out by qs_sample_layout(n, shots); *total gets the

@@ -144,15 +144,22 @@ int sample(const char* who, const void* state, int n, int max_n, int64_t shots, 
   return QSIM_OK;
 }
 
+// The checks of the rotation entry points after the masks and the states: density-matrix size, angles.
+int rotation_args(const std::string& w, int n, int64_t n_rot, const double* angles, bool dm) {
+  if (dm && n > 31) return qs::fail(QSIM_ERR_ARG, w + ": n_qubits must be in [1, 31]");
+  for (int64_t t = 0; t < n_rot; ++t)
+    if (!std::isfinite(angles[t])) return qs::fail(QSIM_ERR_ARG, w + ": non-finite angle");
+  return QSIM_OK;
+}
+
 int pauli_rotations(const char* who, void* state, int n, int64_t n_rot, const uint64_t* x_masks,
                     const uint64_t* z_masks, const double* angles, bool dm, void* stream) {
   int rc = qs::check_pauli_args(who, n, n_rot, x_masks, z_masks, angles);
   if (rc != QSIM_OK || n_rot == 0) return rc;
   const std::string w(who);
   if (!state) return qs::fail(QSIM_ERR_ARG, w + ": null state");
-  if (dm && n > 31) return qs::fail(QSIM_ERR_ARG, w + ": n_qubits must be in [1, 31]");
-  for (int64_t t = 0; t < n_rot; ++t)
-    if (!std::isfinite(angles[t])) return qs::fail(QSIM_ERR_ARG, w + ": non-finite angle");
+  rc = rotation_args(w, n, n_rot, angles, dm);
+  if (rc != QSIM_OK) return rc;
   qs::PauliRotPlan plan;
   try {
     rc = qs::plan_pauli_rotations(n, n_rot, x_masks, z_masks, angles, dm, &plan);
@@ -161,6 +168,52 @@ int pauli_rotations(const char* who, void* state, int n, int64_t n_rot, const ui
   }
   if (rc != QSIM_OK || plan.passes.empty()) return rc;
   return qs::dev::apply_pauli_rotations((qs_c128*)state, dm ? 2 * n : n, plan, stream);
+}
+
+int pauli_sum(const char* who, const void* in, void* out, int n, int64_t n_terms, const uint64_t* x_masks,
+              const uint64_t* z_masks, const double* coeffs_re_im, bool accumulate, void* stream) {
+  const std::string w(who);
+  int rc = qs::check_pauli_args(who, n, n_terms, x_masks, z_masks, coeffs_re_im);
+  if (rc != QSIM_OK) return rc;
+  if (!in || !out) return qs::fail(QSIM_ERR_ARG, w + ": null state");
+  if (in == out) return qs::fail(QSIM_ERR_ARG, w + ": in and out must be different buffers");
+  if (n < 1 || n > 63) return qs::fail(QSIM_ERR_ARG, w + ": n_qubits must be in [1, 63]");
+  for (int64_t t = 0; t < 2 * n_terms; ++t)
+    if (!std::isfinite(coeffs_re_im[t])) return qs::fail(QSIM_ERR_ARG, w + ": non-finite coefficient");
+  if (accumulate && n_terms == 0) return QSIM_OK;
+  qs::PauliApplyPlan plan;
+  try {
+    rc = qs::plan_pauli_apply(n, n_terms, x_masks, z_masks, coeffs_re_im, accumulate, &plan);
+  } catch (const std::bad_alloc&) {
+    rc = qs::fail(QSIM_ERR_NOMEM, "out of host memory while grouping the Pauli terms");
+  }
+  if (rc != QSIM_OK) return rc;
+  return qs::dev::apply_pauli_sum((const qs_c128*)in, (qs_c128*)out, n, plan, stream);
+}
+
+int pauli_adjoint(const char* who, void* psi, void* lam, int n, int64_t n_rot, const uint64_t* x_masks,
+                  const uint64_t* z_masks, const double* angles, double* out, bool dm, void* stream) {
+  int rc = qs::check_pauli_args(who, n, n_rot, x_masks, z_masks, angles);
+  if (rc != QSIM_OK || n_rot == 0) return rc;
+  const std::string w(who);
+  if (!psi || !lam) return qs::fail(QSIM_ERR_ARG, w + ": null state");
+  if (!out) return qs::fail(QSIM_ERR_ARG, w + ": null argument");
+  if (psi == lam) return qs::fail(QSIM_ERR_ARG, w + ": psi and lam must be different buffers");
+  rc = rotation_args(w, n, n_rot, angles, dm);
+  if (rc != QSIM_OK) return rc;
+  qs::PauliRotPlan plan;
+  std::vector<double> sums;
+  try {
+    rc = qs::plan_pauli_rotations(n, n_rot, x_masks, z_masks, angles, dm, &plan, true);
+    sums.assign(2 * plan.caller.size(), 0.0);
+  } catch (const std::bad_alloc&) {
+    rc = qs::fail(QSIM_ERR_NOMEM, "out of host memory while packing the Pauli rotations");
+  }
+  if (rc != QSIM_OK) return rc;
+  rc = qs::dev::pauli_rotations_adjoint((qs_c128*)psi, (qs_c128*)lam, dm ? 2 * n : n, plan, sums.data(), stream);
+  if (rc != QSIM_OK) return rc;
+  qs::pauli_adjoint_finish(plan, n_rot, sums.data(), out);
+  return QSIM_OK;
 }
 
 }  // namespace
@@ -441,6 +494,29 @@ int qsim_apply_pauli_rotations_dm(void* vec_rho, int n_qubits, int64_t n_rot, co
                                   const uint64_t* z_masks, const double* angles, void* stream) {
   return pauli_rotations("qsim_apply_pauli_rotations_dm", vec_rho, n_qubits, n_rot, x_masks, z_masks, angles, true,
                          stream);
+}
+
+int qsim_apply_pauli_sum(const void* in, void* out, int n_qubits, int64_t n_terms, const uint64_t* x_masks,
+                         const uint64_t* z_masks, const double* coeffs_re_im, void* stream) {
+  return pauli_sum("qsim_apply_pauli_sum", in, out, n_qubits, n_terms, x_masks, z_masks, coeffs_re_im, false, stream);
+}
+
+int qsim_accumulate_pauli_sum(const void* in, void* out, int n_qubits, int64_t n_terms, const uint64_t* x_masks,
+                              const uint64_t* z_masks, const double* coeffs_re_im, void* stream) {
+  return pauli_sum("qsim_accumulate_pauli_sum", in, out, n_qubits, n_terms, x_masks, z_masks, coeffs_re_im, true,
+                   stream);
+}
+
+int qsim_pauli_rotations_adjoint(void* psi, void* lam, int n_qubits, int64_t n_rot, const uint64_t* x_masks,
+                                 const uint64_t* z_masks, const double* angles, double* out, void* stream) {
+  return pauli_adjoint("qsim_pauli_rotations_adjoint", psi, lam, n_qubits, n_rot, x_masks, z_masks, angles, out,
+                       false, stream);
+}
+
+int qsim_pauli_rotations_adjoint_dm(void* psi, void* lam, int n_qubits, int64_t n_rot, const uint64_t* x_masks,
+                                    const uint64_t* z_masks, const double* angles, double* out, void* stream) {
+  return pauli_adjoint("qsim_pauli_rotations_adjoint_dm", psi, lam, n_qubits, n_rot, x_masks, z_masks, angles, out,
+                       true, stream);
 }
 
 int qsim_marginal_probs(const void* state, int n_qubits, int k, const int* qubits, double* out, void* stream) {

@@ -337,6 +337,145 @@ QS_HD void qs_pauli_rot_item(const QsPauliRotPass& P, qs_c128* __restrict__ stat
   for (int m = 0; m < (1 << D); ++m) state[base ^ P.off[m]] = a[m];
 }
 
+// v[m] <-> v[m ^ x] for the bits of x: one uniform conditional swap per generator bit, so v stays
+// in registers for any x.
+template <int D>
+QS_HD void qs_xor_swap(qs_c128* v, uint32_t x) {
+#pragma unroll
+  for (int k = 0; k < D; ++k) {
+    if ((x >> k) & 1) {
+#pragma unroll
+      for (int m = 0; m < (1 << D); ++m)
+        if (!((m >> k) & 1)) {
+          const qs_c128 tmp = v[m];
+          v[m] = v[m | (1 << k)];
+          v[m | (1 << k)] = tmp;
+        }
+    }
+  }
+}
+
+// One work item (outer index o) of an apply pass (plan.h, QsPauliApplyPass): out[m] += F[m ^ xl]
+// in[m ^ xl] for every group, written as out[u ^ xl] += F[u] a[u].  The accumulators are kept
+// permuted instead of the products: position u of acc holds output entry u ^ cur, and moving from
+// one group's xl to the next is one set of conditional swaps.  spec[k * stride], k < 2^(D+1), is the
+// thread's spectrum scratch (Re, then Im), where the terms scatter by their runtime index spec_t.
+template <int D>
+QS_HD void qs_pauli_apply_item(const QsPauliApplyPass& A, const qs_c128* __restrict__ in, qs_c128* __restrict__ out,
+                               uint64_t o, double* spec, uint32_t stride) {
+  const QsPauliPass& P = A.p;
+  uint64_t base = o;
+#pragma unroll
+  for (int i = 0; i < D; ++i) base = qs_insert_bit(base, P.pivot[i], 0);
+  qs_c128 a[1 << D], acc[1 << D];
+#pragma unroll
+  for (int m = 0; m < (1 << D); ++m) {
+    a[m] = in[base ^ P.off[m]];
+    if (A.accumulate) {
+      acc[m] = out[base ^ P.off[m]];
+    } else {
+      acc[m].x = 0.0;
+      acc[m].y = 0.0;
+    }
+  }
+  uint32_t cur = 0;
+  for (uint32_t g = 0; g < P.ngroups; ++g) {
+    const QsPauliGroup G = P.groups[g];
+    const uint32_t t1 = (uint32_t)G.first + G.count;
+#pragma unroll
+    for (int k = 0; k < (2 << D); ++k) spec[k * stride] = 0.0;
+    for (uint32_t t = G.first; t < t1; ++t) {
+      const bool neg = qs_par64(base & P.z[t]);
+      spec[P.spec[t] * stride] += neg ? -A.kre[t] : A.kre[t];
+      spec[((1u << D) + P.spec[t]) * stride] += neg ? -A.kim[t] : A.kim[t];
+    }
+    qs_xor_swap<D>(acc, G.xl ^ cur);
+    cur = G.xl;
+    double f[1 << D];
+#pragma unroll
+    for (int u = 0; u < (1 << D); ++u) f[u] = spec[u * stride];
+    qs_walsh<D>(f);
+#pragma unroll
+    for (int u = 0; u < (1 << D); ++u) {
+      acc[u].x += f[u] * a[u].x;
+      acc[u].y += f[u] * a[u].y;
+    }
+#pragma unroll
+    for (int u = 0; u < (1 << D); ++u) f[u] = spec[((1 << D) + u) * stride];
+    qs_walsh<D>(f);
+#pragma unroll
+    for (int u = 0; u < (1 << D); ++u) {
+      acc[u].x -= f[u] * a[u].y;
+      acc[u].y += f[u] * a[u].x;
+    }
+  }
+  qs_xor_swap<D>(acc, cur);
+#pragma unroll
+  for (int m = 0; m < (1 << D); ++m) out[base ^ P.off[m]] = acc[m];
+}
+
+// One work item of an adjoint sweep pass (plan.h): the rotations of P (reverse caller order,
+// negated angles) act on psi and lam together.  Before rotation r acts, acc[r * stride] gains this
+// item's share of Re sum_m conj(l[m]) t[m] with t = -i P psi, i.e. of Im<lam|P|psi>; t[m] is the
+// kappa sigma(m) b[m] of qs_pauli_rot_item.
+template <int D>
+QS_HD void qs_pauli_adjoint_item(const QsPauliRotPass& P, qs_c128* __restrict__ psi, qs_c128* __restrict__ lam,
+                                 uint64_t o, double* acc, uint32_t stride) {
+  uint64_t base = o;
+#pragma unroll
+  for (int i = 0; i < D; ++i) base = qs_insert_bit(base, P.pivot[i], 0);
+  qs_c128 a[1 << D], l[1 << D];
+#pragma unroll
+  for (int m = 0; m < (1 << D); ++m) {
+    a[m] = psi[base ^ P.off[m]];
+    l[m] = lam[base ^ P.off[m]];
+  }
+  for (uint32_t r = 0; r < P.nrot; ++r) {
+    const uint32_t xl = P.xl[r], spec = P.spec[r], cls = P.cls[r];
+    const double c = P.c[r];
+    const bool neg = qs_par64(base & P.z[r]) ^ (cls >> 1);
+    const double s = neg ? -P.s[r] : P.s[r];
+    qs_c128 b[1 << D], k[1 << D];
+#pragma unroll
+    for (int m = 0; m < (1 << D); ++m) {
+      b[m] = a[m];
+      k[m] = l[m];
+    }
+    qs_xor_swap<D>(b, xl);
+    qs_xor_swap<D>(k, xl);
+    if (cls & 1u) {                        // times i
+#pragma unroll
+      for (int m = 0; m < (1 << D); ++m) {
+        const double tb = b[m].x, tk = k[m].x;
+        b[m].x = -b[m].y;
+        b[m].y = tb;
+        k[m].x = -k[m].y;
+        k[m].y = tk;
+      }
+    }
+    double ov = 0.0;
+#pragma unroll
+    for (int m = 0; m < (1 << D); ++m) {
+      const double v = l[m].x * b[m].x + l[m].y * b[m].y;
+      ov += qs_par64(((uint32_t)m ^ xl) & spec) ? -v : v;
+    }
+    acc[r * stride] += neg ? -ov : ov;
+#pragma unroll
+    for (int m = 0; m < (1 << D); ++m) {
+      const double sm = qs_par64(((uint32_t)m ^ xl) & spec) ? -s : s;
+      a[m].x = c * a[m].x + sm * b[m].x;
+      a[m].y = c * a[m].y + sm * b[m].y;
+      l[m].x = c * l[m].x + sm * k[m].x;
+      l[m].y = c * l[m].y + sm * k[m].y;
+    }
+  }
+#pragma unroll
+  for (int m = 0; m < (1 << D); ++m) {
+    psi[base ^ P.off[m]] = a[m];
+    lam[base ^ P.off[m]] = l[m];
+  }
+}
+
 // Density matrix: entry c of tr(rho X^x Z^z) = sum_c (-1)^popc(c & z) rho[c, c ^ x] (the phase
 // i^popc(x & z) is applied by the host).  rho is the row-major vec of an N-qubit matrix.
 QS_HD qs_c128 qs_pauli_dm_elem(const qs_c128* __restrict__ rho, int N, uint64_t x, uint64_t z, uint64_t c) {

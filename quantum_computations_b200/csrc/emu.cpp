@@ -274,6 +274,45 @@ int apply_pauli_rotations(qs_c128* s, int n, const PauliRotPlan& plan, void*) {
   return QSIM_OK;
 }
 
+// one launch per pass, as in the CUDA library
+int apply_pauli_sum(const qs_c128* in, qs_c128* out, int n, const PauliApplyPlan& plan, void*) {
+  const uint64_t count = 1ull << (n - plan.d);
+  double spec[2 << QS_PAULI_MAX_D];
+  for (const QsPauliApplyPass& A : plan.passes) {
+    for (uint64_t o = 0; o < count; ++o) {
+      switch (plan.d) {
+        case 1: qs_pauli_apply_item<1>(A, in, out, o, spec, 1); break;
+        case 2: qs_pauli_apply_item<2>(A, in, out, o, spec, 1); break;
+        case 3: qs_pauli_apply_item<3>(A, in, out, o, spec, 1); break;
+        default: qs_pauli_apply_item<4>(A, in, out, o, spec, 1); break;
+      }
+    }
+    ++g_launches;
+  }
+  return QSIM_OK;
+}
+
+// one launch per pass plus the final sum, as in the CUDA library
+int pauli_rotations_adjoint(qs_c128* psi, qs_c128* lam, int n, const PauliRotPlan& plan, double* sums, void*) {
+  const uint64_t count = 1ull << (n - plan.d);
+  size_t row0 = 0;
+  for (const QsPauliRotPass& P : plan.passes) {
+    double acc[QS_PAULI_ROT_MAX] = {0.0};
+    for (uint64_t o = 0; o < count; ++o) {
+      switch (plan.d) {
+        case 1: qs_pauli_adjoint_item<1>(P, psi, lam, o, acc, 1); break;
+        case 2: qs_pauli_adjoint_item<2>(P, psi, lam, o, acc, 1); break;
+        default: qs_pauli_adjoint_item<QS_PAULI_ADJ_MAX_D>(P, psi, lam, o, acc, 1); break;
+      }
+    }
+    for (uint32_t r = 0; r < P.nrot; ++r) sums[2 * (row0 + r)] = acc[r];
+    row0 += P.nrot;
+    ++g_launches;
+  }
+  ++g_launches;                              // the final sum
+  return QSIM_OK;
+}
+
 int expect_pauli_dm(const qs_c128* rho, int n, int64_t n_terms, const uint64_t* xi, const uint64_t* zi,
                     double* sums, void*) {
   for (int64_t t = 0; t < n_terms; ++t)

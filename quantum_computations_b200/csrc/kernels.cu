@@ -788,6 +788,46 @@ k_pauli_rotate(qs_c128* __restrict__ state, const __grid_constant__ QsPauliRotPa
 }
 
 // =====================================================================================
+// H|psi> for a Pauli sum and the adjoint sweep (plan.h, elem_ops.h, pauli.cpp)
+// =====================================================================================
+// The apply pass has the rotation pass's grid; every thread keeps its group spectrum in shared
+// memory ([entry][thread]: conflict-free), where the terms scatter by a runtime index.
+template <int D>
+__global__ void __launch_bounds__(kRotThreads)
+k_pauli_apply(const qs_c128* __restrict__ in, qs_c128* __restrict__ out, const __grid_constant__ QsPauliApplyPass A,
+              uint64_t count) {
+  __shared__ double spec[(2 << D) * kRotThreads];
+  for (uint64_t o = blockIdx.x * (uint64_t)kRotThreads + threadIdx.x; o < count; o += (uint64_t)gridDim.x * kRotThreads)
+    qs_pauli_apply_item<D>(A, in, out, o, spec + threadIdx.x, kRotThreads);
+}
+
+// One sweep pass: psi and lam together, one accumulator per rotation and thread in shared memory;
+// the block writes one partial per rotation, to row row0 + r of the call's partials (k_pauli_final
+// sums them as it sums the expectation values' terms).
+constexpr int kAdjBlocksPerSM = 4;
+
+template <int D>
+__global__ void __launch_bounds__(kPauliThreads)
+k_pauli_adjoint(qs_c128* __restrict__ psi, qs_c128* __restrict__ lam, const __grid_constant__ QsPauliRotPass P,
+                uint64_t count, uint32_t row0, double* __restrict__ partials) {
+  __shared__ double acc[QS_PAULI_ROT_MAX * kPauliThreads];
+  for (uint32_t r = 0; r < P.nrot; ++r) acc[r * kPauliThreads + threadIdx.x] = 0.0;
+  for (uint64_t o = blockIdx.x * (uint64_t)kPauliThreads + threadIdx.x; o < count;
+       o += (uint64_t)gridDim.x * kPauliThreads)
+    qs_pauli_adjoint_item<D>(P, psi, lam, o, acc + threadIdx.x, kPauliThreads);
+  __syncthreads();
+  const int warp = threadIdx.x >> 5;
+  for (uint32_t r = warp; r < P.nrot; r += kPauliThreads / 32) {
+    const double s = pauli_warp_sum(acc + r * kPauliThreads);
+    if ((threadIdx.x & 31) == 0) {
+      double* dst = partials + 2 * ((uint64_t)(row0 + r) * gridDim.x + blockIdx.x);
+      dst[0] = s;
+      dst[1] = 0.0;
+    }
+  }
+}
+
+// =====================================================================================
 // Marginal probabilities (elem_ops.h, QsMargGeom): one read-only pass, then a fixed-tree final sum
 // =====================================================================================
 constexpr int kMargThreads = 256;
@@ -1640,6 +1680,58 @@ int apply_pauli_rotations(qs_c128* state, int n, const PauliRotPlan& plan, void*
     if (rc != QSIM_OK) return rc;
   }
   return QSIM_OK;
+}
+
+int apply_pauli_sum(const qs_c128* in, qs_c128* out, int n, const PauliApplyPlan& plan, void* stream) {
+  Bound bound;
+  int rc = bind_device(out, &bound);
+  DevCtx* ctx = bound.ctx;
+  if (rc != QSIM_OK) return rc;
+  const uint64_t count = 1ull << (n - plan.d);
+  const unsigned blocks = (unsigned)std::min<uint64_t>((count + kRotThreads - 1) / kRotThreads,
+                                                       (uint64_t)ctx->sms * kRotBlocksPerSM);
+  const cudaStream_t st = (cudaStream_t)stream;
+  for (const QsPauliApplyPass& A : plan.passes) {
+    switch (plan.d) {
+      case 1: k_pauli_apply<1><<<blocks, kRotThreads, 0, st>>>(in, out, A, count); break;
+      case 2: k_pauli_apply<2><<<blocks, kRotThreads, 0, st>>>(in, out, A, count); break;
+      case 3: k_pauli_apply<3><<<blocks, kRotThreads, 0, st>>>(in, out, A, count); break;
+      default: k_pauli_apply<4><<<blocks, kRotThreads, 0, st>>>(in, out, A, count); break;
+    }
+    rc = launched();
+    if (rc != QSIM_OK) return rc;
+  }
+  return QSIM_OK;
+}
+
+int pauli_rotations_adjoint(qs_c128* psi, qs_c128* lam, int n, const PauliRotPlan& plan, double* sums, void* stream) {
+  Bound bound;
+  int rc = bind_device(psi, &bound);
+  DevCtx* ctx = bound.ctx;
+  if (rc != QSIM_OK) return rc;
+  const uint64_t count = 1ull << (n - plan.d);
+  const unsigned blocks = (unsigned)std::min<uint64_t>((count + kPauliThreads - 1) / kPauliThreads,
+                                                       (uint64_t)ctx->sms * kAdjBlocksPerSM);
+  const int64_t rows = (int64_t)plan.caller.size();
+  const cudaStream_t st = (cudaStream_t)stream;
+  std::lock_guard<std::mutex> guard(ctx->reduce_lock);
+  rc = pauli_scratch(ctx, (size_t)rows, blocks);
+  if (rc != QSIM_OK) return rc;
+  uint32_t row0 = 0;
+  for (const QsPauliRotPass& P : plan.passes) {
+    double* partials = ctx->d_pauli_partials;
+    switch (plan.d) {
+      case 1: k_pauli_adjoint<1><<<blocks, kPauliThreads, 0, st>>>(psi, lam, P, count, row0, partials); break;
+      case 2: k_pauli_adjoint<2><<<blocks, kPauliThreads, 0, st>>>(psi, lam, P, count, row0, partials); break;
+      default:
+        k_pauli_adjoint<QS_PAULI_ADJ_MAX_D><<<blocks, kPauliThreads, 0, st>>>(psi, lam, P, count, row0, partials);
+        break;
+    }
+    rc = launched();
+    if (rc != QSIM_OK) return rc;
+    row0 += P.nrot;
+  }
+  return pauli_sums_to_host(ctx, rows, (int)blocks, sums, st);
 }
 
 int marginal_probs(const QsProbSrc& src, const QsMargGeom& G, double* out, void* stream) {

@@ -1,6 +1,7 @@
-// Host half of the Pauli-sum expectation values (qsim_expect_pauli / _dm) and of the Pauli-string
-// rotations (qsim_apply_pauli_rotations / _dm): argument checks, the reference-qubit -> index-bit
-// conversion and the packing of the terms into Pauli passes.  Shared verbatim by libqsim_b200.so
+// Host half of the Pauli-sum expectation values (qsim_expect_pauli / _dm), of H|psi>
+// (qsim_apply_pauli_sum / qsim_accumulate_pauli_sum), of the Pauli-string rotations (qsim_apply_pauli_rotations / _dm) and of
+// their adjoint sweep (qsim_pauli_rotations_adjoint / _dm): argument checks, the reference-qubit ->
+// index-bit conversion and the packing of the terms into Pauli passes.  Shared verbatim by libqsim_b200.so
 // and the host emulator, so the CPU tests check the very grouping the GPU runs.
 #include <algorithm>
 #include <cmath>
@@ -211,26 +212,72 @@ int plan_pauli(int n, int64_t n_terms, const uint64_t* x_masks, const uint64_t* 
   return QSIM_OK;
 }
 
+int plan_pauli_apply(int n, int64_t n_terms, const uint64_t* x_masks, const uint64_t* z_masks,
+                     const double* coeffs_re_im, bool accumulate, PauliApplyPlan* out) {
+  // no terms: the layout of one identity term, and a pass without groups that writes the zeros
+  const uint64_t none = 0;
+  PauliPlan plan;
+  const int rc = n_terms ? plan_pauli(n, n_terms, x_masks, z_masks, &plan) : plan_pauli(n, 1, &none, &none, &plan);
+  if (rc != QSIM_OK) return rc;
+  out->d = plan.d;
+  out->passes.clear();
+  for (const QsPauliPass& P : plan.passes) {
+    QsPauliApplyPass A;
+    memset(&A, 0, sizeof(A));
+    A.p = P;
+    A.accumulate = (accumulate || !out->passes.empty()) ? 1u : 0u;
+    if (n_terms == 0) A.p.ngroups = A.p.nterms = 0;
+    for (uint32_t t = 0; t < A.p.nterms; ++t) {
+      const int64_t term = plan.order[P.term0 + t];
+      const double re = coeffs_re_im[2 * term], im = coeffs_re_im[2 * term + 1];
+      switch (popc64(x_masks[term] & z_masks[term]) & 3) {     // times i^popc(x & z)
+        case 0: A.kre[t] = re; A.kim[t] = im; break;
+        case 1: A.kre[t] = -im; A.kim[t] = re; break;
+        case 2: A.kre[t] = -re; A.kim[t] = -im; break;
+        default: A.kre[t] = im; A.kim[t] = -re; break;
+      }
+    }
+    out->passes.push_back(A);
+  }
+  return QSIM_OK;
+}
+
 int plan_pauli_rotations(int n, int64_t n_rot, const uint64_t* x_masks, const uint64_t* z_masks, const double* angles,
-                         bool dm, PauliRotPlan* out) {
-  // the rotations on the register, in caller order; a unit is what must share a pass (for a density
-  // matrix the row and the column half of one caller rotation: they commute, and one pass holds both)
+                         bool dm, PauliRotPlan* out, bool adjoint) {
+  // the rotations on the register, in caller order (an adjoint sweep: reverse caller order, negated
+  // angles); a unit is what must share a pass (for a density matrix the row and the column half of
+  // one caller rotation: they commute, and one pass holds both)
   struct Rot { uint64_t x, z; double theta; int cls; };
   const int nreg = dm ? 2 * n : n;
   std::vector<Rot> rots;
   std::vector<size_t> unit_end;
-  for (int64_t t = 0; t < n_rot; ++t) {
-    if (angles[t] == 0.0) continue;                    // the identity
+  out->caller.clear();
+  out->weight.clear();
+  for (int64_t i = 0; i < n_rot; ++i) {
+    const int64_t t = adjoint ? n_rot - 1 - i : i;
+    // the identity; a sweep keeps it, for its derivative
+    if (angles[t] == 0.0 && !adjoint) continue;
+    const double theta = adjoint ? -angles[t] : angles[t];
     const int c = popc64(x_masks[t] & z_masks[t]) & 3;
     const int cls = (c + 3) & 3;                       // -i i^c
-    rots.push_back({to_index_bits(x_masks[t], nreg), to_index_bits(z_masks[t], nreg), angles[t], cls});
+    rots.push_back({to_index_bits(x_masks[t], nreg), to_index_bits(z_masks[t], nreg), theta, cls});
     // column half: conj(exp(-i theta/2 P)) = exp(+i theta/2 conj(P)) and conj(P) = (-1)^c P
     if (dm)
       rots.push_back({to_index_bits(x_masks[t] << n, nreg), to_index_bits(z_masks[t] << n, nreg),
-                      (c & 1) ? angles[t] : -angles[t], cls});
+                      (c & 1) ? theta : -theta, cls});
     unit_end.push_back(rots.size());
+    if (adjoint) {
+      // d/dtheta = d/dtheta_row + (+-1) d/dtheta_col, each half's overlap twice its derivative of
+      // the linear Re<<lam|rho>>
+      out->caller.push_back(t);
+      out->weight.push_back(dm ? 0.5 : 1.0);
+      if (dm) {
+        out->caller.push_back(t);
+        out->weight.push_back((c & 1) ? 0.5 : -0.5);
+      }
+    }
   }
-  const int d = std::min(nreg, QS_PAULI_MAX_D);
+  const int d = std::min(nreg, adjoint ? QS_PAULI_ADJ_MAX_D : QS_PAULI_MAX_D);
   out->d = d;
   out->passes.clear();
 
@@ -295,6 +342,11 @@ int plan_pauli_rotations(int n, int64_t n_rot, const uint64_t* x_masks, const ui
 
 void pauli_finish(const PauliPlan& plan, const double* sums, double* out) {
   for (size_t s = 0; s < plan.order.size(); ++s) out[plan.order[s]] = sums[2 * s];
+}
+
+void pauli_adjoint_finish(const PauliRotPlan& plan, int64_t n_rot, const double* sums, double* out) {
+  for (int64_t t = 0; t < n_rot; ++t) out[t] = 0.0;
+  for (size_t s = 0; s < plan.caller.size(); ++s) out[plan.caller[s]] += plan.weight[s] * sums[2 * s];
 }
 
 void pauli_finish_dm(int64_t n_terms, const std::vector<uint8_t>& phase, const double* sums, double* out_re_im) {

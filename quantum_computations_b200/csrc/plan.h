@@ -242,3 +242,25 @@ struct QsPauliRotPass {
   uint8_t  cls[QS_PAULI_ROT_MAX];            // kappa = -i i^popc(x & z) = i^cls
 };
 static_assert(sizeof(QsPauliRotPass) <= 4096, "QsPauliRotPass is a kernel parameter");
+
+// ---- H|psi> for a Pauli sum (qsim_apply_pauli_sum) -------------------------------------------
+// The terms are packed as for the expectation values (QsPauliPass: same grouping, layout and
+// spec), and every slot t carries k_t = c_t i^popc(x & z).  With b[m] = in[base ^ off[m ^ xl]]
+//     out[m] += sum_t k_t (-1)^(par(base & z_t) + popc((m ^ xl) & spec_t)) b[m] = F[m ^ xl] b[m],
+// F the Walsh transform of the spectrum that holds +-k_t at index spec_t: one transform per group,
+// whatever the number of its terms.  The first pass of a qsim_apply_pauli_sum call writes out, later
+// passes add to it; every pass of a qsim_accumulate_pauli_sum call adds.
+struct QsPauliApplyPass {
+  QsPauliPass p;
+  double   kre[QS_PAULI_MAX_TERMS];          // k_t, slot order of p
+  double   kim[QS_PAULI_MAX_TERMS];
+  uint32_t accumulate;                       // 0: write out; 1: add to it
+};
+static_assert(sizeof(QsPauliApplyPass) <= 4096, "QsPauliApplyPass is a kernel parameter");
+
+// ---- adjoint sweep (qsim_pauli_rotations_adjoint / _dm) ----------------------------------------
+// A sweep pass is a QsPauliRotPass whose rotations are in reverse caller order with negated angles,
+// applied to two states at once; a work item holds 2^d amplitudes of each, so the kernel keeps four
+// times the amplitudes of one state in registers.  Generators per sweep pass (no register spills
+// for sm_100a; DESIGN.md section 3.2.4 lists the registers of every d):
+#define QS_PAULI_ADJ_MAX_D 3

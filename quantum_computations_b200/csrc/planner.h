@@ -107,19 +107,38 @@ struct PauliPlan {
 // Greedy grouping by X mask: at most one pass per chunk of <= QS_PAULI_MAX_TERMS terms of one
 // non-zero X mask, the Z strings in passes with room (a pass of their own only if none has).
 int plan_pauli(int n, int64_t n_terms, const uint64_t* x_masks, const uint64_t* z_masks, PauliPlan* out);
-// The rotation passes of one qsim_apply_pauli_rotations(_dm) call, in caller order.
+// The passes of one qsim_apply_pauli_sum / qsim_accumulate_pauli_sum call: plan_pauli's, each slot
+// with k_t = c_t i^popc(x & z).  The first pass writes out, or adds to it with `accumulate`; with no
+// terms one pass that writes zeros (the caller launches nothing when it accumulates).
+struct PauliApplyPlan {
+  int d = 0;
+  std::vector<QsPauliApplyPass> passes;
+};
+int plan_pauli_apply(int n, int64_t n_terms, const uint64_t* x_masks, const uint64_t* z_masks,
+                     const double* coeffs_re_im, bool accumulate, PauliApplyPlan* out);
+// The rotation passes of one qsim_apply_pauli_rotations(_dm) call, in caller order, or of one
+// adjoint sweep.
 struct PauliRotPlan {
-  int d = 0;                                 // generators per pass: min(register bits, QS_PAULI_MAX_D)
+  int d = 0;                                 // generators per pass: min(register bits, QS_PAULI_MAX_D
+                                             // or, for a sweep, QS_PAULI_ADJ_MAX_D)
   std::vector<QsPauliRotPass> passes;
+  // sweeps only: per rotation slot (pass by pass) its caller rotation and the weight of its
+  // overlap in that rotation's derivative
+  std::vector<int64_t> caller;
+  std::vector<double> weight;
 };
 // Greedy in caller order, never reordered: a rotation joins the open pass while the cap allows and
 // its X mask is in the span or the span has room; angle-0 rotations are skipped.  dm: n is N and
 // every rotation becomes its row half and its conjugated column half on the 2N-bit vec of rho,
-// always in one pass.
+// always in one pass.  adjoint: the sweep of qsim_pauli_rotations_adjoint -- the same packing of
+// the rotations in reverse caller order with negated angles, angle-0 rotations kept, at most
+// QS_PAULI_ADJ_MAX_D generators per pass.
 int plan_pauli_rotations(int n, int64_t n_rot, const uint64_t* x_masks, const uint64_t* z_masks, const double* angles,
-                         bool dm, PauliRotPlan* out);
+                         bool dm, PauliRotPlan* out, bool adjoint = false);
 // sums: 2 doubles per slot (re, im) -> out[caller term] (real).
 void pauli_finish(const PauliPlan& plan, const double* sums, double* out);
+// sums: 2 doubles per sweep slot -> out[caller rotation] = sum of weight x overlap, in slot order.
+void pauli_adjoint_finish(const PauliRotPlan& plan, int64_t n_rot, const double* sums, double* out);
 // sums: 2 doubles per term, times i^phase -> out_re_im.
 void pauli_finish_dm(int64_t n_terms, const std::vector<uint8_t>& phase, const double* sums, double* out_re_im);
 

@@ -450,6 +450,48 @@ class DeviceState:
         self.host_dtype = np.dtype(np.complex128)
         return self
 
+    def apply_pauli_sum(self, x_masks, z_masks, coeffs, out: "DeviceState | None" = None) -> "DeviceState":
+        """H|psi> for a ket, H rho for a density matrix, with H = sum_t coeffs[t] P_t (complex
+        coefficients, strings as in ``expect_pauli``), into a new state or into ``out`` (a state of
+        the same kind and size in another buffer); returns the result.  The state is unchanged."""
+        x = np.ascontiguousarray(x_masks, dtype=np.uint64).reshape(-1)
+        z = np.ascontiguousarray(z_masks, dtype=np.uint64).reshape(-1)
+        c = np.ascontiguousarray(coeffs, dtype=np.complex128).reshape(-1)
+        if x.shape != z.shape or x.shape != c.shape:
+            raise ValueError("x_masks, z_masks and coeffs must have the same length")
+        if self.ndim == 2 and len(x) and (int(x.max()) >> self.num_qubits or int(z.max()) >> self.num_qubits):
+            raise ValueError("a Pauli mask has a bit at or above n_qubits")
+        be = self.backend
+        if out is None:
+            out = DeviceState(be, be.empty(1 << self.n_bits), self.n_bits, self.ndim)
+        elif out.ndim != self.ndim or out.n_bits != self.n_bits:
+            raise ValueError("out must be a state of the same kind and size")
+        # a density matrix is its vec: a 2N-qubit ket whose qubits 0..N-1 are the row qubits of rho
+        _capi.check(be.lib, be.lib.qsim_apply_pauli_sum(be.ptr(self.buf), be.ptr(out.buf), self.n_bits, len(x),
+                                                        x.ctypes.data, z.ctypes.data, c.ctypes.data, be.stream()))
+        out.host_dtype = np.dtype(np.complex128)
+        return out
+
+    def pauli_rotations_adjoint(self, lam: "DeviceState", x_masks, z_masks, angles) -> np.ndarray:
+        """The backward sweep of the adjoint method (``qsim_pauli_rotations_adjoint`` / ``_dm``) over
+        U = R_{k-1} ... R_0, the rotation list of ``apply_pauli_rotations``, in place on two states:
+        ``self`` (psi = U psi0 on entry) returns to psi0 and ``lam`` becomes U^dagger lam.  Returns
+        out[t] = Im<lam_t|P_t|psi_t> (kets; d<H>/d theta_t when lam = H psi) or d Re<<lam|rho>>/d theta_t
+        (density matrices) as float64, in caller order.  Synchronises."""
+        x = np.ascontiguousarray(x_masks, dtype=np.uint64).reshape(-1)
+        z = np.ascontiguousarray(z_masks, dtype=np.uint64).reshape(-1)
+        a = np.ascontiguousarray(angles, dtype=np.float64).reshape(-1)
+        if x.shape != z.shape or x.shape != a.shape:
+            raise ValueError("x_masks, z_masks and angles must have the same length")
+        if lam.ndim != self.ndim or lam.n_bits != self.n_bits:
+            raise ValueError("psi and lam must be states of the same kind and size")
+        lib, be = self.backend.lib, self.backend
+        fn = lib.qsim_pauli_rotations_adjoint if self.ndim == 1 else lib.qsim_pauli_rotations_adjoint_dm
+        out = np.zeros(len(x), dtype=np.float64)
+        _capi.check(lib, fn(be.ptr(self.buf), be.ptr(lam.buf), self.num_qubits, len(x), x.ctypes.data, z.ctypes.data,
+                            a.ctypes.data, out.ctypes.data, be.stream()))
+        self.host_dtype = lam.host_dtype = np.dtype(np.complex128)
+        return out
 
     # -- measurement statistics ------------------------------------------------------------------
     def probabilities(self, qubits=None, *, device: bool = False):

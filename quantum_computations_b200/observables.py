@@ -14,6 +14,10 @@ The same masks drive evolution: ``evolve`` applies a Trotterised exp(-i H t) for
 device or sharded state, ``qsim_apply_pauli_rotations``), up to 32 rotations per read
 and write of the state.
 
+``apply`` gives H|psi> (or H rho) for a ``PauliSum`` on the device (``qsim_apply_pauli_sum``), and
+``expect_and_gradient`` gives <H> after a rotation list together with its gradient with respect to
+every angle, by the adjoint method (``qsim_pauli_rotations_adjoint``).
+
 Convention: a string is a pair of masks ``(x, z)`` with bit q for reference
 qubit q; I = (0, 0), X = (1, 0), Z = (0, 1), Y = (1, 1), and the operator is
 ``i^popc(x & z) X^x Z^z`` (Z first), so every string is Hermitian.
@@ -144,6 +148,83 @@ def expect(observable: PauliSum, state, *, per_term: bool = False):
     if per_term:
         return values
     return complex(np.dot(observable.coeffs, values))
+
+
+def _device_state(state, num_qubits: int, what: str):
+    """``state`` itself if sharded or on the device, else uploaded; refuses a sharded density matrix and
+    an operator wider than the state."""
+    from . import engine
+    if isinstance(state, _sharded_type()):
+        if state.is_density:
+            raise NotImplementedError(f"a {what} on a sharded density matrix is not implemented")
+        width = state.n
+    else:
+        if not isinstance(state, engine.DeviceState):
+            state = engine.DeviceState.from_numpy(np.asarray(state))
+        width = state.num_qubits
+    if num_qubits > width:
+        raise ValueError(f"the {what} acts on {num_qubits} qubits, the state has {width}")
+    return state
+
+
+def apply(operator: PauliSum, state):
+    """H|psi> for a ket, H rho for a density matrix, as a new state (``qsim_apply_pauli_sum``: one
+    read of the state and one write of the result per pass of up to 32 strings); the state is
+    unchanged.  ``state``: an ``engine.DeviceState``, a ``sharded.ShardedState`` ket (collective, a new
+    sharded ket; a sharded density matrix raises NotImplementedError) or a host ndarray, uploaded first.  Complex coefficients are allowed."""
+    if not isinstance(operator, PauliSum):
+        raise TypeError("apply needs a PauliSum operator")
+    state = _device_state(state, operator.num_qubits, "operator")
+    return state.apply_pauli_sum(operator.x_masks, operator.z_masks, operator.coeffs)
+
+
+def _vec_identity(backend, n: int):
+    """vec(I) of an n-qubit identity on the device: |+>^n (unnormalised) on the row qubits, |0>^n on
+    the column qubits, then a CNOT from every row qubit to its column qubit."""
+    from . import engine
+    ket = engine.DeviceState.product([np.array([1.0, 1.0])] * n + [np.array([1.0, 0.0])] * n, backend)
+    cnot = np.eye(4, dtype=np.complex128)[[0, 1, 3, 2]]
+    engine.apply_lowered(ket, [([q, q + n], cnot) for q in range(n)])
+    return engine.DeviceState(backend, ket.buf, 2 * n, 2)
+
+
+def expect_and_gradient(hamiltonian: PauliSum, rotations, state):
+    """(E, dE/dtheta) for E(theta) = <H> on U(theta) state, U = R_{k-1} ... R_0 the rotation list
+    ``rotations = (x_masks, z_masks, angles)`` of ``trotter_rotations`` / ``apply_pauli_rotations``,
+    by the adjoint method: one forward sweep, one application of H and one backward sweep
+    (``qsim_pauli_rotations_adjoint``), whatever k is.  E is a float, the gradient a float64 array in
+    caller order.  Parameters shared between rotations (QAOA's gamma on every ZZ term) are the
+    caller's chain rule: sum the entries of the rotations that share one.
+
+    ``state``: a ket or density matrix (``engine.DeviceState``, or a host ndarray, uploaded first) or
+    a ``sharded.ShardedState`` ket (collective; a sharded density matrix raises NotImplementedError).  It is left unchanged: the work happens on two
+    scratch states of its size, psi = U state and lam = H psi (for a density matrix lam = vec(H)).
+    H must have real coefficients."""
+    if not isinstance(hamiltonian, PauliSum):
+        raise TypeError("expect_and_gradient needs a PauliSum Hamiltonian")
+    if np.any(hamiltonian.coeffs.imag != 0):
+        raise ValueError("the Hamiltonian has a coefficient with a nonzero imaginary part (not Hermitian)")
+    x, z, angles = rotations
+    state = _device_state(state, hamiltonian.num_qubits, "Hamiltonian")
+    if getattr(state, "ndim", 1) == 1:
+        psi = state.copy().apply_pauli_rotations(x, z, angles)
+        lam = psi.apply_pauli_sum(hamiltonian.x_masks, hamiltonian.z_masks, hamiltonian.coeffs)
+        value = psi.inner(lam).real
+    else:
+        from . import engine
+        # vec(H) first, so that vec(I) is gone before the copy of rho is made
+        lam = _vec_identity(state.backend, state.num_qubits).apply_pauli_sum(
+            hamiltonian.x_masks, hamiltonian.z_masks, hamiltonian.coeffs)
+        psi = state.copy().apply_pauli_rotations(x, z, angles)
+        as_ket = lambda s: engine.DeviceState(s.backend, s.buf, s.n_bits, 1)     # noqa: E731
+        value = as_ket(lam).inner(as_ket(psi)).real                              # Re tr(H^dagger rho)
+    grad = psi.pauli_rotations_adjoint(lam, x, z, angles)
+    if isinstance(state, _sharded_type()):
+        # after the sweep's all-reduce no rank exchanges with these shards any more: release their
+        # exchange staging and peer mappings now rather than whenever they are collected
+        psi.close()
+        lam.close()
+    return float(value), grad
 
 
 def trotter_rotations(hamiltonian: PauliSum, time: float, steps: int = 1, order: int = 1):

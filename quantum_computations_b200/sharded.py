@@ -89,7 +89,7 @@ class Comm:
 class ShardedState:
     """One rank's shard plus the logical->physical bit table (same on all ranks)."""
 
-    def __init__(self, n: int, comm: Comm, backend=None, as_torch=None):
+    def __init__(self, n: int, comm: Comm, backend=None, as_torch=None, buf=None):
         self.n = int(n)
         self.comm = comm
         self.g = comm.size.bit_length() - 1
@@ -99,7 +99,7 @@ class ShardedState:
         self.backend = backend or engine.get_backend()
         self.phys = list(range(self.n))           # phys[logical bit] = physical bit
         self.flip = [0] * self.g                  # flip[i]: rank bit i holds the complemented logical value
-        self.buf = self.backend.empty(1 << self.n_local)
+        self.buf = self.backend.empty(1 << self.n_local) if buf is None else buf
         self.swaps = 0
         self.swap_seconds = 0.0
         self.amps_sent = 0
@@ -188,25 +188,154 @@ class ShardedState:
         values = np.zeros(len(x), dtype=np.float64)
         remaining = list(range(len(x)))
         while remaining:
-            is_local = lambda bits: all(self.phys[l] < self.n_local for l in bits)   # noqa: E731
-            chosen = [t for t in remaining if is_local(xs[t])]
-            support = set().union(*[xs[t] for t in chosen])
-            for t in remaining:
-                if t in chosen:
-                    continue
-                wider = support | xs[t]
-                need = [l for l in wider if self.phys[l] >= self.n_local]
-                free = [l for l in range(n) if self.phys[l] < self.n_local and l not in wider]
-                if len(need) <= len(free):
-                    chosen.append(t)
-                    support = wider
-            if not chosen:
-                raise NotImplementedError("a Pauli string's X/Y support is wider than a shard; use fewer ranks")
+            chosen, support = self._next_batch(remaining, xs)
             self._localise(support)
             self._expect_local(sorted(chosen), x, xs, zs, values)
             done = set(chosen)
             remaining = [t for t in remaining if t not in done]
         return self.comm.allreduce_sum(values)
+
+    def _next_batch(self, remaining, xs):
+        """The terms of ``remaining`` (order free: they commute) that one ``_localise`` can serve: those
+        whose X support is local already, then any whose support still fits; and their joint support."""
+        n = self.n
+        is_local = lambda bits: all(self.phys[l] < self.n_local for l in bits)   # noqa: E731
+        chosen = [t for t in remaining if is_local(xs[t])]
+        support = set().union(*[xs[t] for t in chosen])
+        for t in remaining:
+            if t in chosen:
+                continue
+            wider = support | xs[t]
+            need = [l for l in wider if self.phys[l] >= self.n_local]
+            free = [l for l in range(n) if self.phys[l] < self.n_local and l not in wider]
+            if len(need) <= len(free):
+                chosen.append(t)
+                support = wider
+        if not chosen:
+            raise NotImplementedError("a Pauli string's X/Y support is wider than a shard; use fewer ranks")
+        return chosen, support
+
+    def _pauli_args(self, x_masks, z_masks, values, what: str):
+        """Checks the masks of a collective Pauli call against ``values`` (its coefficients or angles) and
+        returns the logical bits of every X and Z mask (logical bit l = n-1-q of reference qubit q)."""
+        if self.is_density:
+            raise NotImplementedError(f"{what} of a sharded density matrix are not implemented")
+        x = np.ascontiguousarray(x_masks, dtype=np.uint64).reshape(-1)
+        z = np.ascontiguousarray(z_masks, dtype=np.uint64).reshape(-1)
+        if x.shape != z.shape or x.shape != values.shape:
+            raise ValueError("the masks and the coefficients or angles must have the same length")
+        n = self.n
+        if len(x) and (int(x.max()) >> n or int(z.max()) >> n):
+            raise ValueError("a Pauli mask has a bit at or above the number of qubits")
+        xs = [{n - 1 - q for q in range(n) if int(v) >> q & 1} for v in x]
+        zs = [{n - 1 - q for q in range(n) if int(v) >> q & 1} for v in z]
+        return xs, zs
+
+    def _local_masks(self, terms, xs, zs):
+        """Shard masks of ``terms`` (X supports local) and the sign (-1)^v that their Z factors on rank
+        qubits contribute on this rank, v the logical values (flip flags included)."""
+        nl = self.n_local
+        lx = np.zeros(len(terms), dtype=np.uint64)
+        lz = np.zeros(len(terms), dtype=np.uint64)
+        sign = np.ones(len(terms))
+        for k, t in enumerate(terms):
+            for l in xs[t]:
+                lx[k] |= np.uint64(1 << (nl - 1 - self.phys[l]))         # shard reference qubit
+            for l in zs[t]:
+                p = self.phys[l]
+                if p < nl:
+                    lz[k] |= np.uint64(1 << (nl - 1 - p))
+                elif self.rank_value(p):
+                    sign[k] = -sign[k]
+        return lx, lz, sign
+
+    def empty_like(self, buf=None) -> "ShardedState":
+        """A state of the same kind (ket or vec of a density matrix), register and ranks in the same
+        layout (``phys`` / ``flip``) on ``buf`` (default: a new shard, uninitialised)."""
+        out = ShardedState(self.n, self.comm, self.backend, self._as_torch, buf)
+        out.phys, out.flip = list(self.phys), list(self.flip)
+        out.is_density = self.is_density
+        return out
+
+    def copy(self) -> "ShardedState":
+        return self.empty_like(self.backend.clone(self.buf))
+
+    def apply_pauli_sum(self, x_masks, z_masks, coeffs) -> "ShardedState":
+        """H|psi> with H = sum_t coeffs[t] P_t (``engine.DeviceState.apply_pauli_sum``) as a new sharded
+        ket; a collective.  This state is logically unchanged (its layout may change, as in
+        ``expect_pauli``); the result ends in the same layout.
+
+        Terms are taken in batches that one ``_localise`` serves, with this state and the result
+        localised in lockstep.  A Z factor on a rank qubit becomes a sign on the coefficient.  The first
+        batch is written by ``qsim_apply_pauli_sum``, every later one is added to the result in place by
+        ``qsim_accumulate_pauli_sum``."""
+        c = np.ascontiguousarray(coeffs, dtype=np.complex128).reshape(-1)
+        xs, zs = self._pauli_args(x_masks, z_masks, c, "Pauli sums")
+        if not np.all(np.isfinite(c)):
+            raise ValueError("non-finite coefficient")
+        be = self.backend
+        out = None
+        remaining = list(range(len(c)))
+        while out is None or remaining:
+            chosen, support = self._next_batch(remaining, xs) if remaining else ([], set())
+            self._localise(support)
+            if out is None:
+                out = self.empty_like()
+                fn = be.lib.qsim_apply_pauli_sum
+            else:
+                out._localise(support)
+                fn = be.lib.qsim_accumulate_pauli_sum
+            terms = sorted(chosen)
+            lx, lz, sign = self._local_masks(terms, xs, zs)
+            lc = np.ascontiguousarray(c[terms] * sign, dtype=np.complex128)
+            _capi.check(be.lib, fn(be.ptr(self.buf), be.ptr(out.buf), self.n_local, len(terms), lx.ctypes.data,
+                                   lz.ctypes.data, lc.ctypes.data, be.stream()))
+            done = set(chosen)
+            remaining = [t for t in remaining if t not in done]
+        return out
+
+    def pauli_rotations_adjoint(self, lam: "ShardedState", x_masks, z_masks, angles) -> np.ndarray:
+        """The adjoint sweep (``engine.DeviceState.pauli_rotations_adjoint``) on this ket (psi = U psi0
+        on entry, psi0 on return) and ``lam`` (U^dagger lam on return), a collective; returns
+        Im<lam_t|P_t|psi_t> for every rotation in caller order, identical on every rank.
+
+        ``lam`` must be laid out as this state (``inner`` accepts the pair).  The rotations are cut,
+        from the last one back, into runs whose joint X/Y support fits in a shard; both states are made
+        local in lockstep (``_localise`` is deterministic) and swept with one
+        ``qsim_pauli_rotations_adjoint`` call per run.  A Z factor on a rank qubit negates the angle and
+        the overlap where its logical value is 1.  The gradients are all-reduced once."""
+        a = np.ascontiguousarray(angles, dtype=np.float64).reshape(-1)
+        xs, zs = self._pauli_args(x_masks, z_masks, a, "Pauli rotations")
+        if lam.n != self.n or lam.phys != self.phys or lam.flip != self.flip:
+            raise ValueError("psi and lam are laid out differently")
+        if not np.all(np.isfinite(a)):
+            raise ValueError("non-finite angle")
+        if any(len(s) > self.n_local for s in xs):
+            raise NotImplementedError("a Pauli string's X/Y support is wider than a shard; use fewer ranks")
+        n, be = self.n, self.backend
+        grads = np.zeros(len(a), dtype=np.float64)
+        end = len(a)
+        while end > 0:
+            support, start = set(xs[end - 1]), end - 1
+            while start > 0:
+                wider = support | xs[start - 1]
+                need = [l for l in wider if self.phys[l] >= self.n_local]
+                free = [l for l in range(n) if self.phys[l] < self.n_local and l not in wider]
+                if len(need) > len(free):
+                    break
+                support, start = wider, start - 1
+            self._localise(support)
+            lam._localise(support)
+            run = list(range(start, end))
+            lx, lz, sign = self._local_masks(run, xs, zs)
+            la = np.ascontiguousarray(a[run] * sign)
+            out = np.zeros(len(run), dtype=np.float64)
+            _capi.check(be.lib, be.lib.qsim_pauli_rotations_adjoint(
+                be.ptr(self.buf), be.ptr(lam.buf), self.n_local, len(run), lx.ctypes.data, lz.ctypes.data,
+                la.ctypes.data, out.ctypes.data, be.stream()))
+            grads[start:end] = sign * out
+            end = start
+        return self.comm.allreduce_sum(grads)
 
     def expect(self, observable, per_term: bool = False):
         """``observables.expect`` on this sharded ket (collective)."""
@@ -256,22 +385,11 @@ class ShardedState:
 
     def _rotate_local(self, run, xs, zs, angles) -> None:
         """The rotations ``run`` (X supports local) on this shard, Z factors on rank qubits as signs."""
-        nl = self.n_local
         run = list(run)
-        lx = np.zeros(len(run), dtype=np.uint64)
-        lz = np.zeros(len(run), dtype=np.uint64)
-        la = np.array(angles[run], dtype=np.float64)
-        for k, t in enumerate(run):
-            for l in xs[t]:
-                lx[k] |= np.uint64(1 << (nl - 1 - self.phys[l]))         # shard reference qubit
-            for l in zs[t]:
-                p = self.phys[l]
-                if p < nl:
-                    lz[k] |= np.uint64(1 << (nl - 1 - p))
-                elif self.rank_value(p):
-                    la[k] = -la[k]
+        lx, lz, sign = self._local_masks(run, xs, zs)
+        la = np.ascontiguousarray(angles[run] * sign)
         be = self.backend
-        _capi.check(be.lib, be.lib.qsim_apply_pauli_rotations(be.ptr(self.buf), nl, len(run), lx.ctypes.data,
+        _capi.check(be.lib, be.lib.qsim_apply_pauli_rotations(be.ptr(self.buf), self.n_local, len(run), lx.ctypes.data,
                                                               lz.ctypes.data, la.ctypes.data, be.stream()))
 
     def _localise(self, support) -> None:
@@ -299,22 +417,10 @@ class ShardedState:
 
     def _expect_local(self, terms, x, xs, zs, values) -> None:
         """values[t] += this rank's share of <P_t> for terms whose X support is local."""
-        nl = self.n_local
-        lx = np.zeros(len(terms), dtype=np.uint64)
-        lz = np.zeros(len(terms), dtype=np.uint64)
-        sign = np.ones(len(terms))
-        for k, t in enumerate(terms):
-            for l in xs[t]:
-                lx[k] |= np.uint64(1 << (nl - 1 - self.phys[l]))         # shard reference qubit
-            for l in zs[t]:
-                p = self.phys[l]
-                if p < nl:
-                    lz[k] |= np.uint64(1 << (nl - 1 - p))
-                elif self.rank_value(p):
-                    sign[k] = -sign[k]
+        lx, lz, sign = self._local_masks(terms, xs, zs)
         be = self.backend
         out = np.zeros(len(terms), dtype=np.float64)
-        _capi.check(be.lib, be.lib.qsim_expect_pauli(be.ptr(self.buf), nl, len(terms), lx.ctypes.data, lz.ctypes.data,
+        _capi.check(be.lib, be.lib.qsim_expect_pauli(be.ptr(self.buf), self.n_local, len(terms), lx.ctypes.data, lz.ctypes.data,
                                                      out.ctypes.data_as(_capi.c_double_p), be.stream()))
         values[terms] += sign * out
 

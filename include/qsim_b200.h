@@ -264,28 +264,22 @@ int qsim_traj_batch(int n_qubits, int64_t shots, int n_ops, const int32_t* ops, 
  * amplitudes whose k local bits spell the PARTNER's rank bits, and receives into the
  * same positions (k = 1 is the plain global<->local swap of half a shard).  These two
  * kernels gather such a block into a contiguous send buffer and scatter a received
- * block back; the transfer itself is the caller's (P2P copy or NCCL/gloo send/recv).
+ * block back; the transfer itself is the caller's (NCCL/gloo send/recv).
  * local_qubits[i] (reference-style numbering inside the shard) is fixed to
- * bit_values[i]; first/count select a chunk of the block (for pipelining); the buffer
- * holds `count` amplitudes.  nbits <= 8. */
+ * bit_values[i]; first/count select a chunk of the block; the buffer holds `count`
+ * amplitudes.  nbits <= 8. */
 int qsim_swap_pack(const void* shard, void* sendbuf, int n_local, int nbits, const int* local_qubits,
                    const int* bit_values, uint64_t first, uint64_t count, void* stream);
 int qsim_swap_unpack(void* shard, const void* recvbuf, int n_local, int nbits, const int* local_qubits,
                      const int* bit_values, uint64_t first, uint64_t count, void* stream);
 
-/* ---- peer-to-peer staging for the exchanges (one process per GPU) --------------------
- * The travelling blocks move with the copy engines, not with SM kernels: every rank packs
- * a chunk into a library-allocated staging buffer, exports its RECEIVE staging once through
- * CUDA IPC, and PUSHES each packed chunk into the partner's receive staging over NVLink
- * with cudaMemcpyAsync (writes are the fast direction of NVLink P2P) while both GPUs' SMs
- * keep gathering / scattering the neighbouring chunks.  Ordering between the two
- * processes is the caller's (stream-ordered token exchanges, see sharded.py). */
-int qsim_peer_alloc(int device, uint64_t bytes, void** out_ptr);       /* cudaMalloc                      */
-int qsim_peer_free(void* ptr);
-int qsim_ipc_export(void* ptr, unsigned char* handle64);               /* 64-byte cudaIpcMemHandle_t      */
+/* ---- exchanges over NVLink peer memory (one process per GPU) -------------------------
+ * Every rank exports its shard once through CUDA IPC and maps the other ranks' shards
+ * into its own address space; the exchange is then one kernel per rank that reads and
+ * writes the partners' shards directly.  Handles are 64-byte cudaIpcMemHandle_t.
+ * qsim_ipc_import maps a handle on `device`; qsim_ipc_release unmaps what it returned. */
 int qsim_ipc_import(int device, const unsigned char* handle64, void** out_ptr);
 int qsim_ipc_release(void* imported_ptr);
-int qsim_peer_copy(void* dst, const void* src, uint64_t bytes, void* stream);
 /* CUDA-IPC handle of the allocation that holds `ptr` (any cudaMalloc'ed memory, e.g. a
  * PyTorch tensor) and the byte offset of `ptr` inside it: the importer adds the offset to
  * what qsim_ipc_import returns. */

@@ -105,12 +105,8 @@ SIGNATURES = {
                                  C.c_uint64, C.c_uint64, C.c_void_p]),
     "qsim_swap_unpack": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.POINTER(C.c_int), C.POINTER(C.c_int),
                                    C.c_uint64, C.c_uint64, C.c_void_p]),
-    "qsim_peer_alloc": (C.c_int, [C.c_int, C.c_uint64, c_void_pp]),
-    "qsim_peer_free": (C.c_int, [C.c_void_p]),
-    "qsim_ipc_export": (C.c_int, [C.c_void_p, C.c_char_p]),
     "qsim_ipc_import": (C.c_int, [C.c_int, C.c_char_p, c_void_pp]),
     "qsim_ipc_release": (C.c_int, [C.c_void_p]),
-    "qsim_peer_copy": (C.c_int, [C.c_void_p, C.c_void_p, C.c_uint64, C.c_void_p]),
     "qsim_ipc_export_ex": (C.c_int, [C.c_void_p, C.c_char_p, C.POINTER(C.c_uint64)]),
     "qsim_exchange_p2p": (C.c_int, [C.c_void_p, C.POINTER(C.c_void_p), C.c_int, C.c_int, C.POINTER(C.c_int),
                                     C.POINTER(C.c_int), C.POINTER(C.c_int), C.c_void_p]),

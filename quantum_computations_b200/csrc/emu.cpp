@@ -478,24 +478,12 @@ extern "C" {
 int qsim_has_cuda(void) { return 0; }
 int64_t qsim_launch_count(void) { return g_launches; }
 
-// peer staging: the emulator has one address space; these are plain host operations
-int qsim_peer_alloc(int, uint64_t bytes, void** out_ptr) {
-  if (!out_ptr || bytes == 0) return qs::fail(QSIM_ERR_ARG, "qsim_peer_alloc: bad argument");
-  *out_ptr = malloc(bytes);
-  return *out_ptr ? QSIM_OK : qs::fail(QSIM_ERR_NOMEM, "out of host memory");
-}
-int qsim_peer_free(void* ptr) { free(ptr); return QSIM_OK; }
-int qsim_ipc_export(void*, unsigned char*) { return qs::fail(QSIM_ERR_UNSUPPORTED, "no IPC in the host emulator"); }
+// peer memory: the emulator has no IPC; its exchanges go through qsim_swap_pack / _unpack
 int qsim_ipc_import(int, const unsigned char*, void**) { return qs::fail(QSIM_ERR_UNSUPPORTED, "no IPC in the host emulator"); }
 int qsim_ipc_release(void*) { return QSIM_OK; }
 int qsim_ipc_export_ex(void*, unsigned char*, uint64_t*) { return qs::fail(QSIM_ERR_UNSUPPORTED, "no IPC in the host emulator"); }
 int qsim_exchange_p2p(void*, void* const*, int, int, const int*, const int*, const int*, void*) {
   return qs::fail(QSIM_ERR_UNSUPPORTED, "no peer memory in the host emulator (the exchange goes through send/recv)");
-}
-int qsim_peer_copy(void* dst, const void* src, uint64_t bytes, void*) {
-  if (!dst || !src) return qs::fail(QSIM_ERR_ARG, "qsim_peer_copy: null argument");
-  memcpy(dst, src, bytes);
-  return QSIM_OK;
 }
 
 // Test-only: shared-memory wavefronts of the 128-bit step accesses of a plan, as the

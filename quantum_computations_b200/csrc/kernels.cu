@@ -466,18 +466,21 @@ struct ExchGeom {
   int mine[8];                // this rank's value of the rank bit traded against pos[i]
   qs_c128* peer[256];         // peer[d]: partner shard for the bit pattern d (over pos[] order); [0] unused
   unsigned char higher[256];  // higher[d] = 1 if this rank's number is above the partner's
-  int chunk_log2;             // > 0: work is dealt to the partners in chunks of 2^chunk_log2 pairs (round robin),
-                              // so that all 2^k - 1 partners are being talked to at any time; 0: partner after partner
 };
 constexpr int kExchSplitBit = 5;
+// U = kExchPairs pairs per thread and trip: all 2 U loads (U of them over NVLink) are issued
+// before the first store, which is what keeps enough bytes in flight to cover the NVLink round
+// trip.  The grid is capped at kExchCtasPerSm CTAs per SM.  On 2 and 8 B200s neither 1, 2 or 8
+// pairs, nor 4 or 16 CTAs per SM, nor dealing the work to the partners round robin measured
+// faster: the kernel is bound by NVLink (DESIGN.md section 5).
+constexpr int kExchPairs = 4, kExchCtasPerSm = 8;
 
-// U pairs per thread and trip: all 2 U loads (U of them over NVLink) are issued before the
-// first store, which is what keeps enough bytes in flight to cover the NVLink round trip.
-template <int U>
 __global__ void __launch_bounds__(256)
 k_exchange_p2p(qs_c128* __restrict__ shard, const __grid_constant__ ExchGeom G) {
+  constexpr int U = kExchPairs;
   const int k = G.k;
-  const uint64_t half = 1ull << (G.n_local - k - 1);          // amplitudes per partner that THIS rank moves
+  const int half_log2 = G.n_local - k - 1;
+  const uint64_t half = 1ull << half_log2;                    // amplitudes per partner that THIS rank moves
   const uint64_t total = half * ((1ull << k) - 1ull);
   const uint64_t stride = (uint64_t)gridDim.x * blockDim.x * U;
   for (uint64_t w0 = (uint64_t)blockIdx.x * blockDim.x * U + threadIdx.x; w0 < total; w0 += stride) {
@@ -489,16 +492,8 @@ k_exchange_p2p(qs_c128* __restrict__ shard, const __grid_constant__ ExchGeom G) 
       const uint64_t w = w0 + (uint64_t)u * blockDim.x;
       mine[u] = nullptr;
       if (w >= total) continue;
-      int d;
-      uint64_t q;
-      if (G.chunk_log2 > 0) {
-        const uint64_t chunk = w >> G.chunk_log2, nd = (1ull << k) - 1ull;
-        d = 1 + (int)(chunk % nd);
-        q = ((chunk / nd) << G.chunk_log2) | (w & ((1ull << G.chunk_log2) - 1ull));
-      } else {
-        d = 1 + (int)(w / half);
-        q = w % half;
-      }
+      const int d = 1 + (int)(w >> half_log2);
+      const uint64_t q = w & (half - 1ull);
       // r: index inside the block; bit kExchSplitBit says which of the two ranks moves it
       const uint64_t low = q & ((1ull << kExchSplitBit) - 1ull);
       const uint64_t r = ((q >> kExchSplitBit) << (kExchSplitBit + 1)) | ((uint64_t)G.higher[d] << kExchSplitBit) | low;
@@ -1379,28 +1374,8 @@ int qsim_has_cuda(void) { return 1; }
 
 int64_t qsim_launch_count(void) { return g_launches.load(std::memory_order_relaxed); }
 
-int qsim_peer_alloc(int device, uint64_t bytes, void** out_ptr) {
-  if (!out_ptr || bytes == 0) return qs::fail(QSIM_ERR_ARG, "qsim_peer_alloc: bad argument");
-  QS_CUDA(cudaSetDevice(device));
-  QS_CUDA(cudaMalloc(out_ptr, bytes));
-  return QSIM_OK;
-}
-
-int qsim_peer_free(void* ptr) {
-  if (ptr) QS_CUDA(cudaFree(ptr));
-  return QSIM_OK;
-}
-
-int qsim_ipc_export(void* ptr, unsigned char* handle64) {
-  static_assert(sizeof(cudaIpcMemHandle_t) == 64, "IPC handle size");
-  if (!ptr || !handle64) return qs::fail(QSIM_ERR_ARG, "qsim_ipc_export: null argument");
-  cudaIpcMemHandle_t h;
-  QS_CUDA(cudaIpcGetMemHandle(&h, ptr));
-  memcpy(handle64, &h, 64);
-  return QSIM_OK;
-}
-
 int qsim_ipc_import(int device, const unsigned char* handle64, void** out_ptr) {
+  static_assert(sizeof(cudaIpcMemHandle_t) == 64, "IPC handle size");
   if (!handle64 || !out_ptr) return qs::fail(QSIM_ERR_ARG, "qsim_ipc_import: null argument");
   cudaIpcMemHandle_t h;
   memcpy(&h, handle64, 64);
@@ -1473,28 +1448,12 @@ int qsim_exchange_p2p(void* shard, void* const* peer_shards, int n_local, int nb
   int rc = bind_device(shard, &bound);
   if (rc != QSIM_OK) return rc;
   const uint64_t total = (1ull << (n_local - nbits - 1)) * ((1ull << nbits) - 1ull);
-  // development knobs (defaults measured on 2 and 8 B200s): pairs per thread and trip, CTAs per SM
-  static const int batch = qs::dev_knob("QSIM_EXCH_BATCH", 4);
-  static const int per_sm = qs::dev_knob("QSIM_EXCH_CTAS", 8);
-  static const int chunk_log2 = qs::dev_knob("QSIM_EXCH_CHUNK_LOG2", 0);
-  G.chunk_log2 = (chunk_log2 > 0 && chunk_log2 <= n_local - nbits - 1 && nbits > 1) ? chunk_log2 : 0;
-  const int U = batch >= 8 ? 8 : batch >= 4 ? 4 : batch >= 2 ? 2 : 1;
-  uint64_t blocks = (total + 256ull * U - 1) / (256ull * U);
-  const uint64_t cap = (uint64_t)bound.ctx->sms * (uint64_t)(per_sm > 0 ? per_sm : 8);
+  uint64_t blocks = (total + 256ull * kExchPairs - 1) / (256ull * kExchPairs);
+  const uint64_t cap = (uint64_t)bound.ctx->sms * kExchCtasPerSm;
   if (blocks > cap) blocks = cap;
   if (blocks < 1) blocks = 1;
-  cudaStream_t st = (cudaStream_t)stream;
-  if (U == 8) k_exchange_p2p<8><<<(unsigned)blocks, 256, 0, st>>>((qs_c128*)shard, G);
-  else if (U == 4) k_exchange_p2p<4><<<(unsigned)blocks, 256, 0, st>>>((qs_c128*)shard, G);
-  else if (U == 2) k_exchange_p2p<2><<<(unsigned)blocks, 256, 0, st>>>((qs_c128*)shard, G);
-  else k_exchange_p2p<1><<<(unsigned)blocks, 256, 0, st>>>((qs_c128*)shard, G);
+  k_exchange_p2p<<<(unsigned)blocks, 256, 0, (cudaStream_t)stream>>>((qs_c128*)shard, G);
   return launched();
-}
-
-int qsim_peer_copy(void* dst, const void* src, uint64_t bytes, void* stream) {
-  if (!dst || !src) return qs::fail(QSIM_ERR_ARG, "qsim_peer_copy: null argument");
-  QS_CUDA(cudaMemcpyAsync(dst, src, bytes, cudaMemcpyDefault, (cudaStream_t)stream));
-  return QSIM_OK;
 }
 
 }  // extern "C"

@@ -58,10 +58,6 @@ class CudaBackend:
         _capi.declare(self.lib)
         if self.lib.qsim_has_cuda() != 1:
             raise RuntimeError("libqsim_b200.so was built without CUDA kernels")
-        self._side_streams = []
-
-    def pipeline(self, nstages: int) -> "_StreamPipeline":
-        return _StreamPipeline(self, nstages)
 
     # -- memory ------------------------------------------------------------------
     def empty(self, count: int):
@@ -136,42 +132,6 @@ class _PendingCopy:
         if self._event is not None:
             self._event.synchronize()
             self._event = self._buf = self._dst = None
-
-
-class _StreamPipeline:
-    """A few side streams with event dependencies between them (used by the sharded
-    swap to overlap gather, exchange and scatter)."""
-
-    def __init__(self, backend: "CudaBackend", nstages: int):
-        torch = backend.torch
-        self.torch = torch
-        self.device = backend.device
-        if len(backend._side_streams) < nstages:
-            backend._side_streams += [torch.cuda.Stream(self.device)
-                                      for _ in range(nstages - len(backend._side_streams))]
-        self.streams = backend._side_streams[:nstages]
-        self.main = torch.cuda.current_stream(self.device)
-        start = torch.cuda.Event()
-        start.record(self.main)
-        for st in self.streams:
-            st.wait_event(start)
-
-    def stage(self, i: int):
-        return self.torch.cuda.stream(self.streams[i])
-
-    def record(self):
-        ev = self.torch.cuda.Event()
-        ev.record(self.torch.cuda.current_stream(self.device))
-        return ev
-
-    def wait(self, ev) -> None:
-        self.torch.cuda.current_stream(self.device).wait_event(ev)
-
-    def join(self) -> None:
-        for st in self.streams:
-            ev = self.torch.cuda.Event()
-            ev.record(st)
-            self.main.wait_event(ev)
 
 
 _backend_lock = threading.Lock()

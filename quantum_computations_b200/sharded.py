@@ -24,10 +24,11 @@ is fixed and everything runs on the shard through the single-GPU fused planner:
   local qubits in ONE all-to-all exchange: with ``k`` qubits moving, every rank keeps
   ``1/2^k`` of its shard and sends ``1/2^k`` to each of the ``2^k - 1`` ranks that
   differ in those rank bits (0.875 of a shard for k = 3, where three single swaps
-  would move 1.5).  ``qsim_swap_pack`` / ``qsim_swap_unpack`` gather and scatter the
-  travelling blocks; the transfer is a copy-engine push over NVLink (CUDA IPC) on
-  GPUs and a send/recv elsewhere.  The first stage costs nothing: the initial product
-  state is built directly in the layout the schedule wants.
+  would move 1.5).  On GPUs the exchange is one kernel per rank over the peers' shards
+  mapped through CUDA IPC (``qsim_exchange_p2p``); elsewhere, and on GPUs for blocks
+  under 64 amplitudes, ``qsim_swap_pack`` / ``qsim_swap_unpack`` gather and scatter
+  the travelling blocks around a send/recv.  The first stage costs nothing: the
+  initial product state is built directly in the layout the schedule wants.
 
 ``ShardedSimulator.run_circuit`` adds measurements, insertions and classical control
 (``Simulator.run`` semantics); ``density=True`` shards a vectorised density matrix.
@@ -35,7 +36,6 @@ is fixed and everything runs on the shard through the single-GPU fused planner:
 from __future__ import annotations
 
 import ctypes as C
-import os
 
 import numpy as np
 
@@ -103,7 +103,7 @@ class ShardedState:
         self.swaps = 0
         self.swap_seconds = 0.0
         self.amps_sent = 0
-        self._peer = None
+        self._staging = None                      # (chunk, send, recv) of the send/recv exchange
         self._p2p = None                          # peers' shards mapped through CUDA IPC (fused exchange)
         self._swap_events = []                    # CUDA event pairs of the fused exchanges (timed lazily)
         self.is_density = False                   # set by ShardedSimulator(density=True): vec(rho), 2N bits
@@ -503,63 +503,17 @@ class ShardedState:
         return out
 
     # -- swaps -----------------------------------------------------------------------------------
-    import os as _os
-    # amplitudes per pipeline chunk: 512 MiB measured best (614 GB/s per direction on two B200s;
-    # 580 at 256 MiB, 557 at 1 GiB, 539 at 2 GiB)
-    CHUNK_LOG2 = int(_os.environ.get("QSIM_SWAP_CHUNK_LOG2", "25"))
+    CHUNK_LOG2 = 25                 # blocks travel in chunks of at most 2^25 amplitudes: bounds the staging buffers
 
-    def _peer_setup(self, chunk: int):
-        """Allocate the four staging chunks with the library (plain cudaMalloc, so they can be
-        exported through CUDA IPC) and open every other rank's receive chunks once."""
-        be, lib = self.backend, self.backend.lib
-        if self._peer is not None and self._peer["chunk"] == chunk:
-            return self._peer
-        if self._peer is not None:                # another chunk size: give the old staging back first
-            p2p = self._p2p
-            self._p2p = None
-            self.close()
-            self._p2p = p2p
-        use_ipc = getattr(be, "name", "") == "cuda" and os.environ.get("QSIM_SWAP_IPC", "1") != "0"
-        peer = {"chunk": chunk, "ipc": use_ipc}
-        if not use_ipc:
-            peer["send"] = [be.empty(chunk) for _ in range(2)]
-            peer["recv"] = [be.empty(chunk) for _ in range(2)]
-            self._peer = peer
-            return peer
-        import torch
-        dev = be.device.index
-        ptrs = []
-        for _ in range(4):
-            out = C.c_void_p()
-            _capi.check(lib, lib.qsim_peer_alloc(dev, C.c_uint64(16 * chunk), C.byref(out)))
-            ptrs.append(out.value)
-        peer["send_ptr"], peer["recv_ptr"] = ptrs[:2], ptrs[2:]
-        handles = []
-        for p in peer["recv_ptr"]:
-            h = C.create_string_buffer(64)
-            _capi.check(lib, lib.qsim_ipc_export(C.c_void_p(p), h))
-            handles.append(h.raw)
-        gathered = [None] * self.comm.size
-        self.comm.dist.all_gather_object(gathered, handles, group=self.comm.group)
-        peer["remote_recv"] = {}
-        for r, hs in enumerate(gathered):
-            if r == self.comm.rank:
-                continue
-            opened = []
-            for h in hs:
-                out = C.c_void_p()
-                _capi.check(lib, lib.qsim_ipc_import(dev, h, C.byref(out)))
-                opened.append(out.value)
-            peer["remote_recv"][r] = opened
-        peer["token_out"] = torch.zeros(2, dtype=torch.float64, device=be.device)
-        peer["token_in"] = torch.zeros(2, dtype=torch.float64, device=be.device)
-        self._peer = peer
-        return peer
+    def _staging_setup(self, chunk: int):
+        """One send and one receive buffer of ``chunk`` amplitudes, kept for the next exchange."""
+        if self._staging is None or self._staging[0] != chunk:
+            self._staging = (chunk, self.backend.empty(chunk), self.backend.empty(chunk))
+        return self._staging[1:]
 
     # -- fused exchange over NVLink peer memory (GPUs) ---------------------------------------------
     def _use_fused(self, block: int) -> bool:
-        return (getattr(self.backend, "name", "") == "cuda" and os.environ.get("QSIM_SWAP_FUSED", "1") != "0"
-                and os.environ.get("QSIM_SWAP_IPC", "1") != "0" and block >= 64)
+        return getattr(self.backend, "name", "") == "cuda" and block >= 64
 
     def _p2p_setup(self):
         """Map every other rank's shard into this process (CUDA IPC), once per shard buffer."""
@@ -644,25 +598,13 @@ class ShardedState:
     def close(self) -> None:
         """Release the peer mappings and the staging buffers of the exchanges."""
         self._p2p_release()
-        peer, self._peer = self._peer, None
-        if peer is not None and peer.get("ipc"):
-            lib = self.backend.lib
-            self.backend.synchronize()
-            for opened in peer.get("remote_recv", {}).values():
-                for ptr in opened:
-                    lib.qsim_ipc_release(C.c_void_p(ptr))
-            for ptr in peer.get("send_ptr", []) + peer.get("recv_ptr", []):
-                lib.qsim_peer_free(C.c_void_p(ptr))
+        self._staging = None
 
     def __del__(self):
         try:
             self.close()
         except Exception:
             pass
-
-    def swap(self, global_phys: int, local_phys: int) -> None:
-        """Exchange one rank bit with one local bit (half a shard travels)."""
-        self.exchange([(global_phys, local_phys)])
 
     def exchange(self, pairs) -> None:
         """Exchange the physical rank bits with the physical local bits of ``pairs``
@@ -671,13 +613,12 @@ class ShardedState:
         With k pairs the 2^k ranks that differ in those rank bits form a group; in round
         d = 1 .. 2^k-1 every rank trades one block of 2^(n_local-k) amplitudes with the
         partner whose rank bits differ by the pattern d: it sends the block whose k local
-        bits spell the partner's rank bits and receives into the same positions.  Blocks
-        are cut into chunks that flow through a three-stage pipeline on three streams:
-        gather (``qsim_swap_pack``) into a staging chunk, transfer, scatter
-        (``qsim_swap_unpack``).  On GPUs the transfer is a copy-engine PUSH into the
-        partner's staging chunk over NVLink (CUDA IPC + ``qsim_peer_copy``), fenced on both
-        sides by tiny stream-ordered NCCL token exchanges with that partner, so no SM is
-        spent on communication; elsewhere (gloo tests) it is a send/recv.  Flip flags are
+        bits spell the partner's rank bits and receives into the same positions.  On GPUs
+        this is one kernel per rank over the peers' shards (``_exchange_fused``).  Elsewhere,
+        and on GPUs for blocks under 64 amplitudes, blocks are cut into chunks of at most
+        2^CHUNK_LOG2 amplitudes and each chunk is gathered into a send buffer
+        (``qsim_swap_pack``), traded by a send/recv with the partner and scattered from the
+        receive buffer (``qsim_swap_unpack``), all on the current stream.  Flip flags are
         the caller's business: the bits move as stored."""
         import time
         be, lib = self.backend, self.backend.lib
@@ -691,6 +632,9 @@ class ShardedState:
         qubits = (C.c_int * k)(*[self.n_local - 1 - lp for _gp, lp in pairs])   # local reference-style numbers
         mine = [(self.comm.rank >> gi) & 1 for gi in gis]
         block = 1 << (self.n_local - k)
+        if self._use_fused(block):
+            self._exchange_fused(pairs, gis, qubits, mine, block)
+            return
         chunk = min(block, 1 << self.CHUNK_LOG2)
         per_block = block // chunk
         items = []                                   # (partner, bit values of the travelling block, first)
@@ -703,65 +647,15 @@ class ShardedState:
                 vals.append(mine[i] ^ di)
             for c in range(per_block):
                 items.append((partner, (C.c_int * k)(*vals), c * chunk))
-        if self._use_fused(block):
-            self._exchange_fused(pairs, gis, qubits, mine, block)
-            return
-        peer = self._peer_setup(chunk)
-        ipc = peer["ipc"]
+        send, recv = self._staging_setup(chunk)
         be.synchronize()                           # so the timer below sees the exchange alone
         t0 = time.perf_counter()
-        if ipc:
-            send_ptr, recv_ptr = peer["send_ptr"], peer["recv_ptr"]
-        else:
-            send_ptr = [be.ptr(b) for b in peer["send"]]
-            recv_ptr = [be.ptr(b) for b in peer["recv"]]
-        pipe = be.pipeline(3)                      # stream contexts + events (no-ops on the host emulator)
-        packed, moved, unpacked = {}, {}, {}
-
-        def token(partner):                        # both ranks have reached this point of their comm streams
-            self.comm.exchange(peer["token_out"], peer["token_in"], partner)
-
-        def pack(c):
-            _partner, vals, first = items[c]
-            with pipe.stage(0):
-                if c >= 2:
-                    pipe.wait(moved[c - 2])        # send[c%2] has left (our own push / send of item c-2)
-                _capi.check(lib, lib.qsim_swap_pack(be.ptr(self.buf), C.c_void_p(send_ptr[c % 2]), self.n_local,
-                                                    k, qubits, vals, C.c_uint64(first), C.c_uint64(chunk),
-                                                    be.stream()))
-                packed[c] = pipe.record()
-
-        def unpack(c):
-            _partner, vals, first = items[c]
-            with pipe.stage(2):
-                pipe.wait(moved[c])
-                _capi.check(lib, lib.qsim_swap_unpack(be.ptr(self.buf), C.c_void_p(recv_ptr[c % 2]), self.n_local,
-                                                      k, qubits, vals, C.c_uint64(first), C.c_uint64(chunk),
-                                                      be.stream()))
-                unpacked[c] = pipe.record()
-
-        for c, (partner, _vals, _first) in enumerate(items):
-            pack(c)
-            with pipe.stage(1):
-                pipe.wait(packed[c])
-                if c >= 2:
-                    pipe.wait(unpacked[c - 2])     # our recv[c%2] is free again
-                if ipc:
-                    # first token: both items c are packed and both recv[c%2] are free -> PUSH ours
-                    # into the partner's staging with the copy engine (writes are the fast
-                    # direction of NVLink P2P); second token: both pushes have landed
-                    token(partner)
-                    _capi.check(lib, lib.qsim_peer_copy(C.c_void_p(peer["remote_recv"][partner][c % 2]),
-                                                        C.c_void_p(send_ptr[c % 2]),
-                                                        C.c_uint64(16 * chunk), be.stream()))
-                    token(partner)
-                    self.comm.bytes_exchanged += 16 * chunk
-                else:
-                    self.comm.exchange(self._as_torch(peer["send"][c % 2]), self._as_torch(peer["recv"][c % 2]),
-                                       partner)
-                moved[c] = pipe.record()
-            unpack(c)
-        pipe.join()
+        for partner, vals, first in items:
+            _capi.check(lib, lib.qsim_swap_pack(be.ptr(self.buf), C.c_void_p(be.ptr(send)), self.n_local, k, qubits,
+                                                vals, C.c_uint64(first), C.c_uint64(chunk), be.stream()))
+            self.comm.exchange(self._as_torch(send), self._as_torch(recv), partner)
+            _capi.check(lib, lib.qsim_swap_unpack(be.ptr(self.buf), C.c_void_p(be.ptr(recv)), self.n_local, k,
+                                                  qubits, vals, C.c_uint64(first), C.c_uint64(chunk), be.stream()))
         be.synchronize()
         self.swap_seconds += time.perf_counter() - t0
         self.swaps += 1

@@ -63,32 +63,6 @@ class EmuBackend:
     def pinned_empty(self, count):
         return np.empty(int(count), dtype=np.complex128)
 
-    def pipeline(self, nstages):
-        return _SerialPipeline()
-
-
-class _SerialPipeline:
-    """Host execution is already in program order: stages and events are no-ops."""
-
-    class _Ctx:
-        def __enter__(self):
-            return self
-
-        def __exit__(self, *exc):
-            return False
-
-    def stage(self, i):
-        return self._Ctx()
-
-    def record(self):
-        return None
-
-    def wait(self, ev):
-        pass
-
-    def join(self):
-        pass
-
 
 _EMU = None
 

@@ -395,7 +395,7 @@ def check_edge_cases(backend):
 
 def check_swap_pack_unpack(backend):
     """qsim_swap_pack / _unpack (the gather / scatter of a k-qubit exchange block) against
-    NumPy indexing, chunked like the pipeline does."""
+    NumPy indexing, chunked like the send/recv exchange does."""
     import ctypes as C
     from quantum_computations_b200 import _capi
     rng = np.random.default_rng(17)

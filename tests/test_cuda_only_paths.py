@@ -7,12 +7,11 @@
   dense-block kernel, whose tile needs more than 48 KiB of shared memory from k = 9 on;
 - the tile pass with its tile loaded through TMA boxes against the same pass with plain loads.
 
-The launch variants (pairs per thread, CTAs per SM and round-robin chunks of the exchange; plain
-loads and the dense variants of the tile pass) are A/B switches that only the development build
-of the library reads from the environment, once per process.  Each setting therefore runs in a
-child process -- this file run as a script with the development build -- which prints one JSON
-line; the parent asserts on it.  The child also lists the kernels it launched, so that a setting
-which did not take effect fails instead of repeating the default."""
+The launch variants of the tile pass (plain loads and the dense variants) are A/B switches that
+only the development build of the library reads from the environment, once per process.  Each
+setting therefore runs in a child process -- this file run as a script with the development
+build -- which prints one JSON line; the parent asserts on it.  The child also lists the kernels
+it launched, so that a setting which did not take effect fails instead of repeating the default."""
 import ctypes as C
 import json
 import os
@@ -370,15 +369,15 @@ def run_tile_cases(backend):
     return outs
 
 
-KNOBS = ("QSIM_EXCH_BATCH", "QSIM_EXCH_CTAS", "QSIM_EXCH_CHUNK_LOG2", "QSIM_NO_TMA", "QSIM_FORCE_DENSE_VARIANT")
+KNOBS = ("QSIM_NO_TMA", "QSIM_FORCE_DENSE_VARIANT")
 
 
-def run_child(what, env_knobs, outdir):
+def run_child(env_knobs, outdir):
     """This file as a script with the development build and one setting of the switches."""
     build_native.build_cuda(dev_knobs=True)        # no-op when tests/_build is up to date
     env = {k: v for k, v in os.environ.items() if k not in KNOBS}
     env.update(env_knobs, QSIM_LIB=build_native.CUDA_KNOBS_LIB)
-    cmd = [sys.executable] + (["-s"] if sys.flags.no_user_site else []) + [__file__, what, str(outdir)]
+    cmd = [sys.executable] + (["-s"] if sys.flags.no_user_site else []) + [__file__, str(outdir)]
     out = subprocess.run(cmd, env=env, capture_output=True, text=True, timeout=300, cwd=ROOT)
     assert out.returncode == 0, out.stderr[-3000:]
     lines = [l for l in out.stdout.splitlines() if l.strip()]
@@ -404,43 +403,16 @@ def _kernels(fn):
     return result, seen
 
 
-def _child_main(what, outdir):
+def _child_main(outdir):
     import torch
     be = engine.get_backend()
     assert os.path.samefile(engine._LIB_PATH, build_native.CUDA_KNOBS_LIB)
     torch.cuda.reset_peak_memory_stats()
-    report = {"sms": torch.cuda.get_device_properties(0).multi_processor_count}
-    if what == "exchange":
-        report["failures"], kernels = _kernels(lambda: run_exchange_cases(be.lib))
-        report["batch"] = sorted({int(m) for name in kernels for m in re.findall(r"k_exchange_p2p<(\d+)>", name)})
-        report["grid"] = max(g for name, g in kernels.items() if "k_exchange_p2p" in name)
-    else:
-        outs, kernels = _kernels(lambda: run_tile_cases(be))
-        np.savez(os.path.join(outdir, "tiles.npz"), *[o[2] for o in outs])
-        modes = re.findall(r"k_tile_pass<\s*\d+\s*,\s*(\d+)\s*,\s*\d+\s*>", " ".join(kernels))
-        report["dense_modes"] = sorted({int(m) for m in modes})
-    report["peak_bytes"] = int(torch.cuda.max_memory_allocated())
+    outs, kernels = _kernels(lambda: run_tile_cases(be))
+    np.savez(os.path.join(outdir, "tiles.npz"), *[o[2] for o in outs])
+    modes = re.findall(r"k_tile_pass<\s*\d+\s*,\s*(\d+)\s*,\s*\d+\s*>", " ".join(kernels))
+    report = {"dense_modes": sorted({int(m) for m in modes}), "peak_bytes": int(torch.cuda.max_memory_allocated())}
     print(json.dumps(report))
-
-
-EXCHANGE_SETTINGS = [{"QSIM_EXCH_BATCH": "1"}, {"QSIM_EXCH_BATCH": "2"}, {"QSIM_EXCH_BATCH": "8"},
-                     {"QSIM_EXCH_CHUNK_LOG2": "1"}, {"QSIM_EXCH_CHUNK_LOG2": "5"},
-                     {"QSIM_EXCH_CHUNK_LOG2": "13"},        # n_local - k - 1 of the (k = 2, n_local = 16) case
-                     {"QSIM_EXCH_CTAS": "1"}]
-
-
-@pytest.mark.gpu
-@pytest.mark.parametrize("setting", EXCHANGE_SETTINGS, ids=lambda s: ",".join(f"{k}={v}" for k, v in s.items()))
-def test_exchange_variants(cuda_backend, tmp_path, setting):
-    """Pairs per thread U = 1, 2, 8 (4 is the default, run above), round-robin chunks of 2 and 32
-    pairs and of a whole block (k = 1 ignores the switch), and one CTA per SM: a 148-block grid
-    that takes every case through many trips, the last one ragged."""
-    rep = run_child("exchange", setting, tmp_path)
-    assert rep["failures"] == []
-    assert rep["peak_bytes"] < 1 << 30
-    assert rep["batch"] == [int(setting.get("QSIM_EXCH_BATCH", 4))]
-    if "QSIM_EXCH_CTAS" in setting:
-        assert rep["grid"] == rep["sms"]
 
 
 @pytest.fixture(scope="module")
@@ -455,7 +427,7 @@ def tile_outputs(cuda_backend):
 @pytest.mark.gpu
 def test_plain_tile_loads_match_tma_bit_for_bit(tile_outputs, tmp_path):
     """Both paths fill the same swizzled tile slots and run the same steps on them."""
-    rep = run_child("tiles", {"QSIM_NO_TMA": "1"}, tmp_path)
+    rep = run_child({"QSIM_NO_TMA": "1"}, tmp_path)
     assert rep["peak_bytes"] < 1 << 30
     plain = np.load(tmp_path / "tiles.npz")
     tma, refs = tile_outputs
@@ -467,7 +439,7 @@ def test_plain_tile_loads_match_tma_bit_for_bit(tile_outputs, tmp_path):
 @pytest.mark.gpu
 @pytest.mark.parametrize("variant", [1, 2])
 def test_forced_dense_variants_match_oracle(tile_outputs, tmp_path, variant):
-    rep = run_child("tiles", {"QSIM_FORCE_DENSE_VARIANT": str(variant)}, tmp_path)
+    rep = run_child({"QSIM_FORCE_DENSE_VARIANT": str(variant)}, tmp_path)
     # variant 1 raises passes without dense steps to mode 1; passes of mostly dense steps keep mode 2
     assert rep["dense_modes"][0] == variant and set(rep["dense_modes"]) <= {1, 2}
     got = np.load(tmp_path / "tiles.npz")
@@ -477,4 +449,4 @@ def test_forced_dense_variants_match_oracle(tile_outputs, tmp_path, variant):
 
 
 if __name__ == "__main__":
-    _child_main(sys.argv[1], sys.argv[2])
+    _child_main(sys.argv[1])

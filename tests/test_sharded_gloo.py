@@ -81,7 +81,7 @@ def _worker(rank, world, port, n, depth, seed, out_dir):
         circ += [gates.Y(q) for q in range(n)] + [gates.CZ(0, n - 1), gates.T(1)]
         vecs = [State.PLUS.get(), State.T.get()] + [State.ZERO.get()] * (n - 2)
         st = sharded.ShardedState(n, comm, backend=be, as_torch=torch.from_numpy)
-        sharded.ShardedState.CHUNK_LOG2 = 4                 # several pipeline chunks per block even at this size
+        sharded.ShardedState.CHUNK_LOG2 = 4                 # several chunks per block even at this size
         sim = sharded.ShardedSimulator(circ, st, plan_options=dict(tile_bits=6, low_bits=2))
         sim.prepare(vecs)
         sim.run()

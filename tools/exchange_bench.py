@@ -3,9 +3,7 @@
 
     torchrun --nproc-per-node 2 tools/exchange_bench.py [--shard-qubits 30] [--reps 6]
 
-Prints, on rank 0, ms per exchange and GB/s per direction and GPU for k = 1 .. log2(ranks).
-Knobs of the fused kernel: QSIM_EXCH_BATCH, QSIM_EXCH_CTAS; QSIM_SWAP_FUSED=0 selects the
-copy-engine pipeline (pack / peer copy / unpack)."""
+Prints, on rank 0, ms per exchange and GB/s per direction and GPU for k = 1 .. log2(ranks)."""
 import argparse
 import json
 import os
@@ -53,9 +51,7 @@ def main():
                     "shard_fraction": sent / (16.0 * 2.0 ** st.n_local)})
     norm = st.norm()
     if rank == 0:
-        print(json.dumps({"ranks": world, "n_local": st.n_local, "fused": os.environ.get("QSIM_SWAP_FUSED", "1"),
-                          "batch": os.environ.get("QSIM_EXCH_BATCH", "default"),
-                          "ctas": os.environ.get("QSIM_EXCH_CTAS", "default"), "exchanges": out, "norm": norm}))
+        print(json.dumps({"ranks": world, "n_local": st.n_local, "exchanges": out, "norm": norm}))
     st.close()
     dist.destroy_process_group()
 

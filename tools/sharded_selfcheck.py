@@ -1,9 +1,9 @@
 #!/usr/bin/env python
-"""Full-size parity property for the sharded path (torchrun, one rank per GPU, NCCL + CUDA-IPC
-exchanges): a random circuit followed by its gate-by-gate inverse must bring |0...0> back.
-No oracle can hold 2^34 amplitudes; this checks the whole chain -- stage scheduler, rank
-relabelling, leftovers across exchanges, pack / push / unpack pipeline, tile passes -- on the
-real interconnect.  Prints one JSON line on rank 0.
+"""Full-size parity property for the sharded path (torchrun, one rank per GPU, exchanges over
+CUDA-IPC mapped peer shards): a random circuit followed by its gate-by-gate inverse must bring
+|0...0> back.  No oracle can hold 2^34 amplitudes; this checks the whole chain -- stage
+scheduler, rank relabelling, leftovers across exchanges, the exchange kernel, tile passes -- on
+the real interconnect.  Prints one JSON line on rank 0.
 
     python -m torch.distributed.run --nproc-per-node 8 --master-addr 127.0.0.1 tools/sharded_selfcheck.py --qubits 34 --depth 60
 """
@@ -91,7 +91,7 @@ def main():
                 psi0 = np.kron(psi0, np.asarray(k, dtype=np.complex128))
             ref = Simulator(forward, backend=backend).run(psi0)
             err = float(np.abs(got - ref).max() / np.abs(ref).max())
-            print(json.dumps({"check": "sharded (NCCL + CUDA-IPC) vs single-GPU, element by element", "qubits": n,
+            print(json.dumps({"check": "sharded vs single-GPU, element by element", "qubits": n,
                               "gpus": world, "depth": args.depth, "gates": len(forward), "max_rel_err": err,
                               "plan": sim.stats, "exchanges": state.swaps, "ok": bool(err < 1e-12)}))
         dist.destroy_process_group()

@@ -202,6 +202,25 @@ int qsim_pauli_rotations_adjoint(void* psi, void* lam, int n_qubits, int64_t n_r
 int qsim_pauli_rotations_adjoint_dm(void* psi, void* lam, int n_qubits, int64_t n_rot, const uint64_t* x_masks,
                                     const uint64_t* z_masks, const double* angles, double* out, void* stream);
 
+/* ---- Lanczos building blocks: fused H|psi> and dot, and the fused step --------------------
+ * out <- prev_scale * prev + sum_t c_t P_t in (strings, coefficients and passes as in
+ * qsim_apply_pauli_sum; the first pass reads prev where an accumulating pass reads out).  prev may
+ * be out (out <- prev_scale * out + ...) or null (zeros).  The last pass also reduces Re <in|out>
+ * with fixed summation trees; *out_dot receives it, so two calls on the same inputs give
+ * bit-identical outputs and dots.  n_terms == 0 gives out = prev_scale * prev and its dot.  in ==
+ * out, in == prev, a null in, out or out_dot, a non-finite prev_scale and the checks of
+ * qsim_apply_pauli_sum are QSIM_ERR_ARG.  Synchronises the stream. */
+int qsim_lanczos_apply(const void* in, const void* prev, void* out, int n_qubits, int64_t n_terms,
+                       const uint64_t* x_masks, const uint64_t* z_masks, const double* coeffs_re_im, double prev_scale,
+                       double* out_dot, void* stream);
+/* One streaming pass over n_amps amplitudes: w <- w - a v and, when y is not null, y <- y + b v with
+ * b = (b_re_im[0], b_re_im[1]) (a HOST array).  A null w updates y alone.  With out_norm2 (a HOST
+ * double) the call reduces |w|^2 after the update (|y|^2 when w is null) with fixed summation trees
+ * and synchronises; without it, it does not synchronise.  A null v, w and y both null, a null b_re_im
+ * with y, aliased buffers, n_amps == 0 and non-finite a or b are QSIM_ERR_ARG. */
+int qsim_lanczos_step(void* w, const void* v, void* y, uint64_t n_amps, double a, const double* b_re_im,
+                      double* out_norm2, void* stream);
+
 /* ---- measurement statistics: marginal probabilities and shot sampling -------------------
  * Qubits are the reference's (qubit q is index bit n-1-q).  A marginal over qubits[0..k) has
  * 2^k bins; bit k-1-j of the bin number is the value of qubits[j], so qubits[0] is the most

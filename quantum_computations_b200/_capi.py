@@ -90,6 +90,10 @@ SIGNATURES = {
                                                C.c_void_p, C.c_void_p, C.c_void_p]),
     "qsim_pauli_rotations_adjoint_dm": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int64, C.c_void_p,
                                                   C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "qsim_lanczos_apply": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int64, C.c_void_p,
+                                     C.c_void_p, C.c_void_p, C.c_double, c_double_p, C.c_void_p]),
+    "qsim_lanczos_step": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_uint64, C.c_double, c_double_p,
+                                    c_double_p, C.c_void_p]),
     "qsim_marginal_probs": (C.c_int, [C.c_void_p, C.c_int, C.c_int, c_int_p, C.c_void_p, C.c_void_p]),
     "qsim_marginal_probs_dm": (C.c_int, [C.c_void_p, C.c_int, C.c_int, c_int_p, C.c_void_p, C.c_void_p]),
     "qsim_sample_workspace_bytes": (C.c_int, [C.c_int, C.c_int64, C.POINTER(C.c_uint64)]),

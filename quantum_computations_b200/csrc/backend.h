@@ -36,6 +36,14 @@ int apply_pauli_rotations(qs_c128* state, int n, const PauliRotPlan& plan, void*
 // out <- sum_t c_t P_t in (or out + ..., as the plan's passes say), n index bits, one launch per pass;
 // no allocation, no synchronisation
 int apply_pauli_sum(const qs_c128* in, qs_c128* out, int n, const PauliApplyPlan& plan, void* stream);
+// the passes of a Lanczos apply plan (plan_pauli_apply's, the first starting from prev_scale x prev and
+// the last reducing Re <in|out>) plus the final sum; *out_dot = Re <in|out>; synchronises
+int lanczos_apply(const qs_c128* in, const qs_c128* prev, qs_c128* out, int n, const PauliApplyPlan& plan,
+                  double* out_dot, void* stream);
+// w <- w - a v (w may be null), y <- y + (bre + i bim) v (y may be null), one pass; with out_norm2 the
+// final sum of |w|^2 (|y|^2 when w is null) and a synchronisation
+int lanczos_step(qs_c128* w, const qs_c128* v, qs_c128* y, uint64_t n_amps, double a, double bre, double bim,
+                 double* out_norm2, void* stream);
 // the sweep of an adjoint plan on psi and lam (n index bits), one launch per pass plus the final sum;
 // sums: 2 doubles per rotation slot of `plan`; synchronises the stream
 int pauli_rotations_adjoint(qs_c128* psi, qs_c128* lam, int n, const PauliRotPlan& plan, double* sums, void* stream);

@@ -191,6 +191,37 @@ int pauli_sum(const char* who, const void* in, void* out, int n, int64_t n_terms
   return qs::dev::apply_pauli_sum((const qs_c128*)in, (qs_c128*)out, n, plan, stream);
 }
 
+int lanczos_apply(const void* in, const void* prev, void* out, int n, int64_t n_terms, const uint64_t* x_masks,
+                  const uint64_t* z_masks, const double* coeffs_re_im, double prev_scale, double* out_dot,
+                  void* stream) {
+  const std::string w("qsim_lanczos_apply");
+  int rc = qs::check_pauli_args(w.c_str(), n, n_terms, x_masks, z_masks, coeffs_re_im);
+  if (rc != QSIM_OK) return rc;
+  if (!in || !out) return qs::fail(QSIM_ERR_ARG, w + ": null state");
+  if (!out_dot) return qs::fail(QSIM_ERR_ARG, w + ": null argument");
+  if (in == out) return qs::fail(QSIM_ERR_ARG, w + ": in and out must be different buffers");
+  if (in == prev) return qs::fail(QSIM_ERR_ARG, w + ": in and prev must be different buffers");
+  if (n < 1 || n > 63) return qs::fail(QSIM_ERR_ARG, w + ": n_qubits must be in [1, 63]");
+  if (!std::isfinite(prev_scale)) return qs::fail(QSIM_ERR_ARG, w + ": non-finite prev_scale");
+  for (int64_t t = 0; t < 2 * n_terms; ++t)
+    if (!std::isfinite(coeffs_re_im[t])) return qs::fail(QSIM_ERR_ARG, w + ": non-finite coefficient");
+  qs::PauliApplyPlan plan;
+  try {
+    rc = qs::plan_pauli_apply(n, n_terms, x_masks, z_masks, coeffs_re_im, false, &plan);
+  } catch (const std::bad_alloc&) {
+    rc = qs::fail(QSIM_ERR_NOMEM, "out of host memory while grouping the Pauli terms");
+  }
+  if (rc != QSIM_OK) return rc;
+  // the first pass starts from p x prev (zeros without prev), the last one reduces the dot
+  QsPauliApplyPass& first = plan.passes.front();
+  if (prev) {
+    first.accumulate = prev == out ? QS_APPLY_FROM_OUT : QS_APPLY_FROM_PREV;
+    first.prev_scale = prev_scale;
+  }
+  plan.passes.back().dot = 1;
+  return qs::dev::lanczos_apply((const qs_c128*)in, (const qs_c128*)prev, (qs_c128*)out, n, plan, out_dot, stream);
+}
+
 int pauli_adjoint(const char* who, void* psi, void* lam, int n, int64_t n_rot, const uint64_t* x_masks,
                   const uint64_t* z_masks, const double* angles, double* out, bool dm, void* stream) {
   int rc = qs::check_pauli_args(who, n, n_rot, x_masks, z_masks, angles);
@@ -505,6 +536,26 @@ int qsim_accumulate_pauli_sum(const void* in, void* out, int n_qubits, int64_t n
                               const uint64_t* z_masks, const double* coeffs_re_im, void* stream) {
   return pauli_sum("qsim_accumulate_pauli_sum", in, out, n_qubits, n_terms, x_masks, z_masks, coeffs_re_im, true,
                    stream);
+}
+
+int qsim_lanczos_apply(const void* in, const void* prev, void* out, int n_qubits, int64_t n_terms,
+                       const uint64_t* x_masks, const uint64_t* z_masks, const double* coeffs_re_im, double prev_scale,
+                       double* out_dot, void* stream) {
+  return lanczos_apply(in, prev, out, n_qubits, n_terms, x_masks, z_masks, coeffs_re_im, prev_scale, out_dot, stream);
+}
+
+int qsim_lanczos_step(void* w, const void* v, void* y, uint64_t n_amps, double a, const double* b_re_im,
+                      double* out_norm2, void* stream) {
+  const std::string who("qsim_lanczos_step");
+  if (!v) return qs::fail(QSIM_ERR_ARG, who + ": null v");
+  if (!w && !y) return qs::fail(QSIM_ERR_ARG, who + ": w and y are both null");
+  if (y && !b_re_im) return qs::fail(QSIM_ERR_ARG, who + ": null b_re_im");
+  if (w == v || y == v || (w && w == y)) return qs::fail(QSIM_ERR_ARG, who + ": w, v and y must be different buffers");
+  if (n_amps == 0) return qs::fail(QSIM_ERR_ARG, who + ": n_amps must be positive");
+  if (!std::isfinite(a) || (y && (!std::isfinite(b_re_im[0]) || !std::isfinite(b_re_im[1]))))
+    return qs::fail(QSIM_ERR_ARG, who + ": non-finite coefficient");
+  return qs::dev::lanczos_step((qs_c128*)w, (const qs_c128*)v, (qs_c128*)y, n_amps, a, y ? b_re_im[0] : 0.0,
+                               y ? b_re_im[1] : 0.0, out_norm2, stream);
 }
 
 int qsim_pauli_rotations_adjoint(void* psi, void* lam, int n_qubits, int64_t n_rot, const uint64_t* x_masks,

@@ -360,9 +360,12 @@ QS_HD void qs_xor_swap(qs_c128* v, uint32_t x) {
 // permuted instead of the products: position u of acc holds output entry u ^ cur, and moving from
 // one group's xl to the next is one set of conditional swaps.  spec[k * stride], k < 2^(D+1), is the
 // thread's spectrum scratch (Re, then Im), where the terms scatter by their runtime index spec_t.
-template <int D>
-QS_HD void qs_pauli_apply_item(const QsPauliApplyPass& A, const qs_c128* __restrict__ in, qs_c128* __restrict__ out,
-                               uint64_t o, double* spec, uint32_t stride) {
+// LANCZOS (qsim_lanczos_apply) adds the first pass's start from prev_scale x prev (or x out) and
+// returns the item's share of Re sum conj(in) out when A.dot is set; without it the item is the
+// plain apply, which returns 0.
+template <int D, bool LANCZOS = false>
+QS_HD double qs_pauli_apply_item(const QsPauliApplyPass& A, const qs_c128* __restrict__ in, const qs_c128* prev,
+                                 qs_c128* __restrict__ out, uint64_t o, double* spec, uint32_t stride) {
   const QsPauliPass& P = A.p;
   uint64_t base = o;
 #pragma unroll
@@ -371,7 +374,11 @@ QS_HD void qs_pauli_apply_item(const QsPauliApplyPass& A, const qs_c128* __restr
 #pragma unroll
   for (int m = 0; m < (1 << D); ++m) {
     a[m] = in[base ^ P.off[m]];
-    if (A.accumulate) {
+    if (LANCZOS && A.accumulate >= QS_APPLY_FROM_PREV) {
+      const qs_c128 v = A.accumulate == QS_APPLY_FROM_OUT ? out[base ^ P.off[m]] : prev[base ^ P.off[m]];
+      acc[m].x = A.prev_scale * v.x;
+      acc[m].y = A.prev_scale * v.y;
+    } else if (A.accumulate) {
       acc[m] = out[base ^ P.off[m]];
     } else {
       acc[m].x = 0.0;
@@ -412,6 +419,35 @@ QS_HD void qs_pauli_apply_item(const QsPauliApplyPass& A, const qs_c128* __restr
   qs_xor_swap<D>(acc, cur);
 #pragma unroll
   for (int m = 0; m < (1 << D); ++m) out[base ^ P.off[m]] = acc[m];
+  double dot = 0.0;
+  if (LANCZOS && A.dot) {
+#pragma unroll
+    for (int m = 0; m < (1 << D); ++m) dot += a[m].x * acc[m].x + a[m].y * acc[m].y;
+  }
+  return dot;
+}
+
+// Element i of a Lanczos step (qsim_lanczos_step): w <- w - a v and, with y, y <- y + b v (b complex).
+// Returns |w_i|^2 after the update, or |y_i|^2 when there is no w (the update of y alone).
+QS_HD double qs_lanczos_step_elem(qs_c128* __restrict__ w, const qs_c128* __restrict__ v, qs_c128* __restrict__ y,
+                                  uint64_t i, double a, double bre, double bim) {
+  const qs_c128 vi = v[i];
+  double r = 0.0;
+  if (y) {
+    qs_c128 t = y[i];
+    t.x += bre * vi.x - bim * vi.y;
+    t.y += bre * vi.y + bim * vi.x;
+    y[i] = t;
+    r = t.x * t.x + t.y * t.y;
+  }
+  if (w) {
+    qs_c128 t = w[i];
+    t.x -= a * vi.x;
+    t.y -= a * vi.y;
+    w[i] = t;
+    r = t.x * t.x + t.y * t.y;
+  }
+  return r;
 }
 
 // One work item of an adjoint sweep pass (plan.h): the rotations of P (reverse caller order,

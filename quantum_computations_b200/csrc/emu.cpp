@@ -281,12 +281,46 @@ int apply_pauli_sum(const qs_c128* in, qs_c128* out, int n, const PauliApplyPlan
   for (const QsPauliApplyPass& A : plan.passes) {
     for (uint64_t o = 0; o < count; ++o) {
       switch (plan.d) {
-        case 1: qs_pauli_apply_item<1>(A, in, out, o, spec, 1); break;
-        case 2: qs_pauli_apply_item<2>(A, in, out, o, spec, 1); break;
-        case 3: qs_pauli_apply_item<3>(A, in, out, o, spec, 1); break;
-        default: qs_pauli_apply_item<4>(A, in, out, o, spec, 1); break;
+        case 1: qs_pauli_apply_item<1>(A, in, nullptr, out, o, spec, 1); break;
+        case 2: qs_pauli_apply_item<2>(A, in, nullptr, out, o, spec, 1); break;
+        case 3: qs_pauli_apply_item<3>(A, in, nullptr, out, o, spec, 1); break;
+        default: qs_pauli_apply_item<4>(A, in, nullptr, out, o, spec, 1); break;
       }
     }
+    ++g_launches;
+  }
+  return QSIM_OK;
+}
+
+// one launch per pass plus the final sum, as in the CUDA library
+int lanczos_apply(const qs_c128* in, const qs_c128* prev, qs_c128* out, int n, const PauliApplyPlan& plan,
+                  double* out_dot, void*) {
+  const uint64_t count = 1ull << (n - plan.d);
+  double spec[2 << QS_PAULI_MAX_D], dot = 0.0;
+  for (const QsPauliApplyPass& A : plan.passes) {
+    for (uint64_t o = 0; o < count; ++o) {
+      switch (plan.d) {
+        case 1: dot += qs_pauli_apply_item<1, true>(A, in, prev, out, o, spec, 1); break;
+        case 2: dot += qs_pauli_apply_item<2, true>(A, in, prev, out, o, spec, 1); break;
+        case 3: dot += qs_pauli_apply_item<3, true>(A, in, prev, out, o, spec, 1); break;
+        default: dot += qs_pauli_apply_item<4, true>(A, in, prev, out, o, spec, 1); break;
+      }
+    }
+    ++g_launches;
+  }
+  ++g_launches;                              // the final sum
+  *out_dot = dot;
+  return QSIM_OK;
+}
+
+// the step pass, and the final sum when the caller wants the norm, as in the CUDA library
+int lanczos_step(qs_c128* w, const qs_c128* v, qs_c128* y, uint64_t n_amps, double a, double bre, double bim,
+                 double* out_norm2, void*) {
+  double acc = 0.0;
+  for (uint64_t i = 0; i < n_amps; ++i) acc += qs_lanczos_step_elem(w, v, y, i, a, bre, bim);
+  ++g_launches;
+  if (out_norm2) {
+    *out_norm2 = acc;
     ++g_launches;
   }
   return QSIM_OK;

@@ -586,8 +586,10 @@ struct FnTrace {
   }
 };
 
+// Fixed-tree sum over a block of THREADS threads (a multiple of 64); thread 0 holds the result.
+template <int THREADS = kReduceThreads>
 __device__ __forceinline__ void block_reduce2(double& s0, double& s1) {
-  __shared__ double w0[kReduceThreads / 32], w1[kReduceThreads / 32];
+  __shared__ double w0[THREADS / 32], w1[THREADS / 32];
 #pragma unroll
   for (int off = 16; off > 0; off >>= 1) {
     s0 += __shfl_down_sync(0xffffffffu, s0, off);
@@ -597,10 +599,10 @@ __device__ __forceinline__ void block_reduce2(double& s0, double& s1) {
   if (lane == 0) { w0[warp] = s0; w1[warp] = s1; }
   __syncthreads();
   if (warp == 0) {
-    s0 = lane < kReduceThreads / 32 ? w0[lane] : 0.0;
-    s1 = lane < kReduceThreads / 32 ? w1[lane] : 0.0;
+    s0 = lane < THREADS / 32 ? w0[lane] : 0.0;
+    s1 = lane < THREADS / 32 ? w1[lane] : 0.0;
 #pragma unroll
-    for (int off = 4; off > 0; off >>= 1) {
+    for (int off = THREADS / 64; off > 0; off >>= 1) {
       s0 += __shfl_down_sync(0xffffffffu, s0, off);
       s1 += __shfl_down_sync(0xffffffffu, s1, off);
     }
@@ -786,14 +788,38 @@ k_pauli_rotate(qs_c128* __restrict__ state, const __grid_constant__ QsPauliRotPa
 // H|psi> for a Pauli sum and the adjoint sweep (plan.h, elem_ops.h, pauli.cpp)
 // =====================================================================================
 // The apply pass has the rotation pass's grid; every thread keeps its group spectrum in shared
-// memory ([entry][thread]: conflict-free), where the terms scatter by a runtime index.
-template <int D>
+// memory ([entry][thread]: conflict-free), where the terms scatter by a runtime index.  The LANCZOS
+// instantiation (qsim_lanczos_apply) may start from prev_scale x prev and, in the pass with A.dot,
+// writes one block partial of Re <in|out> to partials[2 * blockIdx.x] (k_pauli_final sums them).
+template <int D, bool LANCZOS = false>
 __global__ void __launch_bounds__(kRotThreads)
-k_pauli_apply(const qs_c128* __restrict__ in, qs_c128* __restrict__ out, const __grid_constant__ QsPauliApplyPass A,
-              uint64_t count) {
+k_pauli_apply(const qs_c128* __restrict__ in, const qs_c128* prev, qs_c128* __restrict__ out,
+              const __grid_constant__ QsPauliApplyPass A, uint64_t count, double* __restrict__ partials) {
   __shared__ double spec[(2 << D) * kRotThreads];
+  double dot = 0.0;
   for (uint64_t o = blockIdx.x * (uint64_t)kRotThreads + threadIdx.x; o < count; o += (uint64_t)gridDim.x * kRotThreads)
-    qs_pauli_apply_item<D>(A, in, out, o, spec + threadIdx.x, kRotThreads);
+    dot += qs_pauli_apply_item<D, LANCZOS>(A, in, prev, out, o, spec + threadIdx.x, kRotThreads);
+  if (LANCZOS && A.dot) {
+    double unused = 0.0;
+    block_reduce2<kRotThreads>(dot, unused);
+    if (threadIdx.x == 0) {
+      partials[2 * blockIdx.x] = dot;
+      partials[2 * blockIdx.x + 1] = 0.0;
+    }
+  }
+}
+
+// One Lanczos step (qs_lanczos_step_elem): a streaming pass over w, v and y with one 16-byte access
+// per amplitude and array, and a block partial of |w|^2 (|y|^2 without w) for k_reduce_final.
+__global__ void __launch_bounds__(kReduceThreads)
+k_lanczos_step(qs_c128* __restrict__ w, const qs_c128* __restrict__ v, qs_c128* __restrict__ y, uint64_t count,
+               double a, double bre, double bim, double* __restrict__ partials) {
+  double s0 = 0.0, s1 = 0.0;
+  for (uint64_t i = blockIdx.x * (uint64_t)kReduceThreads + threadIdx.x; i < count;
+       i += (uint64_t)gridDim.x * kReduceThreads)
+    s0 += qs_lanczos_step_elem(w, v, y, i, a, bre, bim);
+  block_reduce2(s0, s1);
+  if (threadIdx.x == 0) { partials[2 * blockIdx.x] = s0; partials[2 * blockIdx.x + 1] = s1; }
 }
 
 // One sweep pass: psi and lam together, one accumulator per rotation and thread in shared memory;
@@ -1641,25 +1667,74 @@ int apply_pauli_rotations(qs_c128* state, int n, const PauliRotPlan& plan, void*
   return QSIM_OK;
 }
 
+unsigned apply_grid(const DevCtx* ctx, int n, const PauliApplyPlan& plan) {
+  const uint64_t count = 1ull << (n - plan.d);
+  return (unsigned)std::min<uint64_t>((count + kRotThreads - 1) / kRotThreads, (uint64_t)ctx->sms * kRotBlocksPerSM);
+}
+
+template <bool LANCZOS>
+int launch_apply(const qs_c128* in, const qs_c128* prev, qs_c128* out, int n, const PauliApplyPlan& plan,
+                 unsigned blocks, double* partials, cudaStream_t st) {
+  const uint64_t count = 1ull << (n - plan.d);
+  for (const QsPauliApplyPass& A : plan.passes) {
+    switch (plan.d) {
+      case 1: k_pauli_apply<1, LANCZOS><<<blocks, kRotThreads, 0, st>>>(in, prev, out, A, count, partials); break;
+      case 2: k_pauli_apply<2, LANCZOS><<<blocks, kRotThreads, 0, st>>>(in, prev, out, A, count, partials); break;
+      case 3: k_pauli_apply<3, LANCZOS><<<blocks, kRotThreads, 0, st>>>(in, prev, out, A, count, partials); break;
+      default: k_pauli_apply<4, LANCZOS><<<blocks, kRotThreads, 0, st>>>(in, prev, out, A, count, partials); break;
+    }
+    const int rc = launched();
+    if (rc != QSIM_OK) return rc;
+  }
+  return QSIM_OK;
+}
+
 int apply_pauli_sum(const qs_c128* in, qs_c128* out, int n, const PauliApplyPlan& plan, void* stream) {
   Bound bound;
   int rc = bind_device(out, &bound);
   DevCtx* ctx = bound.ctx;
   if (rc != QSIM_OK) return rc;
-  const uint64_t count = 1ull << (n - plan.d);
-  const unsigned blocks = (unsigned)std::min<uint64_t>((count + kRotThreads - 1) / kRotThreads,
-                                                       (uint64_t)ctx->sms * kRotBlocksPerSM);
+  const unsigned blocks = apply_grid(ctx, n, plan);
+  return launch_apply<false>(in, nullptr, out, n, plan, blocks, nullptr, (cudaStream_t)stream);
+}
+
+int lanczos_apply(const qs_c128* in, const qs_c128* prev, qs_c128* out, int n, const PauliApplyPlan& plan,
+                  double* out_dot, void* stream) {
+  Bound bound;
+  int rc = bind_device(out, &bound);
+  DevCtx* ctx = bound.ctx;
+  if (rc != QSIM_OK) return rc;
+  const unsigned blocks = apply_grid(ctx, n, plan);
   const cudaStream_t st = (cudaStream_t)stream;
-  for (const QsPauliApplyPass& A : plan.passes) {
-    switch (plan.d) {
-      case 1: k_pauli_apply<1><<<blocks, kRotThreads, 0, st>>>(in, out, A, count); break;
-      case 2: k_pauli_apply<2><<<blocks, kRotThreads, 0, st>>>(in, out, A, count); break;
-      case 3: k_pauli_apply<3><<<blocks, kRotThreads, 0, st>>>(in, out, A, count); break;
-      default: k_pauli_apply<4><<<blocks, kRotThreads, 0, st>>>(in, out, A, count); break;
-    }
-    rc = launched();
-    if (rc != QSIM_OK) return rc;
-  }
+  std::lock_guard<std::mutex> guard(ctx->reduce_lock);
+  rc = pauli_scratch(ctx, 1, blocks);
+  if (rc != QSIM_OK) return rc;
+  rc = launch_apply<true>(in, prev, out, n, plan, blocks, ctx->d_pauli_partials, st);
+  if (rc != QSIM_OK) return rc;
+  double sums[2];
+  rc = pauli_sums_to_host(ctx, 1, (int)blocks, sums, st);
+  if (rc == QSIM_OK) *out_dot = sums[0];
+  return rc;
+}
+
+int lanczos_step(qs_c128* w, const qs_c128* v, qs_c128* y, uint64_t n_amps, double a, double bre, double bim,
+                 double* out_norm2, void* stream) {
+  Bound bound;
+  int rc = bind_device(v, &bound);
+  DevCtx* ctx = bound.ctx;
+  if (rc != QSIM_OK) return rc;
+  const unsigned blocks = (unsigned)std::min<uint64_t>((n_amps + kReduceThreads - 1) / kReduceThreads, kReduceBlocks);
+  const cudaStream_t st = (cudaStream_t)stream;
+  std::lock_guard<std::mutex> guard(ctx->reduce_lock);
+  k_lanczos_step<<<blocks, kReduceThreads, 0, st>>>(w, v, y, n_amps, a, bre, bim, ctx->d_partials);
+  rc = launched();
+  if (rc != QSIM_OK || !out_norm2) return rc;
+  k_reduce_final<<<1, kReduceThreads, 0, st>>>(ctx->d_partials, (int)blocks, ctx->d_out);
+  rc = launched();
+  if (rc != QSIM_OK) return rc;
+  QS_CUDA(cudaMemcpyAsync(ctx->h_out, ctx->d_out, sizeof(double), cudaMemcpyDeviceToHost, st));
+  QS_CUDA(cudaStreamSynchronize(st));
+  *out_norm2 = ctx->h_out[0];
   return QSIM_OK;
 }
 

@@ -250,11 +250,20 @@ static_assert(sizeof(QsPauliRotPass) <= 4096, "QsPauliRotPass is a kernel parame
 // F the Walsh transform of the spectrum that holds +-k_t at index spec_t: one transform per group,
 // whatever the number of its terms.  The first pass of a qsim_apply_pauli_sum call writes out, later
 // passes add to it; every pass of a qsim_accumulate_pauli_sum call adds.
+//
+// A qsim_lanczos_apply call runs the same passes through the kernel's Lanczos instantiation, which
+// alone reads the two fields after `accumulate`: its first pass starts from prev_scale x prev
+// (QS_APPLY_FROM_PREV) or prev_scale x out when the caller's prev is out (QS_APPLY_FROM_OUT), and
+// its last pass (`dot`) also returns the work item's share of Re sum conj(in) out.
+#define QS_APPLY_FROM_PREV 2u
+#define QS_APPLY_FROM_OUT 3u
 struct QsPauliApplyPass {
   QsPauliPass p;
   double   kre[QS_PAULI_MAX_TERMS];          // k_t, slot order of p
   double   kim[QS_PAULI_MAX_TERMS];
-  uint32_t accumulate;                       // 0: write out; 1: add to it
+  uint32_t accumulate;                       // 0: write out; 1: add to it; QS_APPLY_FROM_PREV / _OUT
+  uint32_t dot;                              // Lanczos only: 1 = reduce Re <in|out> after this pass
+  double   prev_scale;                       // Lanczos only: p of the first pass
 };
 static_assert(sizeof(QsPauliApplyPass) <= 4096, "QsPauliApplyPass is a kernel parameter");
 

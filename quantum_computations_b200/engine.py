@@ -487,6 +487,36 @@ def _qubit_list(qubits, n: int) -> list:
     return q
 
 
+def lanczos_apply(backend, in_buf, prev_buf, out_buf, n_bits: int, x_masks, z_masks, coeffs,
+                  prev_scale: float = 0.0) -> float:
+    """``qsim_lanczos_apply``: out <- prev_scale * prev + sum_t coeffs[t] P_t in on three buffers of
+    2^n_bits amplitudes (``prev_buf`` may be ``out_buf`` or None for zeros); returns Re <in|out>.
+    Strings as in ``DeviceState.expect_pauli``.  Synchronises."""
+    x = np.ascontiguousarray(x_masks, dtype=np.uint64).reshape(-1)
+    z = np.ascontiguousarray(z_masks, dtype=np.uint64).reshape(-1)
+    c = np.ascontiguousarray(coeffs, dtype=np.complex128).reshape(-1)
+    if x.shape != z.shape or x.shape != c.shape:
+        raise ValueError("x_masks, z_masks and coeffs must have the same length")
+    out = np.zeros(1, dtype=np.float64)
+    prev = None if prev_buf is None else backend.ptr(prev_buf)
+    _capi.check(backend.lib, backend.lib.qsim_lanczos_apply(
+        backend.ptr(in_buf), prev, backend.ptr(out_buf), int(n_bits), len(x), x.ctypes.data, z.ctypes.data,
+        c.ctypes.data, float(prev_scale), _dptr(out), backend.stream()))
+    return float(out[0])
+
+
+def lanczos_step(backend, w_buf, v_buf, y_buf, n_amps: int, a: float, b: complex = 0.0, norm: bool = True):
+    """``qsim_lanczos_step``: w <- w - a v and, with ``y_buf``, y <- y + b v in one pass (``w_buf`` None
+    updates y alone).  Returns |w|^2 (|y|^2 without w) when ``norm``, else None without synchronising."""
+    bb = np.array([complex(b).real, complex(b).imag], dtype=np.float64)
+    out = np.zeros(1, dtype=np.float64)
+    ptr = lambda buf: None if buf is None else backend.ptr(buf)     # noqa: E731
+    _capi.check(backend.lib, backend.lib.qsim_lanczos_step(
+        ptr(w_buf), backend.ptr(v_buf), ptr(y_buf), C.c_uint64(int(n_amps)), float(a), _dptr(bb),
+        _dptr(out) if norm else None, backend.stream()))
+    return float(out[0]) if norm else None
+
+
 def marginal_probs(backend, buf, n: int, qubits, dm: bool = False):
     """``qsim_marginal_probs`` (``_dm``) of the buffer over reference qubits ``qubits`` of an
     n-qubit register: a new device array of 2^len(qubits) doubles."""

@@ -18,6 +18,9 @@ and write of the state.
 ``expect_and_gradient`` gives <H> after a rotation list together with its gradient with respect to
 every angle, by the adjoint method (``qsim_pauli_rotations_adjoint``).
 
+``ground_state`` (Lanczos) and ``evolve_krylov`` (exact-to-tolerance exp(-iHt)) are the references
+to judge a variational or Trotterised result against; both keep no Krylov basis (``krylov``).
+
 Convention: a string is a pair of masks ``(x, z)`` with bit q for reference
 qubit q; I = (0, 0), X = (1, 0), Z = (0, 1), Y = (1, 1), and the operator is
 ``i^popc(x & z) X^x Z^z`` (Z first), so every string is Hermitian.
@@ -91,6 +94,34 @@ class PauliSum:
         self.z_masks = np.array(zs, dtype=np.uint64)
         self.coeffs = np.array(coeffs, dtype=np.complex128)
         self.num_qubits = nq
+
+    @classmethod
+    def _from_masks(cls, x_masks, z_masks, coeffs, num_qubits: int) -> "PauliSum":
+        """A sum over distinct strings given as masks, without re-parsing them."""
+        out = cls([])
+        out.x_masks = np.ascontiguousarray(x_masks, dtype=np.uint64)
+        out.z_masks = np.ascontiguousarray(z_masks, dtype=np.uint64)
+        out.coeffs = np.ascontiguousarray(coeffs, dtype=np.complex128)
+        out.num_qubits = int(num_qubits)
+        return out
+
+    def liouvillian(self, n: int | None = None) -> "PauliSum":
+        """L = H (x) I - I (x) H^T on the 2n qubits of the vec of an n-qubit density matrix (qubits
+        0..n-1 are the row qubits, n..2n-1 the column qubits, as in ``DeviceState``), so that
+        vec(H rho - rho H) = L vec(rho) and vec(e^{-iHt} rho e^{iHt}) = exp(-iLt) vec(rho).  A row term
+        is (x, z, c), a column term (x << n, z << n, -c (-1)^popc(x & z)) because P^T = (-1)^popc(x & z) P
+        (Y^T = -Y); the identity terms cancel.  L is Hermitian when H is."""
+        n = self.num_qubits if n is None else int(n)
+        if n < self.num_qubits:
+            raise ValueError(f"the sum acts on {self.num_qubits} qubits, more than n = {n}")
+        if 2 * n > 63:
+            raise PauliError("Pauli strings on more than 63 qubits are not supported")
+        keep = (self.x_masks != 0) | (self.z_masks != 0)
+        x, z, c = self.x_masks[keep], self.z_masks[keep], self.coeffs[keep]
+        odd = np.array([bin(int(v)).count("1") & 1 for v in (x & z)], dtype=bool)
+        shift = np.uint64(n)
+        return PauliSum._from_masks(np.concatenate([x, x << shift]), np.concatenate([z, z << shift]),
+                                    np.concatenate([c, np.where(odd, c, -c)]), 2 * n)
 
     def __len__(self) -> int:
         return len(self.coeffs)
@@ -270,3 +301,50 @@ def evolve(hamiltonian: PauliSum, state, time: float, *, steps: int = 1, order: 
         raise ValueError(f"the Hamiltonian acts on {hamiltonian.num_qubits} qubits, "
                          f"the state has {state.num_qubits}")
     return state.apply_pauli_rotations(x, z, angles)
+
+
+def ground_state(hamiltonian: PauliSum, state, *, tol: float = 1e-10, max_iter: int = 300,
+                 return_state: bool = False):
+    """The lowest eigenvalue of H by the Lanczos method from the ket ``state`` (an
+    ``engine.DeviceState`` or a host ndarray, uploaded first; left unchanged).  Returns
+    ``(energy, residual)`` or, with ``return_state``, ``(energy, residual, DeviceState)``.
+
+    ``residual`` = beta_{k+1} |e_k^T s| (s the lowest Ritz vector of T_k) bounds |E - theta|.  The
+    iteration stops when it is <= ``tol``, at ``max_iter`` iterations, or at a happy breakdown
+    (beta <= 1e-14 |T|: the Krylov space is invariant and the energy exact).  There is no
+    reorthogonalisation: lost orthogonality only adds ghost copies of converged Ritz values, which do
+    not move the lowest one.  The ground-state vector comes from a second pass that regenerates the
+    Lanczos vectors bit for bit (``krylov``); it is normalised up to that loss of orthogonality.
+
+    Each iteration is one ``qsim_lanczos_apply`` (the passes of H|psi> with the dot fused in) and
+    one ``qsim_lanczos_step``; the energy needs 3 state buffers including ``state``, the vector 4.
+    H must have real coefficients.  A density matrix raises ValueError, a sharded state
+    NotImplementedError."""
+    from . import krylov
+    if not isinstance(hamiltonian, PauliSum):
+        raise TypeError("ground_state needs a PauliSum Hamiltonian")
+    if isinstance(state, _sharded_type()):
+        raise NotImplementedError("ground_state on a sharded state is not implemented")
+    state = _device_state(state, hamiltonian.num_qubits, "Hamiltonian")
+    return krylov.ground_state(hamiltonian, state, tol=tol, max_iter=max_iter, return_state=return_state)
+
+
+def evolve_krylov(hamiltonian: PauliSum, state, time: float, *, tol: float = 1e-12):
+    """exp(-i H time) applied in place to ``state`` (an ``engine.DeviceState`` ket or density matrix,
+    rho -> e^{-iHt} rho e^{iHt}), to within ``tol`` in the 2-norm of the state (Frobenius norm of
+    rho); returns the state.  H must have real coefficients; the identity term is a global phase, as
+    in ``evolve``.  A density matrix evolves as the ket vec(rho) under ``PauliSum.liouvillian``.
+
+    The time is cut into substeps.  A substep's first Lanczos pass runs until Saad's a-posteriori
+    error estimate beta_m |[exp(-i T_m dt)]_{m-1,0}| |psi| for the remaining time is within that
+    time's share of ``tol``, or until m = 30; dt then follows from T_m alone, so every substep uses
+    the budget in proportion to dt / time.  A second pass regenerates the m Lanczos vectors and adds
+    them up into the result.  4 state buffers including ``state``; at most one copy back into it at
+    the end.  A sharded state raises NotImplementedError."""
+    from . import krylov
+    if not isinstance(hamiltonian, PauliSum):
+        raise TypeError("evolve_krylov needs a PauliSum Hamiltonian")
+    if isinstance(state, _sharded_type()):
+        raise NotImplementedError("evolve_krylov on a sharded state is not implemented")
+    state = _device_state(state, hamiltonian.num_qubits, "Hamiltonian")
+    return krylov.evolve_krylov(hamiltonian, state, time, tol=tol)
